@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the measurement contract (see DESIGN.md "Measurement").
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (config.workload): BASELINE.json configs[2] per-GPU shard -- UncorEncounterModel.sample on
@@ -83,6 +83,43 @@ class ClockSampler:
                 "reasons": reasons, "samples": len(sm)}
 
 
+DUMP_TRACKS = 2048        # tracks written whole by --dump-outputs: about 35 MB at T = 600
+
+
+def tiled_tracks(buf, nvar, T, idx):
+    """Tracks `idx` of a dense tiled output buffer as (k, nvar, T), read in place: TrackResult.bins / .values would untile
+    all of it ([ceil(T/4)][ceil(n/128)][nvar][128][4], model.untile) into a 14 GB temporary first."""
+    from em_model_manned_bayes_b200.model import TRACK_TILE
+    nch = (T + 3) // 4
+    a = buf.reshape(nch, -1, nvar, TRACK_TILE, 4)[:, idx // TRACK_TILE, :, idx % TRACK_TILE, :]      # (k, nch, nvar, 4)
+    return a.permute(0, 2, 1, 3).reshape(len(idx), nvar, nch * 4)[:, :, :T]
+
+
+def dump_outputs(out_dir, res, hist_initial, hist_transition):
+    """--dump-outputs: what the last timed step returned to its caller, as <out_dir>/<name>.npy in float32 or float64.
+    The full outputs are 14.5 GB, so a fixed seeded sample of DUMP_TRACKS tracks is written (every variable, every
+    second; their indices in track_index.npy), together with the verification histograms, which cover every track."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(0).choice(res.n, size=min(DUMP_TRACKS, res.n), replace=False))
+    t = torch.from_numpy(idx).to(res.bins_tiled.device)
+    arrays = {
+        "track_index": idx.astype(np.float64),
+        "bins": tiled_tracks(res.bins_tiled, len(res.dyn_vars), res.T, t).float(),   # (k, n_dyn, T), 1-based
+        "values": tiled_tracks(res.values_tiled, len(res.tv_vars), res.T, t),         # (k, n_tv, T)
+        "init_bins": res.init_bins[:, t].float(),                                      # (n_initial, k)
+        "init_values": res.init_values[:, t],                                          # (n_initial, k)
+        "attempts": (res.attempts[t].to(torch.int32) & 0xFFFF).float(),                 # uint16 held in an int16 tensor
+        "hist_initial": hist_initial.double(),
+        "hist_transition": hist_transition.double(),
+    }
+    arrays = {k: (v.cpu().numpy() if torch.is_tensor(v) else v) for k, v in arrays.items()}
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def materialise_model():
     from em_model_manned_bayes_b200.model_archive import materialize
     d = os.path.join(tempfile.gettempdir(), "emb_bench_models_%d" % os.getuid())
@@ -154,8 +191,13 @@ def main():
     ap.add_argument("--tracks", type=int, default=TRACKS_PER_GPU, help="tracks per GPU per step")
     ap.add_argument("--e2e-steps", type=int, default=5)
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to the B200 path only")
         return run_reference(args)
 
     import numpy as np
@@ -228,6 +270,8 @@ def main():
     value = units_per_step * args.steps / (total_ms * 1e-3)
     assert int(hi.sum().item()) == world * n * m.n_initial, "verification histogram lost samples"
     assert int(ht.sum().item()) == world * n * (T - 1) * m.n_dyn
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, hi, ht)
 
     # ---- end-to-end arm: C ABI with pinned host buffers, D2H inside the timed region --------------
     nb = int(lib.emb_tracks_bins_len(m._h, n, T))

@@ -16,7 +16,11 @@ if ROOT not in sys.path:
 from em_model_manned_bayes_b200 import _lib as L  # noqa: E402
 from em_model_manned_bayes_b200.model import untile_bins, untile_values  # noqa: E402
 
-REF_MODEL_DIR = "/root/reference/model"
+# A checkout of the upstream MATLAB project (Airspace-Encounter-Models/em-model-manned-bayes), which this repository does
+# not vendor: the sweep over all of its model/*.txt files (more than the packed archive holds) runs only when
+# EMB200_REFERENCE_DIR names one.
+REF_DIR = os.environ.get("EMB200_REFERENCE_DIR", "")
+REF_MODEL_DIR = os.path.join(REF_DIR, "model") if REF_DIR else ""
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 

@@ -76,65 +76,56 @@ def test_terminal_structs_match_header_sizes():
 
 
 MATLAB_DIR = os.path.join(ROOT, "matlab")
-REF_MATLAB = "/root/reference/code/matlab"
 
 
-def _classdef_members(path):
-    """Property and method names declared by a MATLAB classdef file (and the method files of its @folder)."""
-    import re
-    names = set()
-    block = None
-    for ln in open(path, encoding="utf-8", errors="replace"):
-        s = ln.strip()
-        m = re.match(r"(properties|methods|events|enumeration)\b", s)
-        if m:
-            block = m.group(1)
-            continue
-        if s == "end" or s.startswith("end %"):
-            continue
-        if block == "properties":
-            m = re.match(r"([A-Za-z]\w*)\s*(\(|=|;|$|\{|[A-Za-z])", s)
-            if m and not s.startswith("%"):
-                names.add(m.group(1))
-        m = re.match(r"function\s+(?:\[?[^=]*\]?\s*=\s*)?(?:(?:get|set)\.)?([A-Za-z]\w*)", s)
-        if m:
-            names.add(m.group(1))
-    folder = os.path.dirname(path)
-    if os.path.basename(folder).startswith("@"):
-        names |= {os.path.splitext(f)[0] for f in os.listdir(folder) if f.endswith(".m")}
-    return names
+def _upstream():
+    """What these tests need of the upstream classes and functions (tests/golden/upstream_reference.json)."""
+    import json
+    return json.load(open(os.path.join(ROOT, "tests", "golden", "upstream_reference.json")))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_MATLAB), reason="needs the reference checkout (build container only)")
+def _glue_sources():
+    for f in sorted(os.listdir(MATLAB_DIR)):
+        if f.endswith(".m"):
+            yield f, "\n".join(ln.split("%")[0] for ln in open(os.path.join(MATLAB_DIR, f)))
+
+
 def test_matlab_glue_only_reads_members_the_reference_classes_have():
     """Every `self.<name>` / `mdl.<name>` / `m.<name>` the shipped .m files read must be a property or method of the
     reference's classes (EncounterModel, UncorEncounterModel, CorTerminalModel) -- round 1's glue read
     parameters_filename / isOverwriteZeroBoundaries / idxZeroBoundaries, which the objects do not keep
     (@EncounterModel/EncounterModel.m:98-104 are constructor locals)."""
     import re
-    members = set()
-    for cls in ("EncounterModel", "UncorEncounterModel", "CorTerminalModel"):
-        members |= _classdef_members(os.path.join(REF_MATLAB, "@" + cls, cls + ".m"))
+    members = set(_upstream()["class_members"])
     assert {"G_initial", "N_transition", "dirichlet_initial", "start", "temporal_map", "r_initial", "n_initial",
             "boundaries", "resample_rates", "mdlFwd1_1", "dynLimits1", "bounds_sample"} <= members
     assert "parameters_filename" not in members and "idxZeroBoundaries" not in members
     seen = 0
-    for f in sorted(os.listdir(MATLAB_DIR)):
-        if not f.endswith(".m"):
-            continue
-        src = "\n".join(ln.split("%")[0] for ln in open(os.path.join(MATLAB_DIR, f)))
+    for f, src in _glue_sources():
         for obj, name in re.findall(r"\b(self|mdl|m)\.([A-Za-z]\w*)", src):
             assert name in members, "%s reads %s.%s, which the reference classes do not have" % (f, obj, name)
             seen += 1
     assert seen >= 30
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_MATLAB), reason="needs the reference checkout (build container only)")
 def test_matlab_glue_calls_reference_functions_with_their_signatures():
     """The helper functions the glue calls must exist in the reference with the arity used."""
     import re
-    for fn, nargs in (("events2samples", 2), ("events2controls", 3), ("bn_dirichlet_prior", 2), ("setTransitionPriors", 4)):
-        head = open(os.path.join(REF_MATLAB, fn + ".m")).readline()
-        m = re.search(r"%s\s*\(([^)]*)\)" % fn, head)
-        assert m and len(m.group(1).split(",")) == nargs, head
-    assert os.path.exists(os.path.join(REF_MATLAB, "@EncounterModelEvents", "EncounterModelEvents.m"))
+    up = _upstream()
+    calls = {}
+    for f, src in _glue_sources():
+        src = src.replace("...\n", " ")
+        for fn in up["function_arity"]:
+            for m in re.finditer(r"\b%s\s*\(" % fn, src):
+                depth, nargs = 1, 1
+                for ch in src[m.end():]:
+                    depth += {"(": 1, "[": 1, "{": 1, ")": -1, "]": -1, "}": -1}.get(ch, 0)
+                    if depth == 0:
+                        break
+                    nargs += ch == "," and depth == 1
+                calls.setdefault(fn, []).append(nargs)
+    assert sorted(calls) == sorted(up["function_arity"])
+    for fn, used in calls.items():
+        assert set(used) == {up["function_arity"][fn]}, fn
+    assert "EncounterModelEvents" in up["classes"]
+    assert any(re.search(r"\bEncounterModelEvents\b", src) for _, src in _glue_sources())

@@ -228,7 +228,7 @@ def test_tracks_across_a_2_32_sample_boundary(model_paths, fast):
     assert np.all(np.abs(got["values"].astype(np.float64) - want) <= 1e-6 * np.abs(want))
 
 
-@pytest.mark.skipif(not H.have_reference(), reason="needs the reference checkout's model/*.txt (build container only)")
+@pytest.mark.skipif(not H.have_reference(), reason="needs EMB200_REFERENCE_DIR (an upstream checkout with model/*.txt)")
 def test_every_shipped_dbn_model_runs_specialised_and_matches_the_c_oracle():
     """All model/*.txt files with a transition network (not just the archived ones): the specialised code path
     (EMB_FAST_SHAPES covers every shipped shape and sampling order) against the plain-C restatement."""
