@@ -160,6 +160,8 @@ def lib():
         "emb_sample_tracks_xyz": (C.c_int, [vp, P(Rng), i64, i32, P(SampleOpts), P(IntegrateOpts), P(TrackOut), vp, vp]),
         "emb_tracks_bins_len": (i64, [vp, i64, i32]),
         "emb_tracks_values_len": (i64, [vp, i64, i32]),
+        "emb_loglik_initial": (C.c_int, [vp, i64, vp, P(SampleOpts), vp, vp]),
+        "emb_loglik_tracks": (C.c_int, [vp, i64, i32, vp, vp, P(SampleOpts), vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)  # AttributeError if a declared symbol is missing
@@ -176,7 +178,7 @@ EXPORTED = [
     "emb_model_get_packed", "emb_set_prior", "emb_sample_opts_init", "emb_sample_initial", "emb_sample_tracks",
     "emb_tracks_bins_len", "emb_tracks_values_len", "emb_sample_track_events",
     "emb_dyn_limits_named", "emb_terminal_propagate", "emb_terminal_traj_len", "emb_tracks_integrate", "emb_sample_tracks_xyz",
-    "emb_terminal_screen",
+    "emb_terminal_screen", "emb_loglik_initial", "emb_loglik_tracks",
 ]
 TRAJ_FIELDS = ("x_nm", "y_nm", "z_ft", "heading_deg", "v_ft_s")
 

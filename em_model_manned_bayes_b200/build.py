@@ -20,7 +20,7 @@ LIB = os.path.join(HERE, "libemb200.so")
 
 CU_SOURCES = ["emb_kernels.cu", "emb_terminal.cu"]
 CXX_SOURCES = ["emb_model.cpp", "emb_api.cpp", "emb_multi.cpp"]
-HEADERS = ["emb_device.cuh", "emb_fast.cuh", "emb_initial.cuh", "emb_terminal.cuh", "emb_integrate.cuh", "emb_model.h", "emb_launch.h", os.path.join(ROOT, "include", "emb200.h")]
+HEADERS = ["emb_device.cuh", "emb_fast.cuh", "emb_initial.cuh", "emb_terminal.cuh", "emb_integrate.cuh", "emb_loglik.cuh", "emb_model.h", "emb_launch.h", os.path.join(ROOT, "include", "emb200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-fmad=false",

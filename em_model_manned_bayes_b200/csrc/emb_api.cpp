@@ -16,6 +16,7 @@
 #include "../../include/emb200.h"
 #include "emb_integrate.cuh"
 #include "emb_launch.h"
+#include "emb_loglik.cuh"
 #include "emb_model.h"
 
 using emb::DevModel;
@@ -59,6 +60,10 @@ int ensure_device(const HostModel& H, int device, DevModel& D) {
         if (c.thr_transition) cudaFree(c.thr_transition);
         if (c.edges) cudaFree(c.edges);
         if (c.dd32) cudaFree(c.dd32);
+        if (c.logp_initial) cudaFree(c.logp_initial);
+        if (c.logp_transition) cudaFree(c.logp_transition);
+        c.logp_initial = c.logp_transition = nullptr;
+        c.logp_ok = false;
         c.thr_initial = c.thr_transition = nullptr;
         c.edges = nullptr;
         c.dd32 = nullptr;
@@ -81,6 +86,27 @@ int ensure_device(const HostModel& H, int device, DevModel& D) {
     D.thr_trans = c.thr_transition;
     D.edges = c.edges;
     D.dd32 = c.dd32;
+    D.logp_init = D.logp_trans = nullptr;
+    return 0;
+}
+
+// ensure_device plus the scoring tables, uploaded on the first scoring call so that sampling-only callers never hold them in HBM
+int ensure_logp(const HostModel& H, int device, DevModel& D) {
+    int rc = ensure_device(H, device, D);
+    if (rc) return rc;
+    std::lock_guard<std::mutex> lk(H.mu);
+    auto& c = H.device_copies[device];
+    if (!c.logp_ok) {
+        for (auto* t : {&H.logp_initial, &H.logp_transition}) {
+            double*& dst = t == &H.logp_initial ? c.logp_initial : c.logp_transition;
+            if (t->empty()) continue;
+            CU(cudaMalloc((void**)&dst, t->size() * 8));
+            CU(cudaMemcpy(dst, t->data(), t->size() * 8, cudaMemcpyHostToDevice));
+        }
+        c.logp_ok = true;
+    }
+    D.logp_init = c.logp_initial;
+    D.logp_trans = c.logp_transition;
     return 0;
 }
 
@@ -374,6 +400,8 @@ void emb_model_free(emb_model* m) {
                 if (kv.second.thr_transition) cudaFree(kv.second.thr_transition);
                 if (kv.second.edges) cudaFree(kv.second.edges);
                 if (kv.second.dd32) cudaFree(kv.second.dd32);
+                if (kv.second.logp_initial) cudaFree(kv.second.logp_initial);
+                if (kv.second.logp_transition) cudaFree(kv.second.logp_transition);
                 cudaSetDevice(cur);
             }
         }
@@ -968,6 +996,75 @@ int emb_terminal_propagate(const emb_terminal_models* models, const emb_rng* rng
     if (status & 2) return set_err(EMB_E_ARG, "Unknown int_intent: own_intent must be 1..2 and int_intent 1..3 (createEncounter.m:22,37)");
     if (status & 1) return set_err(EMB_E_REJECT, "a trajectory state exhausted max_attempts in the dynamic-limit resample loop");
     return 0;
+}
+
+// ---- log-likelihood of given bins (emb_loglik.cuh) ------------------------------------------------------------------------
+// the device status word of the scoring kernels -> EMB_E_ARG with what was wrong
+static int loglik_status_error(int32_t status) {
+    if (status & emb::LL_BAD_BIN) return set_err(EMB_E_ARG, "loglik: a bin is outside 1..r of its variable");
+    if (status & emb::LL_BAD_COL0)
+        return set_err(EMB_E_ARG, "loglik: column 0 of the track bins differs from init_bins of the dynamic variables");
+    return 0;
+}
+
+// shared by both entry points: checks, device tables, staging, one launch, status
+static int loglik_impl(const emb_model* m, int64_t n, int32_t T, const int8_t* init_bins, const int8_t* bins,
+                       const emb_sample_opts* opts, double* initial, double* per_var, double* transition) {
+    const bool tracks = T > 0;
+    const HostModel& H = *m->h;
+    if (opts->mem & ~0xFF) return set_err(EMB_E_ARG, "loglik: EMB_MEM_ASYNC is not supported; scoring calls are synchronous");
+    if (n == 0) return 0;
+    int device, rc = 0;
+    if ((rc = pick_device(opts, device))) return rc;
+    DevModel D;
+    if ((rc = ensure_logp(H, device, D))) return rc;
+    if (opts->correct_dbn) D.fast = 0;
+    cudaStream_t st = (cudaStream_t)opts->stream;
+    g_call_stream = st;
+    Stager sg{opts->mem, st, {}};
+    const size_t ni = (size_t)H.n_initial;
+    emb::LoglikParams P{};
+    P.n = n;
+    P.T = T;
+    const void* d_in = nullptr;
+    if ((rc = sg.in(init_bins, (size_t)n * ni, &d_in))) return rc;
+    P.init_bins = (const int8_t*)d_in;
+    if (tracks && (rc = sg.in(bins, (size_t)emb_tracks_bins_len(m, n, T), &d_in))) return rc;
+    P.bins = tracks ? (const int8_t*)d_in : nullptr;
+    if ((rc = sg.out(initial, (size_t)n * 8, false, (void**)&P.initial))) return rc;
+    if ((rc = sg.out(per_var, (size_t)n * ni * 8, false, (void**)&P.per_var))) return rc;
+    if ((rc = sg.out(transition, (size_t)n * 8, false, (void**)&P.transition))) return rc;
+    CU(tmp_alloc((void**)&P.status, 4, st));
+    CU(cudaMemsetAsync(P.status, 0, 4, st));
+    cudaError_t e = tracks ? (cudaError_t)emb::launch_loglik_tracks(D, P, st)
+                           : (cudaError_t)emb::launch_loglik_initial(D, P, (int)H.logp_initial.size(), st);
+    if (e != cudaSuccess) {
+        tmp_free(P.status);
+        return cuda_fail(e, tracks ? "launch k_loglik_tracks" : "launch k_loglik_initial");
+    }
+    int32_t status = 0;
+    e = cudaMemcpyAsync(&status, P.status, 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    tmp_free(P.status);
+    if (e != cudaSuccess) return cuda_fail(e, tracks ? "k_loglik_tracks" : "k_loglik_initial");
+    if ((rc = sg.finish())) return rc;
+    return loglik_status_error(status);
+}
+
+int emb_loglik_initial(const emb_model* m, int64_t n, const int8_t* bins, const emb_sample_opts* opts, double* total,
+                       double* per_var) {
+    if (!m || !opts || n < 0 || (n > 0 && (!bins || !total))) return set_err(EMB_E_ARG, "null or out-of-range argument");
+    return loglik_impl(m, n, 0, bins, nullptr, opts, total, per_var, nullptr);
+}
+
+int emb_loglik_tracks(const emb_model* m, int64_t n, int32_t T, const int8_t* init_bins, const int8_t* bins,
+                      const emb_sample_opts* opts, double* initial, double* transition) {
+    if (!m || !opts || n < 0 || T < 1 || (n > 0 && (!init_bins || !bins)))
+        return set_err(EMB_E_ARG, "null or out-of-range argument");
+    const HostModel& H = *m->h;
+    if (!H.has_transition || H.temporal_map.empty())
+        return set_err(EMB_E_ARG, "dynvar:empty: model has no transition network");
+    return loglik_impl(m, n, T, init_bins, bins, opts, initial, nullptr, transition);
 }
 
 // IntegrateParams from emb_integrate_opts (labels -> tile ordinals, unit ratios); 0 or an error code

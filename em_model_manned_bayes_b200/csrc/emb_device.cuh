@@ -77,6 +77,8 @@ struct DevModel {
     const uint32_t* thr_trans;
     const double* edges;
     const float* dd32;             // per (gated ordinal, bin): {slope, base, s, c}  (emb_model.cpp: pack)
+    const double* logp_init;       // log(w_m / W) at the slots of thr_init / thr_trans; set by the scoring entry points only
+    const double* logp_trans;
 };
 
 struct SampleParams {

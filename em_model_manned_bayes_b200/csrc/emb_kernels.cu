@@ -12,6 +12,7 @@
 #include "emb_fast.cuh"
 #include "emb_initial.cuh"
 #include "emb_launch.h"
+#include "emb_loglik.cuh"
 
 namespace emb {
 
@@ -298,6 +299,38 @@ __global__ void k_publish(const long long* __restrict__ total, const int32_t* __
     dst[1] = (long long)*flag;
 }
 
+
+// ---- log-likelihood of given bins (emb_loglik.cuh) -----------------------------------------------------------------------
+// initial network: one thread per sample, grid-stride over a persistent grid; with SMEM the whole fp64 table is staged in shared
+// memory once per block (glider: 9 156 slots, 73 KB), so the per-variable gathers are LDS instead of L1/L2 lookups
+template <bool SMEM>
+__global__ void __launch_bounds__(256) k_loglik_initial(const __grid_constant__ DevModel M, const __grid_constant__ LoglikParams P,
+                                                        int table_len) {
+    extern __shared__ double s_logp[];
+    const double* logp = M.logp_init;
+    if (SMEM) {
+        for (int q = threadIdx.x; q < table_len; q += blockDim.x) s_logp[q] = __ldg(M.logp_init + q);
+        __syncthreads();
+        logp = s_logp;
+    }
+    uint8_t x[MAXV];
+    for (int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s < P.n; s += (int64_t)gridDim.x * blockDim.x) {
+        const double v = loglik_initial_one(M, logp, P, s, x);
+        if (P.initial) P.initial[s] = v;
+    }
+}
+
+// tracks: one thread per track.  FROZEN: per-thread counters in dynamic shared memory laid out [counter][thread] (consecutive
+// threads in consecutive banks), one byte extract + shared increment per variable-second; otherwise per-second gathers.
+template <bool FROZEN>
+__global__ void __launch_bounds__(128) k_loglik_tracks(const __grid_constant__ DevModel M, const __grid_constant__ LoglikParams P) {
+    extern __shared__ uint32_t s_cnt[];
+    const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= P.n) return;
+    const int tid = threadIdx.x, bs = blockDim.x;
+    loglik_track(M, P, s, FROZEN, [&](int k) -> uint32_t& { return s_cnt[k * bs + tid]; });
+}
+
 }  // namespace
 
 int launch_publish(const long long* total, const int32_t* flag, long long* mapped_dst, void* stream) {
@@ -425,6 +458,46 @@ int launch_tracks(const DevModel& M, const SampleParams& P0, const TrackOut& O, 
         g_launch_count.fetch_add(1);
     }
     g_last_kernel_fast = done ? 1 : 0;
+    return (int)cudaGetLastError();
+}
+
+
+int launch_loglik_initial(const DevModel& M, const LoglikParams& P, int table_len, void* stream) {
+    if (P.n <= 0) return 0;
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const int64_t need = (P.n + 255) / 256;
+    const size_t tbytes = (size_t)table_len * 8;
+    const bool smem = table_len > 0 && tbytes <= 96 * 1024 && need >= 2 * sms;   // staging pays only for large batches
+    unsigned grid = (unsigned)std::min<int64_t>(need, (int64_t)sms * 32);
+    if (smem) {
+        int occ = 1;
+        cudaFuncSetAttribute(k_loglik_initial<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tbytes);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_loglik_initial<true>, 256, tbytes);
+        grid = (unsigned)std::min<int64_t>(need, (int64_t)sms * std::max(occ, 1));
+        k_loglik_initial<true><<<grid, 256, tbytes, (cudaStream_t)stream>>>(M, P, table_len);
+    } else {
+        k_loglik_initial<false><<<grid, 256, 0, (cudaStream_t)stream>>>(M, P, table_len);
+    }
+    g_launch_count.fetch_add(1);
+    return (int)cudaGetLastError();
+}
+
+int launch_loglik_tracks(const DevModel& M, const LoglikParams& P, void* stream) {
+    if (P.n <= 0) return 0;
+    if (M.fast) {
+        // 128 tracks per block while the counters fit 96 KB of shared memory, fewer otherwise (8 variables of 127 bins at 32: 127 KB)
+        const size_t per_thread = (size_t)loglik_counters(M) * 4;
+        int block = 128;
+        while (block > 32 && per_thread * block > 96 * 1024) block /= 2;
+        const size_t bytes = per_thread * block;
+        cudaFuncSetAttribute(k_loglik_tracks<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+        k_loglik_tracks<true><<<(unsigned)((P.n + block - 1) / block), block, bytes, (cudaStream_t)stream>>>(M, P);
+    } else {
+        k_loglik_tracks<false><<<(unsigned)((P.n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(M, P);
+    }
+    g_launch_count.fetch_add(1);
     return (int)cudaGetLastError();
 }
 

@@ -31,6 +31,12 @@ int launch_expand_events(const DevModel& M, const uint32_t* words, const uint8_t
 // {*total, *flag} written by an SM into mapped pinned host memory (two long longs)
 int launch_publish(const long long* total, const int32_t* flag, long long* mapped_dst, void* stream);
 
+// log-likelihood of given bins (emb_loglik.cuh); M.logp_init / M.logp_trans set; table_len = slots of the initial table
+struct LoglikParams;
+int launch_loglik_initial(const DevModel& M, const LoglikParams& P, int table_len, void* stream);
+// M.fast selects the branch: frozen parents (counting kernel) or per-step parents
+int launch_loglik_tracks(const DevModel& M, const LoglikParams& P, void* stream);
+
 // terminal trajectory chains (emb_terminal.cu): 4 chains per encounter
 struct TermParams;
 struct TermOut;

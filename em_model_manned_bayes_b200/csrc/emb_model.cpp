@@ -14,6 +14,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <fstream>
+#include <limits>
 #include <memory>
 #include <queue>
 #include <sstream>
@@ -159,6 +160,19 @@ void pack_column(const double* w, int r, int rp, uint32_t* col) {
         else col[m] = (uint32_t)(lo - 1);  // lo == 2^32 -> 0xFFFFFFFF (never)
     }
     col[rp - 1] = lead;
+}
+
+void logp_column(const double* w, int r, int rp, double* col) {
+    double total = 0.0;
+    for (int m = 0; m < r; ++m) total += w[m];
+    const double ninf = -std::numeric_limits<double>::infinity();
+    for (int m = 0; m < rp; ++m) col[m] = ninf;
+    if (!(total > 0.0)) {
+        col[0] = 0.0;
+        return;
+    }
+    for (int m = 0; m < r; ++m)
+        if (w[m] > 0.0) col[m] = std::log(w[m] / total);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -344,7 +358,7 @@ struct AlphaFn {
 };
 
 void pack_table(const Table& t, const PriorSpec& pr, bool stay_ok, Node& node, std::vector<uint32_t>& out,
-                const std::vector<int32_t>& xindex_of_parent) {
+                std::vector<double>& logp, const std::vector<int32_t>& xindex_of_parent) {
     if (t.r > 127) fail(EMB_E_LIMIT, "more than 127 bins");
     if ((int)t.parents.size() > MAXP) fail(EMB_E_LIMIT, "more than EMB_MAX_PARENTS parents");
     node.r = t.r;
@@ -359,6 +373,7 @@ void pack_table(const Table& t, const PriorSpec& pr, bool stay_ok, Node& node, s
         a.stay_block = t.q / t.r;
     }
     out.resize(out.size() + (size_t)t.q * node.rp);
+    logp.resize(out.size());
     std::vector<double> w(t.r);
     for (int64_t j = 0; j < t.q; ++j) {
         for (int m = 0; m < t.r; ++m) {
@@ -367,6 +382,7 @@ void pack_table(const Table& t, const PriorSpec& pr, bool stay_ok, Node& node, s
             w[m] = v;
         }
         pack_column(w.data(), t.r, node.rp, out.data() + node.off + (size_t)j * node.rp);
+        logp_column(w.data(), t.r, node.rp, logp.data() + node.off + (size_t)j * node.rp);
     }
 }
 
@@ -388,11 +404,13 @@ void HostModel::pack() {
 
     thr_initial.clear();
     thr_transition.clear();
+    logp_initial.clear();
+    logp_transition.clear();
     std::vector<int32_t> ident;
     for (int i = 0; i < n; ++i) {
         const Table& t = T_initial[i];
         Node& nd = D.init[i];
-        pack_table(t, prior_initial, false, nd, thr_initial, ident);
+        pack_table(t, prior_initial, false, nd, thr_initial, logp_initial, ident);
         uint32_t stride = 1;
         for (int p = 0; p < nd.np; ++p) {  // asub2ind.m:13 strides over parents in increasing index
             nd.par[p] = (uint8_t)t.parents[p];
@@ -406,7 +424,7 @@ void HostModel::pack() {
         D.dyn_t1[d] = vt1;
         const Table& t = T_transition[vt1];
         Node& nd = D.dyn[d];
-        pack_table(t, prior_transition, true, nd, thr_transition, ident);
+        pack_table(t, prior_transition, true, nd, thr_transition, logp_transition, ident);
         uint32_t stride = 1;
         for (int p = 0; p < nd.np; ++p) {
             nd.par[p] = (uint8_t)t.parents[p];

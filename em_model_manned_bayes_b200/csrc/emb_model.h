@@ -57,6 +57,8 @@ struct HostModel {
     // ---- packed (rebuilt by pack()) ----
     DevModel dev{};                    // metadata with null table pointers
     std::vector<uint32_t> thr_initial, thr_transition;
+    // log(w_m / W) of the same columns, slot for slot (padding slots -inf): the scoring tables of emb_loglik.cuh
+    std::vector<double> logp_initial, logp_transition;
     std::vector<double> edges;         // per variable: a[bin], w[bin] interleaved
     std::vector<float> dd32;           // per (gated ordinal, bin): {slope, base, s, c}
     uint64_t version = 0;
@@ -68,6 +70,10 @@ struct HostModel {
         uint32_t* thr_transition = nullptr;
         double* edges = nullptr;
         float* dd32 = nullptr;
+        // uploaded by the first scoring call on the device (emb_api.cpp: ensure_logp), dropped with the others on a repack
+        bool logp_ok = false;
+        double* logp_initial = nullptr;
+        double* logp_transition = nullptr;
     };
     mutable std::mutex mu;
     mutable std::map<int, DeviceCopy> device_copies;
@@ -81,6 +87,9 @@ HostModel* load_model_file(const char* path, bool overwrite_zero_boundaries, con
 
 // Word-space thresholds of one column of weights w[0..r): fills col[0..rp) (see emb_device.cuh).
 void pack_column(const double* w, int r, int rp, uint32_t* col);
+// log(w_m / W) of the same column, W = sum(w) summed as select_random.m:17 does; a zero-total column gives bin 1 probability 1
+// (log 0, every other bin -inf), as the sampler does; slots r .. rp-1 are -inf.
+void logp_column(const double* w, int r, int rp, double* col);
 
 // Validates `opts` (bn_sample.m:45-50 preset rule, driver options) and fills the kernel parameters; throws Error.
 void fill_params(const HostModel& H, uint64_t seed, uint64_t first_sample, int64_t n, int32_t T,

@@ -375,6 +375,76 @@ class EncounterModel:
         L.check(lib.emb_sample_tracks(self._h, C.byref(rng), n, T, C.byref(o), C.byref(to)))
         return out
 
+    # -- scoring (emb200.h: emb_loglik_initial / emb_loglik_tracks) ----------------------------------------------------
+    def _score_call(self, arrays, device, correct_dbn):
+        """Options and buffer kind of a scoring call: torch CUDA tensors in -> device buffers on their device, outputs as tensors;
+        numpy in -> host buffers, computed on `device` (CUDA ordinal or torch device; default the current one)."""
+        o = self._opts(start=[None] * self.n_initial)
+        o.correct_dbn = int(bool(correct_dbn))
+        like = None
+        if not isinstance(arrays[0], np.ndarray):
+            import torch
+            dev = arrays[0].device
+            if dev.type != "cuda" or any(a.device != dev for a in arrays):
+                raise L.EmbError(L.EMB_E_ARG, "loglik: tensors must all be on one CUDA device (or pass numpy arrays)")
+            o.mem, o.device = L.EMB_MEM_DEVICE, dev.index if dev.index is not None else torch.cuda.current_device()
+            o.stream = torch.cuda.current_stream(dev).cuda_stream
+            like = dev
+        elif device is not None:
+            import torch
+            dev = torch.device(device) if not isinstance(device, int) else torch.device("cuda", device)
+            o.device = dev.index if dev.index is not None else -1
+        return o, like
+
+    @staticmethod
+    def _int8(a, like):
+        if like is None:
+            return np.ascontiguousarray(np.asarray(a), dtype=np.int8)
+        import torch
+        return a.to(torch.int8).contiguous()
+
+    def loglik_initial(self, bins, device=None, per_var: bool = False):
+        """log p(x) of initial-network bins under this model, sum_i log p(x_i | parents) in fp64 (emb_loglik_initial; the
+        semantics are in include/emb200.h).  `bins`: (n, n_initial) 1-based, as `sample_initial` returns them.  numpy in, numpy
+        out; a torch CUDA tensor in, tensors on its device out.  Returns total (n,) float64, and with `per_var` also the
+        per-variable terms (n, n_initial): drop the columns of preset variables to get the conditional of the free ones."""
+        o, like = self._score_call([bins], device, False)
+        if bins.shape[1] != self.n_initial:
+            raise L.EmbError(L.EMB_E_ARG, "loglik_initial: bins must be n x n_initial")
+        b = self._int8(bins.T, like)                                       # the ABI's [n_initial][n]
+        n = int(b.shape[1])
+        total = self._alloc((n,), np.float64, like)
+        pv = self._alloc((self.n_initial, n), np.float64, like) if per_var else None
+        L.check(L.lib().emb_loglik_initial(self._h, n, _ptr(b), C.byref(o), _ptr(total), _ptr(pv)))
+        return (total, pv.T) if per_var else total
+
+    def loglik_tracks(self, init_bins, bins_tiled=None, T: Optional[int] = None, correct_dbn: bool = False, device=None):
+        """log p of tracks under this model (emb_loglik_tracks): returns (initial (n,), transition (n,)) float64, the initial
+        term scoring column 0 and the transition term summing columns 1..T-1 on the sampler's branch (frozen parents, or
+        re-evaluated every second for models with a dynamic -> dynamic edge or with `correct_dbn`).
+        `init_bins`: (n_initial, n) 1-based as `TrackResult.init_bins`, or a whole `TrackResult` (then `bins_tiled` and `T` come
+        from it).  `bins_tiled`: the flat tiled layout of `sample_tracks`; turn plain (n, n_dyn, T) bins into it with `tile()`.
+        numpy in, numpy out; torch CUDA tensors in, tensors on their device out."""
+        if isinstance(init_bins, TrackResult):
+            r = init_bins
+            if r.init_bins is None or r.bins_tiled is None:
+                raise L.EmbError(L.EMB_E_ARG, "loglik_tracks: the TrackResult needs init_bins and bins (want_init, want_bins)")
+            init_bins, bins_tiled, T = r.init_bins, r.bins_tiled, r.T
+        if bins_tiled is None or T is None:
+            raise L.EmbError(L.EMB_E_ARG, "loglik_tracks: bins_tiled and T are required")
+        o, like = self._score_call([init_bins, bins_tiled], device, correct_dbn)
+        if init_bins.shape[0] != self.n_initial:
+            raise L.EmbError(L.EMB_E_ARG, "loglik_tracks: init_bins must be n_initial x n")
+        ib = self._int8(init_bins, like)
+        n = int(ib.shape[1])
+        bt = self._int8(bins_tiled, like).reshape(-1)
+        if self.n_dyn and int(bt.shape[0]) != int(L.lib().emb_tracks_bins_len(self._h, n, int(T))):
+            raise L.EmbError(L.EMB_E_ARG, "loglik_tracks: bins_tiled must have emb_tracks_bins_len(n, T) elements")
+        init = self._alloc((n,), np.float64, like)
+        trans = self._alloc((n,), np.float64, like)
+        L.check(L.lib().emb_loglik_tracks(self._h, n, int(T), _ptr(ib), _ptr(bt), C.byref(o), _ptr(init), _ptr(trans)))
+        return init, trans
+
 
 def async_status(device: int = -1) -> None:
     """Synchronise `device` and raise if an enqueue_only pass exhausted its rejection loop (emb_async_status)."""

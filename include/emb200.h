@@ -308,6 +308,35 @@ int emb_tracks_integrate(const emb_model* m, int64_t n, int32_t T, const double*
 int emb_sample_tracks_xyz(const emb_model* m, const emb_rng* rng, int64_t n, int32_t T, const emb_sample_opts* opts,
                           const emb_integrate_opts* iopts, const emb_track_out* out, float* xyz, uint8_t* is_good);
 
+/* ---- log-likelihood of given bins under a model: the inverse of the sampling entry points, for importance weights p(x)/q(x),
+ *      model comparison and validation.  Nothing in the reference computes this; the conditionals are the reference's own.
+ *
+ * Every conditional probability is the model's, in fp64: log(w_m / W), w the column of N + alpha that select_random.m:17 selects
+ * from (so emb_set_prior and emb_model_from_arrays weights apply exactly as they do to sampling), W = sum(w).  A zero-total column
+ * gives bin 1 with probability 1 as the sampler does (log-prob 0 for bin 1, -inf otherwise); a zero-weight bin gives -inf.
+ * These are the model's probabilities, not the sampler's word-space ones (emb_device.cuh), which differ by at most 2^-32 per bin.
+ *
+ * Initial network: log p(x) = sum_i log p(x_i | parents), parents addressed by asub2ind.m.
+ * Tracks: the state at dense column c is the tile bins of the dynamic variables at c plus init_bins for the static variables.
+ * The transition term sums over c = 1 .. T-1 and every dynamic variable; the parent configuration follows the branch the sampler
+ * uses: frozen at column 0 for a model without a dynamic -> dynamic edge (dbn_sample.m:110-135, SURVEY F6), re-evaluated every
+ * second otherwise or when opts->correct_dbn = 1 (dbn_sample.m:66-79).  Column 0 is the initial state: the initial term scores it.
+ * Not included: the rejection truncation of EMB_REJECT_* (these are unnormalised model probabilities), within-bin value
+ * densities (de-discretisation), and the resample gates (they change values, not bins).
+ *
+ * opts: only mem (EMB_MEM_HOST / EMB_MEM_DEVICE for every buffer; EMB_MEM_ASYNC is refused), device, stream and correct_dbn are
+ * read.  Calls are synchronous.  EMB_E_ARG when a bin is outside 1..r, when tile column 0 differs from init_bins of the dynamic
+ * variables, or (tracks) for a model without a transition network ("dynvar:empty").  Padding tracks and padding seconds of the
+ * tiles are ignored; the tiles beyond column 0 are read only when `transition` is requested. */
+/* log p of initial-network bins [n_initial][n] (emb_sample_initial's layout): total[n] and, nullable, per_var[n_initial][n]
+ * (a caller who sampled with `start` presets drops the preset variables' rows to get the conditional) */
+int emb_loglik_initial(const emb_model* m, int64_t n, const int8_t* bins, const emb_sample_opts* opts,
+                       double* total, double* per_var);
+/* log p of tracks: init_bins [n_initial][n] and the tiled dense bins of emb_sample_tracks (emb_tracks_bins_len(m, n, T)
+ * elements); initial[n] / transition[n] nullable */
+int emb_loglik_tracks(const emb_model* m, int64_t n, int32_t T, const int8_t* init_bins, const int8_t* bins,
+                      const emb_sample_opts* opts, double* initial, double* transition);
+
 /* ---- misc ------------------------------------------------------------------------------------- */
 int emb_host_alloc(void** p, int64_t bytes); /* pinned host memory */
 int emb_host_free(void* p);

@@ -31,6 +31,10 @@
 //          ur_heading, min_speed, max_speed;  xyz: n x (T+1) x 3 single, is_good: n x 1 uint8
 //   [xyz, is_good, out_inits] = emb_mex('sample_tracks_xyz', h, seed, first, n, T, opts, iopts)
 //          sampling and the loop of sample2track.m:188-244 in one kernel pass (no dense tiles); outputs as above
+//   [total, per_var] = emb_mex('loglik_initial', h, bins)              % log p of initial states (emb_loglik_initial)
+//          bins: n x n_initial int8 (1-based); total n x 1, per_var n x n_initial double
+//   [initial, transition] = emb_mex('loglik_tracks', h, init_bins, bins, T, correct_dbn)   % log p of tracks
+//          init_bins: n x n_initial int8; bins: the tiled int8 array of 'sample_tracks'; initial, transition n x 1 double
 //          emb_mex('free', h)
 // opts: struct with optional fields start (1 x n_initial, 0/NaN = free), reject_mode, idx_v, idx_dh,
 // idx_L, is_quantize500, layers (r_L x 2), box_lo, box_hi, max_attempts, device, start_per_sample (n x n_initial, 0/NaN = free:
@@ -288,7 +292,33 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         if (nlhs > 1) plhs[1] = bins; else mxDestroyArray(bins);
         if (nlhs > 2) plhs[2] = vals; else mxDestroyArray(vals);
         if (nlhs > 3) plhs[3] = att; else mxDestroyArray(att);
-    } else if (c == "sample_tracks_multi") {                      // every GPU of the box from one MATLAB process (SURVEY 8e)
+    } else if (c == "loglik_initial") {                           // log p of initial states (emb200.h: emb_loglik_initial)
+        // [total, per_var] = emb_mex('loglik_initial', h, bins)   bins: n x n_initial int8 (== the ABI's [n_initial][n])
+        const int64_t n = (int64_t)mxGetM(prhs[2]);
+        if ((int64_t)mxGetNumberOfElements(prhs[2]) != n * ni) mexErrMsgIdAndTxt("emb200:arg", "bins must be an int8 n x n_initial matrix");
+        emb_sample_opts o;
+        emb_sample_opts_init(&o);
+        plhs[0] = mxCreateDoubleMatrix(n, 1, mxREAL);
+        mxArray* pv = mxCreateDoubleMatrix(n, ni, mxREAL);
+        CHECK(emb_loglik_initial(m, n, (const int8_t*)mxGetData(prhs[2]), &o, mxGetPr(plhs[0]), mxGetPr(pv)));
+        if (nlhs > 1) plhs[1] = pv; else mxDestroyArray(pv);
+    } else if (c == "loglik_tracks") {                            // log p of tracks (emb200.h: emb_loglik_tracks)
+        // [initial, transition] = emb_mex('loglik_tracks', h, init_bins, bins, T, correct_dbn)
+        //   init_bins: n x n_initial int8; bins: the tiled int8 array of 'sample_tracks'
+        const int64_t n = (int64_t)mxGetM(prhs[2]);
+        if ((int64_t)mxGetNumberOfElements(prhs[2]) != n * ni) mexErrMsgIdAndTxt("emb200:arg", "init_bins must be an int8 n x n_initial matrix");
+        const int32_t T = (int32_t)mxGetScalar(prhs[4]);
+        if ((int64_t)mxGetNumberOfElements(prhs[3]) != emb_tracks_bins_len(m, n, T))
+            mexErrMsgIdAndTxt("emb200:arg", "bins must be the tiled array of n tracks x T seconds");
+        emb_sample_opts o;
+        emb_sample_opts_init(&o);
+        o.correct_dbn = nrhs > 5 ? (int32_t)mxGetScalar(prhs[5]) : 0;
+        plhs[0] = mxCreateDoubleMatrix(n, 1, mxREAL);
+        mxArray* tr = mxCreateDoubleMatrix(n, 1, mxREAL);
+        CHECK(emb_loglik_tracks(m, n, T, (const int8_t*)mxGetData(prhs[2]), (const int8_t*)mxGetData(prhs[3]), &o,
+                                mxGetPr(plhs[0]), mxGetPr(tr)));
+        if (nlhs > 1) plhs[1] = tr; else mxDestroyArray(tr);
+    } else if (c == "sample_tracks_multi") {                    // every GPU of the box from one MATLAB process (SURVEY 8e)
         // [out_inits, bins, values, hist_initial, hist_transition] = emb_mex('sample_tracks_multi', h, seed, first, n, T, opts, n_devices)
         // out_inits n x n_initial; bins / values: 1 x D cells of the per-device tiled arrays (shard d = emb_shard_range(n, d, D))
         emb_rng rng{(uint64_t)mxGetScalar(prhs[2]), (uint64_t)mxGetScalar(prhs[3])};
