@@ -51,34 +51,38 @@ int cuda_fail(cudaError_t e, const char* what) {
         if (e__ != cudaSuccess) return cuda_fail(e__, #call); \
     } while (0)
 
+// Frees the tables of a model held on the current device.
+void release(HostModel::DeviceCopy& c) {
+    for (void* p : {(void*)c.thr_initial, (void*)c.thr_transition, (void*)c.edges, (void*)c.dd32, (void*)c.logp_initial,
+                    (void*)c.logp_transition})
+        if (p) cudaFree(p);
+    c = HostModel::DeviceCopy{};
+}
+
+// One model table to the current device; an empty table stays nullptr, and a failed copy frees what it allocated.
+template <class T>
+int upload(const std::vector<T>& table, T** dst) {
+    *dst = nullptr;
+    if (table.empty()) return 0;
+    CU(cudaMalloc((void**)dst, table.size() * sizeof(T)));
+    const cudaError_t e = cudaMemcpy(*dst, table.data(), table.size() * sizeof(T), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) return 0;
+    cudaFree(*dst);
+    *dst = nullptr;
+    return cuda_fail(e, "cudaMemcpy (model table to the device)");
+}
+
 // Upload (or refresh after emb_set_prior) the packed tables of a model to `device`.
 int ensure_device(const HostModel& H, int device, DevModel& D) {
     std::lock_guard<std::mutex> lk(H.mu);
     auto& c = H.device_copies[device];
     if (c.version != H.version) {
-        if (c.thr_initial) cudaFree(c.thr_initial);
-        if (c.thr_transition) cudaFree(c.thr_transition);
-        if (c.edges) cudaFree(c.edges);
-        if (c.dd32) cudaFree(c.dd32);
-        if (c.logp_initial) cudaFree(c.logp_initial);
-        if (c.logp_transition) cudaFree(c.logp_transition);
-        c.logp_initial = c.logp_transition = nullptr;
-        c.logp_ok = false;
-        c.thr_initial = c.thr_transition = nullptr;
-        c.edges = nullptr;
-        c.dd32 = nullptr;
-        auto up = [&](const void* src, size_t bytes, void** dst) -> int {
-            *dst = nullptr;
-            if (!bytes) return 0;
-            CU(cudaMalloc(dst, bytes));
-            CU(cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice));
-            return 0;
-        };
+        release(c);
         int rc;
-        if ((rc = up(H.thr_initial.data(), H.thr_initial.size() * 4, (void**)&c.thr_initial))) return rc;
-        if ((rc = up(H.thr_transition.data(), H.thr_transition.size() * 4, (void**)&c.thr_transition))) return rc;
-        if ((rc = up(H.edges.data(), H.edges.size() * 8, (void**)&c.edges))) return rc;
-        if ((rc = up(H.dd32.data(), H.dd32.size() * 4, (void**)&c.dd32))) return rc;
+        if ((rc = upload(H.thr_initial, &c.thr_initial))) return rc;
+        if ((rc = upload(H.thr_transition, &c.thr_transition))) return rc;
+        if ((rc = upload(H.edges, &c.edges))) return rc;
+        if ((rc = upload(H.dd32, &c.dd32))) return rc;
         c.version = H.version;
     }
     D = H.dev;
@@ -97,11 +101,12 @@ int ensure_logp(const HostModel& H, int device, DevModel& D) {
     std::lock_guard<std::mutex> lk(H.mu);
     auto& c = H.device_copies[device];
     if (!c.logp_ok) {
-        for (auto* t : {&H.logp_initial, &H.logp_transition}) {
-            double*& dst = t == &H.logp_initial ? c.logp_initial : c.logp_transition;
-            if (t->empty()) continue;
-            CU(cudaMalloc((void**)&dst, t->size() * 8));
-            CU(cudaMemcpy(dst, t->data(), t->size() * 8, cudaMemcpyHostToDevice));
+        int rc;
+        if ((rc = upload(H.logp_initial, &c.logp_initial))) return rc;
+        if ((rc = upload(H.logp_transition, &c.logp_transition))) {
+            cudaFree(c.logp_initial);
+            c.logp_initial = nullptr;
+            return rc;
         }
         c.logp_ok = true;
     }
@@ -168,6 +173,11 @@ thread_local cudaStream_t g_call_stream = nullptr;   // the caller's stream of t
 void tmp_free(void* p) {
     if (p) cudaFreeAsync(p, g_call_stream);
 }
+// a per-call temporary, released when the entry point returns
+struct Tmp {
+    void* p = nullptr;
+    ~Tmp() { tmp_free(p); }
+};
 
 struct Staged {
     void* host = nullptr;
@@ -243,6 +253,84 @@ int status_error(int32_t status) {
         return set_err(EMB_E_ARG, "Attempt to preset a dependent variable (or a preset bin out of range) in start_per_sample");
     if (status) return set_err(EMB_E_REJECT, "a sample exhausted max_attempts in the rejection loop");
     return 0;
+}
+
+// One launching call, opened once its arguments are checked: the device, the model's device tables, the caller's stream,
+// the staging of host buffers and the status word of the launch.
+struct Call {
+    int device = 0;
+    bool async = false;   // EMB_MEM_ASYNC: enqueue only
+    DevModel D{};
+    cudaStream_t st = nullptr;
+    Stager sg{EMB_MEM_HOST, nullptr, {}};
+    Tmp word;
+
+    // Checks o->mem, picks the device, uploads the tables of H (if given; with the scoring tables if logp) and binds the
+    // caller's stream.
+    int open(const emb_sample_opts* o, const HostModel* H, bool allow_async = false, bool logp = false) {
+        int rc = pick_device(o, device, allow_async);
+        if (rc) return rc;
+        if (H) {
+            if ((rc = logp ? ensure_logp(*H, device, D) : ensure_device(*H, device, D))) return rc;
+            if (o->correct_dbn) D.fast = 0;   // parents re-evaluated every second (emb_sample_opts::correct_dbn)
+        }
+        async = (o->mem & EMB_MEM_ASYNC) != 0;
+        st = (cudaStream_t)o->stream;
+        g_call_stream = st;
+        sg.mem = o->mem & 0xFF;
+        sg.stream = st;
+        return 0;
+    }
+    // The zeroed status word of the launch: a per-call temporary, or on the EMB_MEM_ASYNC path the persistent word of the
+    // device that emb_async_status reads.
+    int status_word(int32_t** out) {
+        if (async) return async_status_word(device, out);
+        CU(tmp_alloc(&word.p, 4, st));
+        CU(cudaMemsetAsync(word.p, 0, 4, st));
+        *out = (int32_t*)word.p;
+        return 0;
+    }
+    // After the launch of `kernel`: its error; unless async, the status word to `status`, the wait and the staged outputs.
+    int finish(cudaError_t launched, const char* kernel, int32_t& status) {
+        status = 0;
+        if (launched != cudaSuccess) return cuda_fail(launched, ("launch " + std::string(kernel)).c_str());
+        if (async) return 0;
+        cudaError_t e = cudaMemcpyAsync(&status, word.p, 4, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        if (e != cudaSuccess) return cuda_fail(e, kernel);
+        return sg.finish();
+    }
+};
+
+int sample_params(const HostModel& H, const emb_rng* rng, int64_t n, int32_t T, const emb_sample_opts* o,
+                  emb::SampleParams& P) {
+    try {
+        emb::fill_params(H, rng->seed, rng->first_sample, n, T, *o, P);
+    } catch (const emb::Error& e) {
+        return set_err(e.code, e.msg);
+    }
+    return 0;
+}
+int need_transition(const HostModel& H) {
+    if (!H.has_transition || H.temporal_map.empty()) return set_err(EMB_E_ARG, "dynvar:empty: model has no transition network");
+    return 0;
+}
+int check_stream_index(const HostModel& H, int32_t T) {
+    if ((int64_t)T * (int64_t)H.gated.size() >= (1ll << 33)) return set_err(EMB_E_LIMIT, "T too large for the 32-bit stream index");
+    return 0;
+}
+
+// the caller's emb_track_out -> device pointers of a TrackOut (nullptr where the caller passed none)
+int stage_track_out(Stager& sg, const emb_model* m, int64_t n, int32_t T, const emb_track_out& out, emb::TrackOut& O) {
+    const size_t ni = (size_t)m->h->n_initial;
+    int rc;
+    if ((rc = sg.out(out.bins, (size_t)emb_tracks_bins_len(m, n, T), false, (void**)&O.bins))) return rc;
+    if ((rc = sg.out(out.values, (size_t)emb_tracks_values_len(m, n, T) * 4, false, (void**)&O.values))) return rc;
+    if ((rc = sg.out(out.init_bins, (size_t)n * ni, false, (void**)&O.init_bins))) return rc;
+    if ((rc = sg.out(out.init_values, (size_t)n * ni * 8, false, (void**)&O.init_values))) return rc;
+    if ((rc = sg.out(out.attempts, (size_t)n * 2, false, (void**)&O.attempts))) return rc;
+    if ((rc = sg.out(out.hist_initial, ni * 64 * 8, true, (void**)&O.hist_initial))) return rc;
+    return sg.out(out.hist_transition, m->h->temporal_map.size() * 64 * 8, true, (void**)&O.hist_transition);
 }
 
 template <class T>
@@ -396,12 +484,7 @@ void emb_model_free(emb_model* m) {
         for (auto& kv : m->h->device_copies) {
             int cur = 0;
             if (cudaGetDevice(&cur) == cudaSuccess && cudaSetDevice(kv.first) == cudaSuccess) {
-                if (kv.second.thr_initial) cudaFree(kv.second.thr_initial);
-                if (kv.second.thr_transition) cudaFree(kv.second.thr_transition);
-                if (kv.second.edges) cudaFree(kv.second.edges);
-                if (kv.second.dd32) cudaFree(kv.second.dd32);
-                if (kv.second.logp_initial) cudaFree(kv.second.logp_initial);
-                if (kv.second.logp_transition) cudaFree(kv.second.logp_transition);
+                release(kv.second);
                 cudaSetDevice(cur);
             }
         }
@@ -522,56 +605,27 @@ static int sample_initial_impl(const emb_model* m, const emb_rng* rng, int64_t n
     if (!m || !rng || !opts || n < 0) return set_err(EMB_E_ARG, "null or negative argument");
     const HostModel& H = *m->h;
     emb::SampleParams P;
-    int rc = 0;
-    try {
-        emb::fill_params(H, rng->seed, rng->first_sample, n, 0, *opts, P);
-    } catch (const emb::Error& e) {
-        return set_err(e.code, e.msg);
-    }
-    if (n == 0) return 0;
-    int device;
-    if ((rc = pick_device(opts, device, true))) return rc;
-    DevModel D;
-    if ((rc = ensure_device(H, device, D))) return rc;
-    cudaStream_t st = (cudaStream_t)opts->stream;
-    g_call_stream = st;
-    const int tw = (int)H.thr_initial.size();
-    auto launch = [&](int8_t* b, double* v64, float* v32, uint16_t* a, int32_t* word) {
-        return v32 ? (cudaError_t)emb::launch_initial_f32(D, P, tw, b, v32, a, nullptr, word, st)
-                   : (cudaError_t)emb::launch_initial(D, P, tw, b, v64, a, nullptr, word, st);
-    };
-    P.start_ps = opts->start_per_sample;   // device pointer in the enqueue-only path; staged below otherwise
-    P.start_stride = n;
-    if (opts->mem & EMB_MEM_ASYNC) {   // enqueue only (device buffers): see emb_sample_tracks
-        int32_t* word = nullptr;
-        if ((rc = async_status_word(device, &word))) return rc;
-        const cudaError_t ea = launch(bins, values64, values32, attempts, word);
-        return ea == cudaSuccess ? 0 : cuda_fail(ea, "launch k_initial");
-    }
-    Stager sg{opts->mem, st, {}};
+    int rc = sample_params(H, rng, n, 0, opts, P);
+    if (rc || n == 0) return rc;
+    Call call;
+    if ((rc = call.open(opts, &H, true))) return rc;
+    // with EMB_MEM_ASYNC (device buffers) nothing below is staged: the call only enqueues, see emb_sample_tracks
     int8_t* d_bins;
     double* d_v64;
     float* d_v32;
     uint16_t* d_att;
-    if ((rc = sg.out(bins, (size_t)n * H.n_initial, false, (void**)&d_bins))) return rc;
-    if ((rc = sg.out(values64, (size_t)n * H.n_initial * 8, false, (void**)&d_v64))) return rc;
-    if ((rc = sg.out(values32, (size_t)n * H.n_initial * 4, false, (void**)&d_v32))) return rc;
-    if ((rc = sg.out(attempts, (size_t)n * 2, false, (void**)&d_att))) return rc;
-    if ((rc = stage_start(sg, opts, H, n, P))) return rc;
-    int32_t* d_status = nullptr;
-    CU(tmp_alloc((void**)&d_status, 4, st));
-    CU(cudaMemsetAsync(d_status, 0, 4, st));
-    cudaError_t e = launch(d_bins, d_v64, d_v32, d_att, d_status);
-    if (e != cudaSuccess) {
-        tmp_free(d_status);
-        return cuda_fail(e, "launch k_initial");
-    }
-    int32_t status = 0;
-    e = cudaMemcpyAsync(&status, d_status, 4, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    tmp_free(d_status);
-    if (e != cudaSuccess) return cuda_fail(e, "k_initial");
-    if ((rc = sg.finish())) return rc;
+    int32_t* d_status;
+    if ((rc = call.sg.out(bins, (size_t)n * H.n_initial, false, (void**)&d_bins))) return rc;
+    if ((rc = call.sg.out(values64, (size_t)n * H.n_initial * 8, false, (void**)&d_v64))) return rc;
+    if ((rc = call.sg.out(values32, (size_t)n * H.n_initial * 4, false, (void**)&d_v32))) return rc;
+    if ((rc = call.sg.out(attempts, (size_t)n * 2, false, (void**)&d_att))) return rc;
+    if ((rc = stage_start(call.sg, opts, H, n, P))) return rc;
+    if ((rc = call.status_word(&d_status))) return rc;
+    const int tw = (int)H.thr_initial.size();
+    const cudaError_t e = values32 ? (cudaError_t)emb::launch_initial_f32(call.D, P, tw, d_bins, d_v32, d_att, nullptr, d_status, call.st)
+                                   : (cudaError_t)emb::launch_initial(call.D, P, tw, d_bins, d_v64, d_att, nullptr, d_status, call.st);
+    int32_t status;
+    if ((rc = call.finish(e, "k_initial", status))) return rc;
     return status_error(status);
 }
 
@@ -600,59 +654,24 @@ int emb_sample_tracks(const emb_model* m, const emb_rng* rng, int64_t n, int32_t
                       const emb_track_out* out) {
     if (!m || !rng || !opts || !out || n < 0 || T < 1) return set_err(EMB_E_ARG, "null or out-of-range argument");
     const HostModel& H = *m->h;
-    if (!H.has_transition || H.temporal_map.empty())
-        return set_err(EMB_E_ARG, "dynvar:empty: model has no transition network");
-    if ((int64_t)T * (int64_t)H.gated.size() >= (1ll << 33))
-        return set_err(EMB_E_LIMIT, "T too large for the 32-bit stream index");
+    int rc;
+    if ((rc = need_transition(H))) return rc;
+    if ((rc = check_stream_index(H, T))) return rc;
     emb::SampleParams P;
-    int rc = 0;
-    try {
-        emb::fill_params(H, rng->seed, rng->first_sample, n, T, *opts, P);
-    } catch (const emb::Error& e) {
-        return set_err(e.code, e.msg);
-    }
-    if (n == 0) return 0;
-    int device;
-    if ((rc = pick_device(opts, device, true))) return rc;
-    DevModel D;
-    if ((rc = ensure_device(H, device, D))) return rc;
-    if (opts->correct_dbn) D.fast = 0;      // parents re-evaluated every second (emb_sample_opts::correct_dbn)
-    cudaStream_t st = (cudaStream_t)opts->stream;
-    g_call_stream = st;
-    const bool async = (opts->mem & EMB_MEM_ASYNC) != 0;
-    Stager sg{opts->mem & 0xFF, st, {}};
-    emb::TrackOut O{};
-    const size_t ni = (size_t)H.n_initial;
-    if ((rc = sg.out(out->bins, (size_t)emb_tracks_bins_len(m, n, T), false, (void**)&O.bins))) return rc;
-    if ((rc = sg.out(out->values, (size_t)emb_tracks_values_len(m, n, T) * 4, false, (void**)&O.values))) return rc;
-    if ((rc = sg.out(out->init_bins, (size_t)n * ni, false, (void**)&O.init_bins))) return rc;
-    if ((rc = sg.out(out->init_values, (size_t)n * ni * 8, false, (void**)&O.init_values))) return rc;
-    if ((rc = sg.out(out->attempts, (size_t)n * 2, false, (void**)&O.attempts))) return rc;
+    if ((rc = sample_params(H, rng, n, T, opts, P)) || n == 0) return rc;
     if (out->hist_initial || out->hist_transition) {   // the histograms have 64 counters per variable
         for (int i = 0; i < H.n_initial; ++i)
             if (H.r_initial[i] > 64) return set_err(EMB_E_LIMIT, "verification histograms hold 64 bins per variable; this model has a variable with more");
     }
-    if ((rc = sg.out(out->hist_initial, ni * 64 * 8, true, (void**)&O.hist_initial))) return rc;
-    if ((rc = sg.out(out->hist_transition, H.temporal_map.size() * 64 * 8, true, (void**)&O.hist_transition))) return rc;
-    if ((rc = stage_start(sg, opts, H, n, P))) return rc;
-    if (async) {   // enqueue only: no host round trip between consecutive passes; emb_async_status collects the flag
-        if ((rc = async_status_word(device, &O.status))) return rc;
-        const cudaError_t ea = (cudaError_t)emb::launch_tracks(D, P, O, st);
-        return ea == cudaSuccess ? 0 : cuda_fail(ea, "launch k_tracks");
-    }
-    CU(tmp_alloc((void**)&O.status, 4, st));
-    CU(cudaMemsetAsync(O.status, 0, 4, st));
-    cudaError_t e = (cudaError_t)emb::launch_tracks(D, P, O, st);
-    if (e != cudaSuccess) {
-        tmp_free(O.status);
-        return cuda_fail(e, "launch k_tracks");
-    }
-    int32_t status = 0;
-    e = cudaMemcpyAsync(&status, O.status, 4, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    tmp_free(O.status);
-    if (e != cudaSuccess) return cuda_fail(e, "k_tracks");
-    if ((rc = sg.finish())) return rc;
+    Call call;
+    if ((rc = call.open(opts, &H, true))) return rc;
+    // EMB_MEM_ASYNC: enqueue only, no host round trip between consecutive passes; emb_async_status collects the flag
+    emb::TrackOut O{};
+    if ((rc = stage_track_out(call.sg, m, n, T, *out, O))) return rc;
+    if ((rc = stage_start(call.sg, opts, H, n, P))) return rc;
+    if ((rc = call.status_word(&O.status))) return rc;
+    int32_t status;
+    if ((rc = call.finish((cudaError_t)emb::launch_tracks(call.D, P, O, call.st), "k_tracks", status))) return rc;
     return status_error(status);
 }
 
@@ -681,8 +700,8 @@ static int sample_events_impl(const emb_model* m, const emb_rng* rng, int64_t n,
     if (init && (init->bins || init->values || init->hist_initial || init->hist_transition))
         return set_err(EMB_E_ARG, "emb_sample_track_events: dense outputs and histograms belong to emb_sample_tracks");
     const HostModel& H = *m->h;
-    if (!H.has_transition || H.temporal_map.empty())
-        return set_err(EMB_E_ARG, "dynvar:empty: model has no transition network");
+    int rc;
+    if ((rc = need_transition(H))) return rc;
     int max_bins = 0;
     for (int v : H.gated) max_bins = std::max(max_bins, (int)H.r_initial[v]);
     emb::EventFormat fm{};
@@ -691,19 +710,12 @@ static int sample_events_impl(const emb_model* m, const emb_rng* rng, int64_t n,
     if (packed && (fm.gord_bits != 3 || fm.dt_bytes != 1))
         return set_err(EMB_E_LIMIT, "packed event rows need <= 7 time-varying variables and T <= 1023 (use emb_sample_track_events)");
     emb::SampleParams P;
-    int rc = 0;
-    try {
-        emb::fill_params(H, rng->seed, rng->first_sample, n, T, *opts, P);
-    } catch (const emb::Error& e) {
-        return set_err(e.code, e.msg);
-    }
-    int device;
-    if ((rc = pick_device(opts, device))) return rc;
-    DevModel D;
-    if ((rc = ensure_device(H, device, D))) return rc;
-    if (opts->correct_dbn) D.fast = 0;
-    cudaStream_t st = (cudaStream_t)opts->stream;
-    g_call_stream = st;
+    if ((rc = sample_params(H, rng, n, T, opts, P))) return rc;
+    Call call;
+    if ((rc = call.open(opts, &H))) return rc;
+    DevModel& D = call.D;
+    const cudaStream_t st = call.st;
+    Stager& sg = call.sg;
     if (total_rows) *total_rows = 0;
     if (n == 0) {
         const int64_t zero = 0;
@@ -712,28 +724,19 @@ static int sample_events_impl(const emb_model* m, const emb_rng* rng, int64_t n,
         return 0;
     }
     PhaseTrace tr;
-    Stager sg{opts->mem, st, {}};
-    const size_t ni = (size_t)H.n_initial;
     emb::TrackOut O{};
     O.ev_gord_bits = fm.gord_bits;
     O.ev_dt_bytes = fm.dt_bytes;
     long long* d_off = nullptr;
     if ((rc = sg.out(offsets, (size_t)(n + 1) * 8, false, (void**)&d_off))) return rc;
-    if (init) {
-        if ((rc = sg.out(init->init_bins, (size_t)n * ni, false, (void**)&O.init_bins))) return rc;
-        if ((rc = sg.out(init->init_values, (size_t)n * ni * 8, false, (void**)&O.init_values))) return rc;
-        if ((rc = sg.out(init->attempts, (size_t)n * 2, false, (void**)&O.attempts))) return rc;
-    }
+    if ((rc = stage_track_out(sg, m, n, T, init ? *init : emb_track_out{}, O))) return rc;   // dense and histograms refused above
     if ((rc = stage_start(sg, opts, H, n, P))) return rc;
-    struct Scratch {
-        void* p = nullptr;
-        ~Scratch() { tmp_free(p); }
-    } counts, status, tiles, pw, pd;
+    Tmp counts, tiles, pw, pd;
     CU(tmp_alloc(&counts.p, (size_t)n * 4, st));
     CU(tmp_alloc(&tiles.p, (size_t)emb::scan_scratch_len(n) * 8, st));
-    CU(tmp_alloc(&status.p, 4, st));
-    CU(cudaMemsetAsync(status.p, 0, 4, st));
-    O.status = (int32_t*)status.p;
+    int32_t* status;
+    if ((rc = call.status_word(&status))) return rc;
+    O.status = status;
     const bool host = (opts->mem & 0xFF) == EMB_MEM_HOST;
     const bool pipelined = host && n >= 8192;
     if (!pipelined) {
@@ -746,7 +749,7 @@ static int sample_events_impl(const emb_model* m, const emb_rng* rng, int64_t n,
         long long total = 0;
         int32_t flag = 0;
         CU(cudaMemcpyAsync(&total, d_off + n, 8, cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(&flag, status.p, 4, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(&flag, status, 4, cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         tr.mark("alloc + count pass + scan");
         if (total_rows) *total_rows = total;
@@ -790,7 +793,7 @@ static int sample_events_impl(const emb_model* m, const emb_rng* rng, int64_t n,
     // of the finished chunks to the host (rows of a track range are contiguous: [offsets[a], offsets[b])).  Only the first
     // chunk's count pass is not hidden behind a copy.
     struct Guard {
-        void* rows = nullptr;       // 8-byte rows (legacy entry point only)
+        Tmp rows;                   // 8-byte rows (legacy entry point only), released after the copy stream is drained
         cudaStream_t copy = nullptr;
         cudaEvent_t done[16] = {};
         ~Guard() {
@@ -799,13 +802,12 @@ static int sample_events_impl(const emb_model* m, const emb_rng* rng, int64_t n,
                 cudaStreamSynchronize(copy);
                 cudaStreamDestroy(copy);
             }
-            tmp_free(rows);
         }
     } g;
     if (capacity > 0) {
         CU(tmp_alloc(&pw.p, (size_t)capacity * 4, st));
         CU(tmp_alloc(&pd.p, (size_t)capacity * fm.dt_bytes, st));
-        if (!packed) CU(tmp_alloc(&g.rows, (size_t)capacity * 8, st));
+        if (!packed) CU(tmp_alloc(&g.rows.p, (size_t)capacity * 8, st));
     }
     CU(cudaStreamCreateWithFlags(&g.copy, cudaStreamNonBlocking));
     CU(cudaMemsetAsync(d_off, 0, 8, st));                 // carry of the first chunk
@@ -835,7 +837,7 @@ static int sample_events_impl(const emb_model* m, const emb_rng* rng, int64_t n,
         if (e != cudaSuccess) return cuda_fail(e, "launch k_scan_counts");
         // the chunk's running total and the rejection flag reach the host through mapped memory (an SM store): a cudaMemcpy
         // would queue on the copy engine behind the previous chunk's rows and serialise the pipeline
-        e = (cudaError_t)emb::launch_publish(d_off + b, (const int32_t*)status.p, pub + 2 * c, st);
+        e = (cudaError_t)emb::launch_publish(d_off + b, status, pub + 2 * c, st);
         if (e != cudaSuccess) return cuda_fail(e, "launch k_publish");
         CU(cudaStreamSynchronize(st));
         const long long r0 = total, r1 = pub[2 * c];
@@ -858,7 +860,7 @@ static int sample_events_impl(const emb_model* m, const emb_rng* rng, int64_t n,
         e = (cudaError_t)emb::launch_tracks(D, Pc, Ow, st);
         if (e != cudaSuccess) return cuda_fail(e, "launch k_tracks (event write)");
         if (!packed) {
-            e = (cudaError_t)emb::launch_expand_events(D, (const uint32_t*)pw.p, (const uint8_t*)pd.p, g.rows, r0, r1 - r0, fm, st);
+            e = (cudaError_t)emb::launch_expand_events(D, (const uint32_t*)pw.p, (const uint8_t*)pd.p, g.rows.p, r0, r1 - r0, fm, st);
             if (e != cudaSuccess) return cuda_fail(e, "launch k_expand_events");
         }
         CU(cudaEventCreateWithFlags(&g.done[c], cudaEventDisableTiming));
@@ -868,7 +870,7 @@ static int sample_events_impl(const emb_model* m, const emb_rng* rng, int64_t n,
             CU(cudaMemcpyAsync(words + r0, (const uint32_t*)pw.p + r0, (size_t)(r1 - r0) * 4, cudaMemcpyDeviceToHost, g.copy));
             CU(cudaMemcpyAsync(dts + r0, (const uint8_t*)pd.p + r0, (size_t)(r1 - r0), cudaMemcpyDeviceToHost, g.copy));
         } else {
-            CU(cudaMemcpyAsync(events + r0, (const char*)g.rows + (size_t)r0 * 8, (size_t)(r1 - r0) * 8, cudaMemcpyDeviceToHost, g.copy));
+            CU(cudaMemcpyAsync(events + r0, (const char*)g.rows.p + (size_t)r0 * 8, (size_t)(r1 - r0) * 8, cudaMemcpyDeviceToHost, g.copy));
         }
     }
     tr.mark("chunks enqueued");
@@ -955,44 +957,28 @@ int emb_terminal_propagate(const emb_terminal_models* models, const emb_rng* rng
         return set_err(e.code, e.msg);
     }
     if (n == 0) return 0;
-    int device, rc = 0;
-    if ((rc = pick_device(opts, device))) return rc;
+    Call call;
+    int rc;
+    if ((rc = call.open(opts, nullptr))) return rc;
     for (int k = 0; k < emb::TERM_NMODELS; ++k) {
         DevModel D;
-        if ((rc = ensure_device(*slot[k]->h, device, D))) return rc;
+        if ((rc = ensure_device(*slot[k]->h, call.device, D))) return rc;
         P.m[k].thr = D.thr_trans;
         P.m[k].edges = D.edges;
     }
-    cudaStream_t st = (cudaStream_t)opts->stream;
-    g_call_stream = st;
-    Stager sg{opts->mem, st, {}};
-    struct Scratch {
-        void* p = nullptr;
-        ~Scratch() { tmp_free(p); }
-    } d_geo, d_status, d_cuts;
-    CU(tmp_alloc(&d_cuts.p, cuts.size() * 8, st));
-    CU(cudaMemcpyAsync(d_cuts.p, cuts.data(), cuts.size() * 8, cudaMemcpyHostToDevice, st));   // pageable: staged before return
+    Tmp d_cuts;
+    CU(tmp_alloc(&d_cuts.p, cuts.size() * 8, call.st));
+    CU(cudaMemcpyAsync(d_cuts.p, cuts.data(), cuts.size() * 8, cudaMemcpyHostToDevice, call.st));   // pageable: staged before return
     P.cuts = (const double*)d_cuts.p;
-    if (opts->mem == EMB_MEM_DEVICE) {
-        P.geo = geo;
-    } else {   // stage the rows that are read
-        const size_t bytes = (size_t)(max_row + 1) * (size_t)geo_stride * 8;
-        CU(tmp_alloc(&d_geo.p, bytes, st));
-        CU(cudaMemcpyAsync(d_geo.p, geo, bytes, cudaMemcpyHostToDevice, st));
-        P.geo = (const double*)d_geo.p;
-    }
+    const void* d_geo;
+    if ((rc = call.sg.in(geo, (size_t)(max_row + 1) * (size_t)geo_stride * 8, &d_geo))) return rc;   // the rows that are read
+    P.geo = (const double*)d_geo;
     emb::TermOut O{};
-    if ((rc = sg.out(out->traj, (size_t)emb_terminal_traj_len(n, tmax_s) * 4, false, (void**)&O.traj))) return rc;
-    if ((rc = sg.out(out->len, (size_t)n * 4 * 2, false, (void**)&O.len))) return rc;
-    CU(tmp_alloc(&d_status.p, 4, st));
-    CU(cudaMemsetAsync(d_status.p, 0, 4, st));
-    O.status = (int32_t*)d_status.p;
-    cudaError_t e = (cudaError_t)emb::launch_terminal(P, O, st);
-    if (e != cudaSuccess) return cuda_fail(e, "launch k_terminal_chains");
-    int32_t status = 0;
-    CU(cudaMemcpyAsync(&status, d_status.p, 4, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    if ((rc = sg.finish())) return rc;
+    if ((rc = call.sg.out(out->traj, (size_t)emb_terminal_traj_len(n, tmax_s) * 4, false, (void**)&O.traj))) return rc;
+    if ((rc = call.sg.out(out->len, (size_t)n * 4 * 2, false, (void**)&O.len))) return rc;
+    if ((rc = call.status_word(&O.status))) return rc;
+    int32_t status;
+    if ((rc = call.finish((cudaError_t)emb::launch_terminal(P, O, call.st), "k_terminal_chains", status))) return rc;
     if (status & 2) return set_err(EMB_E_ARG, "Unknown int_intent: own_intent must be 1..2 and int_intent 1..3 (createEncounter.m:22,37)");
     if (status & 1) return set_err(EMB_E_REJECT, "a trajectory state exhausted max_attempts in the dynamic-limit resample loop");
     return 0;
@@ -1014,40 +1000,26 @@ static int loglik_impl(const emb_model* m, int64_t n, int32_t T, const int8_t* i
     const HostModel& H = *m->h;
     if (opts->mem & ~0xFF) return set_err(EMB_E_ARG, "loglik: EMB_MEM_ASYNC is not supported; scoring calls are synchronous");
     if (n == 0) return 0;
-    int device, rc = 0;
-    if ((rc = pick_device(opts, device))) return rc;
-    DevModel D;
-    if ((rc = ensure_logp(H, device, D))) return rc;
-    if (opts->correct_dbn) D.fast = 0;
-    cudaStream_t st = (cudaStream_t)opts->stream;
-    g_call_stream = st;
-    Stager sg{opts->mem, st, {}};
+    Call call;
+    int rc;
+    if ((rc = call.open(opts, &H, false, true))) return rc;
     const size_t ni = (size_t)H.n_initial;
     emb::LoglikParams P{};
     P.n = n;
     P.T = T;
     const void* d_in = nullptr;
-    if ((rc = sg.in(init_bins, (size_t)n * ni, &d_in))) return rc;
+    if ((rc = call.sg.in(init_bins, (size_t)n * ni, &d_in))) return rc;
     P.init_bins = (const int8_t*)d_in;
-    if (tracks && (rc = sg.in(bins, (size_t)emb_tracks_bins_len(m, n, T), &d_in))) return rc;
+    if (tracks && (rc = call.sg.in(bins, (size_t)emb_tracks_bins_len(m, n, T), &d_in))) return rc;
     P.bins = tracks ? (const int8_t*)d_in : nullptr;
-    if ((rc = sg.out(initial, (size_t)n * 8, false, (void**)&P.initial))) return rc;
-    if ((rc = sg.out(per_var, (size_t)n * ni * 8, false, (void**)&P.per_var))) return rc;
-    if ((rc = sg.out(transition, (size_t)n * 8, false, (void**)&P.transition))) return rc;
-    CU(tmp_alloc((void**)&P.status, 4, st));
-    CU(cudaMemsetAsync(P.status, 0, 4, st));
-    cudaError_t e = tracks ? (cudaError_t)emb::launch_loglik_tracks(D, P, st)
-                           : (cudaError_t)emb::launch_loglik_initial(D, P, (int)H.logp_initial.size(), st);
-    if (e != cudaSuccess) {
-        tmp_free(P.status);
-        return cuda_fail(e, tracks ? "launch k_loglik_tracks" : "launch k_loglik_initial");
-    }
-    int32_t status = 0;
-    e = cudaMemcpyAsync(&status, P.status, 4, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    tmp_free(P.status);
-    if (e != cudaSuccess) return cuda_fail(e, tracks ? "k_loglik_tracks" : "k_loglik_initial");
-    if ((rc = sg.finish())) return rc;
+    if ((rc = call.sg.out(initial, (size_t)n * 8, false, (void**)&P.initial))) return rc;
+    if ((rc = call.sg.out(per_var, (size_t)n * ni * 8, false, (void**)&P.per_var))) return rc;
+    if ((rc = call.sg.out(transition, (size_t)n * 8, false, (void**)&P.transition))) return rc;
+    if ((rc = call.status_word(&P.status))) return rc;
+    const cudaError_t e = tracks ? (cudaError_t)emb::launch_loglik_tracks(call.D, P, call.st)
+                                 : (cudaError_t)emb::launch_loglik_initial(call.D, P, (int)H.logp_initial.size(), call.st);
+    int32_t status;
+    if ((rc = call.finish(e, tracks ? "k_loglik_tracks" : "k_loglik_initial", status))) return rc;
     return loglik_status_error(status);
 }
 
@@ -1061,9 +1033,7 @@ int emb_loglik_tracks(const emb_model* m, int64_t n, int32_t T, const int8_t* in
                       const emb_sample_opts* opts, double* initial, double* transition) {
     if (!m || !opts || n < 0 || T < 1 || (n > 0 && (!init_bins || !bins)))
         return set_err(EMB_E_ARG, "null or out-of-range argument");
-    const HostModel& H = *m->h;
-    if (!H.has_transition || H.temporal_map.empty())
-        return set_err(EMB_E_ARG, "dynvar:empty: model has no transition network");
+    if (int rc = need_transition(*m->h)) return rc;
     return loglik_impl(m, n, T, init_bins, bins, opts, initial, nullptr, transition);
 }
 
@@ -1095,6 +1065,12 @@ static int fill_integrate(const HostModel& H, const emb_integrate_opts* opts, in
     return 0;
 }
 
+// the integration constants of IntegrateParams, for the kernel that samples and integrates in one pass
+static emb::XyzOut xyz_out(const emb::IntegrateParams& P, float* xyz, uint8_t* is_good) {
+    return emb::XyzOut{xyz, is_good, P.g_acc, P.g_vr, P.g_turn, P.i_alt, P.i_speed,
+                       P.ur_speed, P.ur_vertrate, P.ur_heading, P.min_speed, P.max_speed};
+}
+
 int emb_tracks_integrate(const emb_model* m, int64_t n, int32_t T, const double* init_values, const float* values,
                          const emb_integrate_opts* opts, float* xyz, uint8_t* is_good) {
     if (!m || !opts || n < 0 || T < 1 || (n > 0 && (!init_values || !values)))
@@ -1103,37 +1079,25 @@ int emb_tracks_integrate(const emb_model* m, int64_t n, int32_t T, const double*
     emb::IntegrateParams P;
     if (int rcf = fill_integrate(H, opts, n, T, P)) return rcf;
     if (n == 0) return 0;
-    emb_sample_opts so;
+    emb_sample_opts so;   // device and stream; emb_integrate_opts.mem goes to the staging as given
     emb_sample_opts_init(&so);
     so.device = opts->device;
-    int device, rc = 0;
-    if ((rc = pick_device(&so, device))) return rc;
-    cudaStream_t st = (cudaStream_t)opts->stream;
-    g_call_stream = st;
-    Stager sg{opts->mem, st, {}};
-    struct Scratch {
-        void* p = nullptr;
-        ~Scratch() { tmp_free(p); }
-    } d_init, d_vals;
-    const size_t init_bytes = (size_t)H.n_initial * (size_t)n * 8;
-    const size_t val_bytes = (size_t)emb_tracks_values_len(m, n, T) * 4;
-    if (opts->mem == EMB_MEM_DEVICE) {
-        P.init_values = init_values;
-        P.values = values;
-    } else {
-        CU(tmp_alloc(&d_init.p, init_bytes, st));
-        CU(tmp_alloc(&d_vals.p, val_bytes, st));
-        CU(cudaMemcpyAsync(d_init.p, init_values, init_bytes, cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(d_vals.p, values, val_bytes, cudaMemcpyHostToDevice, st));
-        P.init_values = (const double*)d_init.p;
-        P.values = (const float*)d_vals.p;
-    }
-    if ((rc = sg.out(xyz, (size_t)3 * (size_t)(T + 1) * (size_t)n * 4, false, (void**)&P.xyz))) return rc;
-    if ((rc = sg.out(is_good, (size_t)n, false, (void**)&P.is_good))) return rc;
-    cudaError_t e = (cudaError_t)emb::launch_integrate(P, st);
+    so.stream = opts->stream;
+    Call call;
+    int rc;
+    if ((rc = call.open(&so, nullptr))) return rc;
+    call.sg.mem = opts->mem;
+    const void* d_in;
+    if ((rc = call.sg.in(init_values, (size_t)H.n_initial * (size_t)n * 8, &d_in))) return rc;
+    P.init_values = (const double*)d_in;
+    if ((rc = call.sg.in(values, (size_t)emb_tracks_values_len(m, n, T) * 4, &d_in))) return rc;
+    P.values = (const float*)d_in;
+    if ((rc = call.sg.out(xyz, (size_t)3 * (size_t)(T + 1) * (size_t)n * 4, false, (void**)&P.xyz))) return rc;
+    if ((rc = call.sg.out(is_good, (size_t)n, false, (void**)&P.is_good))) return rc;
+    cudaError_t e = (cudaError_t)emb::launch_integrate(P, call.st);
     if (e != cudaSuccess) return cuda_fail(e, "launch k_tracks_integrate");
-    CU(cudaStreamSynchronize(st));
-    return sg.finish();
+    CU(cudaStreamSynchronize(call.st));
+    return call.sg.finish();
 }
 
 int emb_sample_tracks_xyz(const emb_model* m, const emb_rng* rng, int64_t n, int32_t T, const emb_sample_opts* opts,
@@ -1143,52 +1107,28 @@ int emb_sample_tracks_xyz(const emb_model* m, const emb_rng* rng, int64_t n, int
         return set_err(EMB_E_ARG, "emb_sample_tracks_xyz: histograms belong to emb_sample_tracks");
     if (opts->mem & EMB_MEM_ASYNC) return set_err(EMB_E_ARG, "emb_sample_tracks_xyz: EMB_MEM_ASYNC is not supported");
     const HostModel& H = *m->h;
-    if (!H.has_transition || H.temporal_map.empty())
-        return set_err(EMB_E_ARG, "dynvar:empty: model has no transition network");
-    if ((int64_t)T * (int64_t)H.gated.size() >= (1ll << 33))
-        return set_err(EMB_E_LIMIT, "T too large for the 32-bit stream index");
+    int rc;
+    if ((rc = need_transition(H))) return rc;
+    if ((rc = check_stream_index(H, T))) return rc;
     emb::SampleParams P;
     emb::IntegrateParams IP;
-    int rc = 0;
-    try {
-        emb::fill_params(H, rng->seed, rng->first_sample, n, T, *opts, P);
-    } catch (const emb::Error& e) {
-        return set_err(e.code, e.msg);
-    }
-    if ((rc = fill_integrate(H, iopts, n, T, IP))) return rc;
-    if (n == 0) return 0;
-    int device;
-    if ((rc = pick_device(opts, device, true))) return rc;
-    DevModel D;
-    if ((rc = ensure_device(H, device, D))) return rc;
-    if (opts->correct_dbn) D.fast = 0;
-    cudaStream_t st = (cudaStream_t)opts->stream;
-    g_call_stream = st;
-    Stager sg{opts->mem & 0xFF, st, {}};
+    if ((rc = sample_params(H, rng, n, T, opts, P))) return rc;
+    if ((rc = fill_integrate(H, iopts, n, T, IP)) || n == 0) return rc;
+    if (!xyz && !is_good) return set_err(EMB_E_ARG, "emb_sample_tracks_xyz: xyz and is_good are both null");
+    Call call;
+    if ((rc = call.open(opts, &H))) return rc;
+    const cudaStream_t st = call.st;
     emb::TrackOut O{};
-    const size_t ni = (size_t)H.n_initial;
-    const emb_track_out none{};
-    const emb_track_out* o = out ? out : &none;
-    if ((rc = sg.out(o->bins, (size_t)emb_tracks_bins_len(m, n, T), false, (void**)&O.bins))) return rc;
-    if ((rc = sg.out(o->values, (size_t)emb_tracks_values_len(m, n, T) * 4, false, (void**)&O.values))) return rc;
-    if ((rc = sg.out(o->init_bins, (size_t)n * ni, false, (void**)&O.init_bins))) return rc;
-    if ((rc = sg.out(o->init_values, (size_t)n * ni * 8, false, (void**)&O.init_values))) return rc;
-    if ((rc = sg.out(o->attempts, (size_t)n * 2, false, (void**)&O.attempts))) return rc;
-    if ((rc = sg.out(xyz, (size_t)3 * (size_t)(T + 1) * (size_t)n * 4, false, (void**)&O.x.xyz))) return rc;
-    if ((rc = sg.out(is_good, (size_t)n, false, (void**)&O.x.is_good))) return rc;
-    if (!O.x.xyz && !O.x.is_good) return set_err(EMB_E_ARG, "emb_sample_tracks_xyz: xyz and is_good are both null");
-    O.x.g_acc = IP.g_acc; O.x.g_vr = IP.g_vr; O.x.g_turn = IP.g_turn; O.x.i_alt = IP.i_alt; O.x.i_speed = IP.i_speed;
-    O.x.ur_speed = IP.ur_speed; O.x.ur_vertrate = IP.ur_vertrate; O.x.ur_heading = IP.ur_heading;
-    O.x.min_speed = IP.min_speed; O.x.max_speed = IP.max_speed;
-    if ((rc = stage_start(sg, opts, H, n, P))) return rc;
-    struct Scratch {
-        void* p = nullptr;
-        ~Scratch() { tmp_free(p); }
-    } d_status, d_values, d_inits;
-    CU(tmp_alloc(&d_status.p, 4, st));
-    CU(cudaMemsetAsync(d_status.p, 0, 4, st));
-    O.status = (int32_t*)d_status.p;
-    int le = emb::launch_tracks(D, P, O, st);
+    if ((rc = stage_track_out(call.sg, m, n, T, out ? *out : emb_track_out{}, O))) return rc;   // histograms refused above
+    float* d_xyz;
+    uint8_t* d_good;
+    if ((rc = call.sg.out(xyz, (size_t)3 * (size_t)(T + 1) * (size_t)n * 4, false, (void**)&d_xyz))) return rc;
+    if ((rc = call.sg.out(is_good, (size_t)n, false, (void**)&d_good))) return rc;
+    O.x = xyz_out(IP, d_xyz, d_good);
+    if ((rc = stage_start(call.sg, opts, H, n, P))) return rc;
+    if ((rc = call.status_word(&O.status))) return rc;
+    Tmp d_values, d_inits;
+    int le = emb::launch_tracks(call.D, P, O, st);
     if (le == -1) {   // no fused kernel for this shape: sample the dense values (into a temporary if the caller wants none), then integrate
         emb::TrackOut O2 = O;
         O2.x = emb::XyzOut{};
@@ -1197,23 +1137,20 @@ int emb_sample_tracks_xyz(const emb_model* m, const emb_rng* rng, int64_t n, int
             O2.values = (float*)d_values.p;
         }
         if (!O2.init_values) {
-            CU(tmp_alloc(&d_inits.p, (size_t)n * ni * 8, st));
+            CU(tmp_alloc(&d_inits.p, (size_t)n * H.n_initial * 8, st));
             O2.init_values = (double*)d_inits.p;
         }
-        le = emb::launch_tracks(D, P, O2, st);
+        le = emb::launch_tracks(call.D, P, O2, st);
         if (le == 0) {
             IP.init_values = O2.init_values;
             IP.values = O2.values;
-            IP.xyz = O.x.xyz;
-            IP.is_good = O.x.is_good;
+            IP.xyz = d_xyz;
+            IP.is_good = d_good;
             le = emb::launch_integrate(IP, st);
         }
     }
-    if (le != 0) return cuda_fail((cudaError_t)le, "launch k_tracks (xyz)");
-    int32_t status = 0;
-    CU(cudaMemcpyAsync(&status, d_status.p, 4, cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    if ((rc = sg.finish())) return rc;
+    int32_t status;
+    if ((rc = call.finish((cudaError_t)le, "k_tracks (xyz)", status))) return rc;
     return status_error(status);
 }
 
@@ -1222,41 +1159,29 @@ int emb_terminal_screen(const float* traj, const int16_t* len, int64_t n, double
     if (!opts || !out || n < 0 || (n > 0 && (!traj || !len))) return set_err(EMB_E_ARG, "null or out-of-range argument");
     if (!(tmax_s >= 0.0) || tmax_s >= 32767.0) return set_err(EMB_E_ARG, "tmax_s must be in [0, 32767)");
     if (n == 0) return 0;
-    int device, rc = 0;
-    if ((rc = pick_device(opts, device))) return rc;
-    cudaStream_t st = (cudaStream_t)opts->stream;
-    g_call_stream = st;
+    Call call;
+    int rc;
+    if ((rc = call.open(opts, nullptr))) return rc;
     emb::ScreenParams P;
     std::memset(&P, 0, sizeof(P));
     P.n = n;
     P.tmax = (int32_t)tmax_s;
     P.thres_dist_ft = thres_dist_ft;
     P.thres_altlow_ft = thres_altlow_ft;
-    struct Scratch {
-        void* p = nullptr;
-        ~Scratch() { tmp_free(p); }
-    } d_traj, d_len;
-    const size_t tb = (size_t)emb_terminal_traj_len(n, tmax_s) * 4, lb = (size_t)n * 4 * 2;
-    if (opts->mem == EMB_MEM_DEVICE) {
-        P.traj = traj;
-        P.len = len;
-    } else {
-        CU(tmp_alloc(&d_traj.p, tb, st));
-        CU(tmp_alloc(&d_len.p, lb, st));
-        CU(cudaMemcpyAsync(d_traj.p, traj, tb, cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(d_len.p, len, lb, cudaMemcpyHostToDevice, st));
-        P.traj = (const float*)d_traj.p;
-        P.len = (const int16_t*)d_len.p;
-    }
-    Stager sg{opts->mem, st, {}};
+    Stager& sg = call.sg;
+    const void* d_in;
+    if ((rc = sg.in(traj, (size_t)emb_terminal_traj_len(n, tmax_s) * 4, &d_in))) return rc;
+    P.traj = (const float*)d_in;
+    if ((rc = sg.in(len, (size_t)n * 4 * 2, &d_in))) return rc;
+    P.len = (const int16_t*)d_in;
     if ((rc = sg.out(out->hmd_ft, (size_t)n * 8, false, (void**)&P.hmd_ft))) return rc;
     if ((rc = sg.out(out->vmd_ft, (size_t)n * 8, false, (void**)&P.vmd_ft))) return rc;
     if ((rc = sg.out(out->tcpa, (size_t)n * 3 * 2, false, (void**)&P.tcpa))) return rc;
     if ((rc = sg.out(out->enc_time_s, (size_t)n * 2, false, (void**)&P.enc_time_s))) return rc;
     if ((rc = sg.out(out->runway, (size_t)n, false, (void**)&P.runway))) return rc;
-    cudaError_t e = (cudaError_t)emb::launch_screen(P, st);
+    cudaError_t e = (cudaError_t)emb::launch_screen(P, call.st);
     if (e != cudaSuccess) return cuda_fail(e, "launch k_terminal_screen");
-    CU(cudaStreamSynchronize(st));
+    CU(cudaStreamSynchronize(call.st));
     return sg.finish();
 }
 
