@@ -162,6 +162,8 @@ def lib():
         "emb_tracks_values_len": (i64, [vp, i64, i32]),
         "emb_loglik_initial": (C.c_int, [vp, i64, vp, P(SampleOpts), vp, vp]),
         "emb_loglik_tracks": (C.c_int, [vp, i64, i32, vp, vp, P(SampleOpts), vp, vp]),
+        "emb_loglik_track_events": (C.c_int, [vp, i64, i32, vp, vp, vp, P(SampleOpts), vp, vp]),
+        "emb_loglik_track_events_packed": (C.c_int, [vp, i64, i32, vp, vp, vp, vp, P(SampleOpts), vp, vp]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)  # AttributeError if a declared symbol is missing
@@ -179,6 +181,7 @@ EXPORTED = [
     "emb_tracks_bins_len", "emb_tracks_values_len", "emb_sample_track_events",
     "emb_dyn_limits_named", "emb_terminal_propagate", "emb_terminal_traj_len", "emb_tracks_integrate", "emb_sample_tracks_xyz",
     "emb_terminal_screen", "emb_loglik_initial", "emb_loglik_tracks",
+    "emb_loglik_track_events", "emb_loglik_track_events_packed",
 ]
 TRAJ_FIELDS = ("x_nm", "y_nm", "z_ft", "heading_deg", "v_ft_s")
 

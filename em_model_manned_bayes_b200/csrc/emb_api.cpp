@@ -17,6 +17,7 @@
 #include "emb_integrate.cuh"
 #include "emb_launch.h"
 #include "emb_loglik.cuh"
+#include "emb_loglik_events.cuh"
 #include "emb_model.h"
 
 using emb::DevModel;
@@ -987,9 +988,14 @@ int emb_terminal_propagate(const emb_terminal_models* models, const emb_rng* rng
 // ---- log-likelihood of given bins (emb_loglik.cuh) ------------------------------------------------------------------------
 // the device status word of the scoring kernels -> EMB_E_ARG with what was wrong
 static int loglik_status_error(int32_t status) {
+    if (status & emb::LL_BAD_OFFSETS) return set_err(EMB_E_ARG, "loglik: offsets must be non-negative and non-decreasing");
+    if (status & emb::LL_BAD_VAR)
+        return set_err(EMB_E_ARG, "loglik: a row's variable id is outside 0..n_initial (or its gated ordinal above n_gated)");
     if (status & emb::LL_BAD_BIN) return set_err(EMB_E_ARG, "loglik: a bin is outside 1..r of its variable");
     if (status & emb::LL_BAD_COL0)
         return set_err(EMB_E_ARG, "loglik: column 0 of the track bins differs from init_bins of the dynamic variables");
+    if (status & emb::LL_BAD_STATIC)
+        return set_err(EMB_E_ARG, "loglik: a row of a static variable sets a bin other than its init_bins value");
     return 0;
 }
 
@@ -1035,6 +1041,56 @@ int emb_loglik_tracks(const emb_model* m, int64_t n, int32_t T, const int8_t* in
         return set_err(EMB_E_ARG, "null or out-of-range argument");
     if (int rc = need_transition(*m->h)) return rc;
     return loglik_impl(m, n, T, init_bins, bins, opts, initial, nullptr, transition);
+}
+
+// both event-list forms: checks, device tables, staging, one launch, status
+static int loglik_events_impl(const emb_model* m, int64_t n, int32_t T, const int8_t* init_bins, const void* words,
+                              const uint8_t* dts, const int64_t* offsets, bool packed, const emb_sample_opts* opts,
+                              double* initial, double* transition) {
+    if (!m || !opts || n < 0 || T < 1 || (n > 0 && (!init_bins || !words || !offsets || (packed && !dts))))
+        return set_err(EMB_E_ARG, "null or out-of-range argument");
+    const HostModel& H = *m->h;
+    int rc;
+    if ((rc = need_transition(H))) return rc;
+    if (packed && T > 1023) return set_err(EMB_E_ARG, "loglik: packed rows need T <= 1023");
+    if (!packed && T > 65535) return set_err(EMB_E_ARG, "loglik: 8-byte rows need T <= 65535");
+    if (opts->mem & ~0xFF) return set_err(EMB_E_ARG, "loglik: EMB_MEM_ASYNC is not supported; scoring calls are synchronous");
+    if (n == 0) return 0;
+    Call call;
+    if ((rc = call.open(opts, &H, false, true))) return rc;
+    emb::LoglikParams P{};
+    P.n = n;
+    P.T = T;
+    emb::EventRows R{};
+    const void* d_in = nullptr;
+    if ((rc = call.sg.in(init_bins, (size_t)n * (size_t)H.n_initial, &d_in))) return rc;
+    P.init_bins = (const int8_t*)d_in;
+    if ((rc = call.sg.in(offsets, (size_t)(n + 1) * 8, &d_in))) return rc;
+    R.offsets = (const int64_t*)d_in;
+    // host rows are staged up to offsets[n] (the kernel refuses a track whose rows end beyond it); device rows are read in place
+    const size_t rows = call.sg.mem == EMB_MEM_DEVICE ? 1 : (size_t)std::max<int64_t>(offsets[n], 0);
+    if ((rc = call.sg.in(words, rows * (packed ? 4 : 8), &d_in))) return rc;
+    R.words = (const uint32_t*)d_in;
+    if (packed && (rc = call.sg.in(dts, rows, &d_in))) return rc;
+    R.dts = packed ? (const uint8_t*)d_in : nullptr;
+    if ((rc = call.sg.out(initial, (size_t)n * 8, false, (void**)&P.initial))) return rc;
+    if ((rc = call.sg.out(transition, (size_t)n * 8, false, (void**)&P.transition))) return rc;
+    if ((rc = call.status_word(&P.status))) return rc;
+    const cudaError_t e = (cudaError_t)emb::launch_loglik_events(call.D, P, R, packed, call.st);
+    int32_t status;
+    if ((rc = call.finish(e, packed ? "k_loglik_events (packed)" : "k_loglik_events", status))) return rc;
+    return loglik_status_error(status);
+}
+
+int emb_loglik_track_events(const emb_model* m, int64_t n, int32_t T, const int8_t* init_bins, const emb_event* events,
+                            const int64_t* offsets, const emb_sample_opts* opts, double* initial, double* transition) {
+    return loglik_events_impl(m, n, T, init_bins, events, nullptr, offsets, false, opts, initial, transition);
+}
+
+int emb_loglik_track_events_packed(const emb_model* m, int64_t n, int32_t T, const int8_t* init_bins, const uint32_t* words,
+                                   const uint8_t* dts, const int64_t* offsets, const emb_sample_opts* opts, double* initial,
+                                   double* transition) {
+    return loglik_events_impl(m, n, T, init_bins, words, dts, offsets, true, opts, initial, transition);
 }
 
 // IntegrateParams from emb_integrate_opts (labels -> tile ordinals, unit ratios); 0 or an error code

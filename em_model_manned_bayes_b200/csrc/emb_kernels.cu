@@ -13,6 +13,7 @@
 #include "emb_initial.cuh"
 #include "emb_launch.h"
 #include "emb_loglik.cuh"
+#include "emb_loglik_events.cuh"
 
 namespace emb {
 
@@ -331,6 +332,20 @@ __global__ void __launch_bounds__(128) k_loglik_tracks(const __grid_constant__ D
     loglik_track(M, P, s, FROZEN, [&](int k) -> uint32_t& { return s_cnt[k * bs + tid]; });
 }
 
+// tracks as event lists: one thread per track walking its rows, the dynamic state in a register; FROZEN counters as k_loglik_tracks
+template <bool PACKED, bool FROZEN>
+__global__ void __launch_bounds__(128) k_loglik_events(const __grid_constant__ DevModel M, const __grid_constant__ LoglikParams P,
+                                                       const __grid_constant__ EventRows R) {
+    extern __shared__ uint32_t s_cnt[];
+    __shared__ int8_t s_dyn[MAXV];
+    if (threadIdx.x < MAXV) s_dyn[threadIdx.x] = (int8_t)ll_dyn_of(M, threadIdx.x);
+    __syncthreads();
+    const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= P.n) return;
+    const int tid = threadIdx.x, bs = blockDim.x;
+    loglik_track_events<PACKED>(M, P, R, s_dyn, s, FROZEN, [&](int k) -> uint32_t& { return s_cnt[k * bs + tid]; });
+}
+
 }  // namespace
 
 int launch_publish(const long long* total, const int32_t* flag, long long* mapped_dst, void* stream) {
@@ -484,19 +499,45 @@ int launch_loglik_initial(const DevModel& M, const LoglikParams& P, int table_le
     return (int)cudaGetLastError();
 }
 
+// tracks per block of the frozen-branch scoring kernels: 128 while the counters fit 96 KB of shared memory, fewer otherwise
+// (8 variables of 127 bins at 32: 127 KB)
+static int loglik_frozen_block(const DevModel& M) {
+    const size_t per_thread = (size_t)loglik_counters(M) * 4;
+    int block = 128;
+    while (block > 32 && per_thread * block > 96 * 1024) block /= 2;
+    return block;
+}
+
 int launch_loglik_tracks(const DevModel& M, const LoglikParams& P, void* stream) {
     if (P.n <= 0) return 0;
     if (M.fast) {
-        // 128 tracks per block while the counters fit 96 KB of shared memory, fewer otherwise (8 variables of 127 bins at 32: 127 KB)
-        const size_t per_thread = (size_t)loglik_counters(M) * 4;
-        int block = 128;
-        while (block > 32 && per_thread * block > 96 * 1024) block /= 2;
-        const size_t bytes = per_thread * block;
+        const int block = loglik_frozen_block(M);
+        const size_t bytes = (size_t)loglik_counters(M) * 4 * block;
         cudaFuncSetAttribute(k_loglik_tracks<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
         k_loglik_tracks<true><<<(unsigned)((P.n + block - 1) / block), block, bytes, (cudaStream_t)stream>>>(M, P);
     } else {
         k_loglik_tracks<false><<<(unsigned)((P.n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(M, P);
     }
+    g_launch_count.fetch_add(1);
+    return (int)cudaGetLastError();
+}
+
+template <bool PACKED>
+static void launch_loglik_events_t(const DevModel& M, const LoglikParams& P, const EventRows& R, cudaStream_t stream) {
+    if (M.fast) {
+        const int block = loglik_frozen_block(M);
+        const size_t bytes = (size_t)loglik_counters(M) * 4 * block;
+        cudaFuncSetAttribute(k_loglik_events<PACKED, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+        k_loglik_events<PACKED, true><<<(unsigned)((P.n + block - 1) / block), block, bytes, stream>>>(M, P, R);
+    } else {
+        k_loglik_events<PACKED, false><<<(unsigned)((P.n + 127) / 128), 128, 0, stream>>>(M, P, R);
+    }
+}
+
+int launch_loglik_events(const DevModel& M, const LoglikParams& P, const EventRows& R, bool packed, void* stream) {
+    if (P.n <= 0) return 0;
+    if (packed) launch_loglik_events_t<true>(M, P, R, (cudaStream_t)stream);
+    else launch_loglik_events_t<false>(M, P, R, (cudaStream_t)stream);
     g_launch_count.fetch_add(1);
     return (int)cudaGetLastError();
 }

@@ -36,6 +36,9 @@ struct LoglikParams;
 int launch_loglik_initial(const DevModel& M, const LoglikParams& P, int table_len, void* stream);
 // M.fast selects the branch: frozen parents (counting kernel) or per-step parents
 int launch_loglik_tracks(const DevModel& M, const LoglikParams& P, void* stream);
+// tracks as event lists (emb_loglik_events.cuh): 8-byte rows or, with `packed`, the 5-byte packed rows; M.fast as above
+struct EventRows;
+int launch_loglik_events(const DevModel& M, const LoglikParams& P, const EventRows& R, bool packed, void* stream);
 
 // terminal trajectory chains (emb_terminal.cu): 4 chains per encounter
 struct TermParams;

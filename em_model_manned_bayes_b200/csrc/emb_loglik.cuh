@@ -82,6 +82,23 @@ EMB_HD void loglik_check_col0(const DevModel& M, const LoglikParams& P, int64_t 
     }
 }
 
+// The frozen-branch transition term from the counters: sum over (variable d, bin b) of count(d, b) * logp[col_d + b], in (d, b)
+// order, counter k = (sum of r over the variables before d) + b.  x: the initial bins, dynamic (t+1) slots set to their time-t bins.
+template <class Cnt>
+EMB_HD double loglik_frozen_sum(const DevModel& M, const uint8_t* x, Cnt cnt) {
+    double acc = 0.0;
+    int k = 0;
+    for (int d = 0; d < M.n_dyn; ++d) {
+        const uint32_t col = ll_column(M.dyn[d], x);
+        for (int b = 0; b < M.dyn[d].r; ++b) {
+            const uint32_t c = cnt(k + b);
+            if (c) acc = dadd(acc, dmul((double)c, ldg64(M.logp_trans + col + b)));   // c == 0 skipped: 0 * -inf is NaN
+        }
+        k += M.dyn[d].r;
+    }
+    return acc;
+}
+
 // Frozen-parent branch (dbn_sample.m:110-135): the column of every dynamic variable is fixed by column 0, so the transition term is
 // sum over (variable d, bin b) of count(d, b) * logp[col_d + b], the counts taken over columns 1..T-1 and the sum in (d, b) order.
 // cnt(k) is the counter k = cbase[d] + b of this track (thread-private; shared memory [k][thread] on the device).
@@ -114,15 +131,7 @@ EMB_HD double loglik_transition_frozen(const DevModel& M, const LoglikParams& P,
         }
     }
     if (bad) ll_flag(P.status, LL_BAD_BIN);
-    double acc = 0.0;
-    for (int d = 0; d < nd; ++d) {
-        const uint32_t col = ll_column(M.dyn[d], x);
-        for (int b = 0; b < M.dyn[d].r; ++b) {
-            const uint32_t c = cnt(cbase[d] + b);
-            if (c) acc = dadd(acc, dmul((double)c, ldg64(M.logp_trans + col + b)));   // c == 0 skipped: 0 * -inf is NaN
-        }
-    }
-    return acc;
+    return loglik_frozen_sum(M, x, cnt);
 }
 
 // Per-step branch (dbn_sample.m:66-79, or correct_dbn): at column c the parents see the time-t slots at column c-1 and the (t+1)

@@ -445,6 +445,47 @@ class EncounterModel:
         L.check(L.lib().emb_loglik_tracks(self._h, n, int(T), _ptr(ib), _ptr(bt), C.byref(o), _ptr(init), _ptr(trans)))
         return init, trans
 
+    def loglik_events(self, events, offsets=None, T: Optional[int] = None, init_bins=None, dts=None, correct_dbn: bool = False,
+                      device=None):
+        """log p of tracks given as event lists (emb_loglik_track_events[_packed]): the same (initial (n,), transition (n,))
+        float64 as `loglik_tracks` on the dense bins the lists expand to (`expand_events`), computed from the rows.
+        `events`: a whole `EventResult` or `PackedEventResult` (it must carry init_bins), or raw rows -- emb_event rows
+        (`EVENT_DTYPE` array, or the int64 tensor of a device `EventResult`), or packed words with their `dts` -- together
+        with `offsets` (int64 [n+1]), `T` and `init_bins` (n_initial, n).  numpy in, numpy out; torch CUDA tensors in, tensors
+        on their device out."""
+        if isinstance(events, (EventResult, PackedEventResult)):
+            r = events
+            if r.init_bins is None:
+                raise L.EmbError(L.EMB_E_ARG, "loglik_events: the result needs init_bins (want_init)")
+            offsets, T, init_bins = r.offsets, r.T, r.init_bins
+            events, dts = (r.words, r.dts) if isinstance(r, PackedEventResult) else (r.events, None)
+        if offsets is None or T is None or init_bins is None:
+            raise L.EmbError(L.EMB_E_ARG, "loglik_events: offsets, T and init_bins are required")
+        arrays = [init_bins, events, offsets] + ([dts] if dts is not None else [])
+        o, like = self._score_call(arrays, device, correct_dbn)
+        if init_bins.shape[0] != self.n_initial:
+            raise L.EmbError(L.EMB_E_ARG, "loglik_events: init_bins must be n_initial x n")
+        ib = self._int8(init_bins, like)
+        n = int(ib.shape[1])
+        if like is None:
+            off = np.ascontiguousarray(offsets, dtype=np.int64)
+            ev = np.ascontiguousarray(events)
+            dt = None if dts is None else np.ascontiguousarray(dts, dtype=np.uint8)
+        else:
+            off, ev, dt = offsets.contiguous(), events.contiguous(), None if dts is None else dts.contiguous()
+        if int(off.shape[0]) != n + 1:
+            raise L.EmbError(L.EMB_E_ARG, "loglik_events: offsets must have n + 1 entries")
+        init = self._alloc((n,), np.float64, like)
+        trans = self._alloc((n,), np.float64, like)
+        lib = L.lib()
+        if dt is None:
+            rc = lib.emb_loglik_track_events(self._h, n, int(T), _ptr(ib), _ptr(ev), _ptr(off), C.byref(o), _ptr(init), _ptr(trans))
+        else:
+            rc = lib.emb_loglik_track_events_packed(self._h, n, int(T), _ptr(ib), _ptr(ev), _ptr(dt), _ptr(off), C.byref(o),
+                                                    _ptr(init), _ptr(trans))
+        L.check(rc)
+        return init, trans
+
 
 def async_status(device: int = -1) -> None:
     """Synchronise `device` and raise if an enqueue_only pass exhausted its rejection loop (emb_async_status)."""

@@ -336,6 +336,25 @@ int emb_loglik_initial(const emb_model* m, int64_t n, const int8_t* bins, const 
  * elements); initial[n] / transition[n] nullable */
 int emb_loglik_tracks(const emb_model* m, int64_t n, int32_t T, const int8_t* init_bins, const int8_t* bins,
                       const emb_sample_opts* opts, double* initial, double* transition);
+/* log p of tracks given as event lists, exactly what emb_sample_track_events / emb_sample_track_events_packed write: init_bins
+ * [n_initial][n], offsets int64 [n+1], and the rows (8-byte rows: `bin` is read, `value` ignored; packed rows: gord through
+ * emb_model_get_gated, bin - 1 in bits 23-26).  Defined by reduction: the result is emb_loglik_tracks on the dense bins the lists
+ * expand to as events2samples.m:9-27 expands them -- a row is visible from column sum(dt up to and including it) on, of several
+ * rows that set one variable in one column the last wins, closing rows (var 0) and rows at column >= T change nothing, and a
+ * track with sum(dt) < T holds its last state to the end.  Same conditionals, branches, options and exclusions as
+ * emb_loglik_tracks.  The initial term and the frozen-branch transition term are bit-identical to it; the per-step term sums
+ * each run of constant state as (run length) * log-prob and so may differ from the second-by-second sum in the last bits
+ * (at most 1e-12 relative).  The work is O(rows), not O(T).
+ * EMB_E_ARG, found on the device: a bin outside 1..r, a variable id outside 0..n_initial (8-byte rows) or a gated ordinal above
+ * n_gated (packed rows), a row of a static variable whose bin differs from init_bins (static bins never change), a dynamic
+ * variable whose bin at column 0 differs from init_bins, offsets negative or decreasing.  Refused before the device is touched:
+ * EMB_MEM_ASYNC, a model without a transition network ("dynvar:empty"), T < 1, T > 65535 (8-byte rows) or T > 1023 (packed
+ * rows).  Host buffers are read up to row offsets[n]; initial[n] / transition[n] nullable. */
+int emb_loglik_track_events(const emb_model* m, int64_t n, int32_t T, const int8_t* init_bins, const emb_event* events,
+                            const int64_t* offsets, const emb_sample_opts* opts, double* initial, double* transition);
+int emb_loglik_track_events_packed(const emb_model* m, int64_t n, int32_t T, const int8_t* init_bins, const uint32_t* words,
+                                   const uint8_t* dts, const int64_t* offsets, const emb_sample_opts* opts, double* initial,
+                                   double* transition);
 
 /* ---- misc ------------------------------------------------------------------------------------- */
 int emb_host_alloc(void** p, int64_t bytes); /* pinned host memory */

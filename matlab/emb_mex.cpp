@@ -16,8 +16,9 @@
 //   [out_inits, bins, values, attempts] = emb_mex('sample_tracks', h, seed, first, n, T, opts)
 //   [out_inits, bins, values, hist_i, hist_t] = emb_mex('sample_tracks_multi', h, seed, first, n, T, opts, n_devices)
 //          all GPUs of the box from one call (emb_sample_tracks_multi): bins / values are 1 x D cells of per-device tiles
-//   [events, offsets, out_inits, attempts] = emb_mex('sample_events', h, seed, first, n, T, opts)
-//          events: 4 x rows double [dt; var; value; bin], offsets: (n+1) x 1 (0-based first row of each track)
+//   [events, offsets, out_inits, attempts, init_bins] = emb_mex('sample_events', h, seed, first, n, T, opts)
+//          events: 4 x rows double [dt; var; value; bin], offsets: (n+1) x 1 (0-based first row of each track),
+//          init_bins: n x n_initial int8 (the initial bins, what 'loglik_events' needs)
 //   [traj, len] = emb_mex('terminal_propagate', hs, seed, first, geo, tmax_s, limits, opts)
 //          hs: 1 x 10 uint64 handles {own_fwd(1:2), own_bck(1:2), int_fwd(1:3), int_bck(1:3)}; geo: n x 12 double
 //          [own_intent own_distance own_bearing own_alt own_heading own_speed int_...]; limits: 5 x 2 double
@@ -35,6 +36,9 @@
 //          bins: n x n_initial int8 (1-based); total n x 1, per_var n x n_initial double
 //   [initial, transition] = emb_mex('loglik_tracks', h, init_bins, bins, T, correct_dbn)   % log p of tracks
 //          init_bins: n x n_initial int8; bins: the tiled int8 array of 'sample_tracks'; initial, transition n x 1 double
+//   [initial, transition] = emb_mex('loglik_events', h, init_bins, events, offsets, T, correct_dbn)   % log p of event lists
+//          init_bins, events (4 x rows [dt; var; value; bin]) and offsets as 'sample_events' returns them; the bin row is
+//          required (a 3-row out_events without bins is refused); equal to 'loglik_tracks' on the same tracks
 //          emb_mex('free', h)
 // opts: struct with optional fields start (1 x n_initial, 0/NaN = free), reject_mode, idx_v, idx_dh,
 // idx_L, is_quantize500, layers (r_L x 2), box_lo, box_hi, max_attempts, device, start_per_sample (n x n_initial, 0/NaN = free:
@@ -318,6 +322,37 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         CHECK(emb_loglik_tracks(m, n, T, (const int8_t*)mxGetData(prhs[2]), (const int8_t*)mxGetData(prhs[3]), &o,
                                 mxGetPr(plhs[0]), mxGetPr(tr)));
         if (nlhs > 1) plhs[1] = tr; else mxDestroyArray(tr);
+    } else if (c == "loglik_events") {                            // log p of event lists (emb200.h: emb_loglik_track_events)
+        // [initial, transition] = emb_mex('loglik_events', h, init_bins, events, offsets, T, correct_dbn)
+        const int64_t n = (int64_t)mxGetM(prhs[2]);
+        if ((int64_t)mxGetNumberOfElements(prhs[2]) != n * ni)
+            mexErrMsgIdAndTxt("emb200:arg", "init_bins must be an int8 n x n_initial matrix");
+        if (mxGetM(prhs[3]) != 4)
+            mexErrMsgIdAndTxt("emb200:arg", "events must be the 4 x rows [dt; var; value; bin] matrix of 'sample_events' "
+                                            "(a 3-row out_events has no bins to score)");
+        if ((int64_t)mxGetNumberOfElements(prhs[4]) != n + 1)
+            mexErrMsgIdAndTxt("emb200:arg", "offsets must be the (n+1) x 1 offsets of 'sample_events'");
+        const int64_t rows = (int64_t)mxGetNumberOfElements(prhs[3]) / 4;
+        const double* e = mxGetPr(prhs[3]);
+        std::vector<emb_event> ev((size_t)rows + 1);
+        for (int64_t k = 0; k < rows; ++k) {
+            const double dt = e[4 * k], var = e[4 * k + 1], bin = e[4 * k + 3];
+            if (!(dt >= 0 && dt <= 65535 && var >= 0 && var <= 255 && bin >= 0 && bin <= 255))
+                mexErrMsgIdAndTxt("emb200:arg", "events: dt, var or bin out of range in row %lld", (long long)k + 1);
+            ev[(size_t)k] = emb_event{(uint16_t)dt, (uint8_t)var, (uint8_t)bin, (float)e[4 * k + 2]};
+        }
+        std::vector<int64_t> off((size_t)n + 1);
+        for (int64_t k = 0; k <= n; ++k) off[(size_t)k] = (int64_t)mxGetPr(prhs[4])[k];
+        if (off[(size_t)n] > rows) mexErrMsgIdAndTxt("emb200:arg", "offsets(end) exceeds the number of event rows");
+        const int32_t T = (int32_t)mxGetScalar(prhs[5]);
+        emb_sample_opts o;
+        emb_sample_opts_init(&o);
+        o.correct_dbn = nrhs > 6 ? (int32_t)mxGetScalar(prhs[6]) : 0;
+        plhs[0] = mxCreateDoubleMatrix(n, 1, mxREAL);
+        mxArray* tr = mxCreateDoubleMatrix(n, 1, mxREAL);
+        CHECK(emb_loglik_track_events(m, n, T, (const int8_t*)mxGetData(prhs[2]), ev.data(), off.data(), &o, mxGetPr(plhs[0]),
+                                      mxGetPr(tr)));
+        if (nlhs > 1) plhs[1] = tr; else mxDestroyArray(tr);
     } else if (c == "sample_tracks_multi") {                    // every GPU of the box from one MATLAB process (SURVEY 8e)
         // [out_inits, bins, values, hist_initial, hist_transition] = emb_mex('sample_tracks_multi', h, seed, first, n, T, opts, n_devices)
         // out_inits n x n_initial; bins / values: 1 x D cells of the per-device tiled arrays (shard d = emb_shard_range(n, d, D))
@@ -418,9 +453,11 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         std::vector<int64_t> off((size_t)n + 1);
         mxArray* inits = mxCreateDoubleMatrix(n, ni, mxREAL);
         mxArray* att = mxCreateNumericMatrix(n, 1, mxUINT16_CLASS, mxREAL);
+        mxArray* ibins = mxCreateNumericMatrix(n, ni, mxINT8_CLASS, mxREAL);   // n x n_initial == the ABI's [n_initial][n]
         emb_track_out init{};
         init.init_values = mxGetPr(inits);
         init.attempts = (uint16_t*)mxGetData(att);
+        init.init_bins = (int8_t*)mxGetData(ibins);
         int64_t total = 0;
         // 5-byte packed rows (what the device writes and what crosses PCIe); the value of a row is evaluated here in fp64 from
         // its bin and 23-bit uniform exactly as dediscretize.m:39 does.  Models outside the packed format (more than 7
@@ -474,6 +511,7 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         if (nlhs > 1) plhs[1] = offs; else mxDestroyArray(offs);
         if (nlhs > 2) plhs[2] = inits; else mxDestroyArray(inits);
         if (nlhs > 3) plhs[3] = att; else mxDestroyArray(att);
+        if (nlhs > 4) plhs[4] = ibins; else mxDestroyArray(ibins);
     } else {
         mexErrMsgIdAndTxt("emb200:arg", "unknown command '%s'", cmd);
     }
