@@ -96,6 +96,10 @@ class IntegrateOpts(C.Structure):
                 ("mem", C.c_int32), ("device", C.c_int32), ("stream", C.c_void_p)]
 
 
+class ControlsSpec(C.Structure):
+    _fields_ = [("n_cols", C.c_int32), ("vars", C.c_int32 * 8), ("mul", C.c_double * 8), ("div", C.c_double * 8)]
+
+
 class TrackOut(C.Structure):
     _fields_ = [
         ("bins", C.c_void_p), ("values", C.c_void_p), ("init_bins", C.c_void_p), ("init_values", C.c_void_p),
@@ -164,6 +168,9 @@ def lib():
         "emb_loglik_tracks": (C.c_int, [vp, i64, i32, vp, vp, P(SampleOpts), vp, vp]),
         "emb_loglik_track_events": (C.c_int, [vp, i64, i32, vp, vp, vp, P(SampleOpts), vp, vp]),
         "emb_loglik_track_events_packed": (C.c_int, [vp, i64, i32, vp, vp, vp, vp, P(SampleOpts), vp, vp]),
+        "emb_track_events_expand": (C.c_int, [vp, i64, i32, vp, vp, vp, P(SampleOpts), P(ControlsSpec), vp, i64, vp, vp, P(i64)]),
+        "emb_track_events_expand_packed": (C.c_int, [vp, i64, i32, vp, vp, vp, vp, P(SampleOpts), P(ControlsSpec), vp, i64, vp, vp,
+                                                     P(i64)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)  # AttributeError if a declared symbol is missing
@@ -182,6 +189,7 @@ EXPORTED = [
     "emb_dyn_limits_named", "emb_terminal_propagate", "emb_terminal_traj_len", "emb_tracks_integrate", "emb_sample_tracks_xyz",
     "emb_terminal_screen", "emb_loglik_initial", "emb_loglik_tracks",
     "emb_loglik_track_events", "emb_loglik_track_events_packed",
+    "emb_track_events_expand", "emb_track_events_expand_packed",
 ]
 TRAJ_FIELDS = ("x_nm", "y_nm", "z_ft", "heading_deg", "v_ft_s")
 

@@ -4,6 +4,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -14,6 +15,7 @@
 #include <vector>
 
 #include "../../include/emb200.h"
+#include "emb_events_expand.cuh"
 #include "emb_integrate.cuh"
 #include "emb_launch.h"
 #include "emb_loglik.cuh"
@@ -1091,6 +1093,141 @@ int emb_loglik_track_events_packed(const emb_model* m, int64_t n, int32_t T, con
                                    const uint8_t* dts, const int64_t* offsets, const emb_sample_opts* opts, double* initial,
                                    double* transition) {
     return loglik_events_impl(m, n, T, init_bins, words, dts, offsets, true, opts, initial, transition);
+}
+
+// ---- event lists -> samples and control rows (emb_events_expand.cuh) -------------------------------------------------------
+// the device status word of the expansion kernels -> EMB_E_ARG with what was wrong
+static int expand_status_error(int32_t status) {
+    if (status & emb::LL_BAD_OFFSETS) return set_err(EMB_E_ARG, "events_expand: offsets must be non-negative and non-decreasing");
+    if (status & emb::LL_BAD_VAR)
+        return set_err(EMB_E_ARG, "events_expand: a row's variable id is outside 0..n_initial (or its gated ordinal above n_gated)");
+    if (status & emb::LL_BAD_BIN) return set_err(EMB_E_ARG, "events_expand: a packed row's bin is outside 1..r of its variable");
+    return 0;
+}
+
+// the control columns of a spec (NULL or n_cols = 0: temporal_map(:,1), unscaled) -> P.n_cols / vars / mul / div
+static int expand_columns(const HostModel& H, const emb_controls_spec* spec, emb::ExpandParams& P) {
+    const int k = spec ? spec->n_cols : 0;
+    if (k < 0 || k > EMB_MAX_DYN) return set_err(EMB_E_ARG, "events_expand: n_cols must be 0..EMB_MAX_DYN");
+    if (k == 0) {
+        if (int rc = need_transition(H)) return rc;
+        P.n_cols = (int32_t)H.temporal_map.size();
+        for (int j = 0; j < P.n_cols; ++j) {
+            P.vars[j] = H.temporal_map[(size_t)j].first;
+            P.mul[j] = P.div[j] = 1.0;
+        }
+        return 0;
+    }
+    P.n_cols = k;
+    for (int j = 0; j < k; ++j) {
+        if (spec->vars[j] < 1 || spec->vars[j] > H.n_initial)
+            return set_err(EMB_E_ARG, "events_expand: a control column's variable is outside 1..n_initial");
+        if (!std::isfinite(spec->mul[j]) || !std::isfinite(spec->div[j]))
+            return set_err(EMB_E_ARG, "events_expand: a control column's mul or div is not finite");
+        P.vars[j] = spec->vars[j] - 1;
+        P.mul[j] = spec->mul[j];
+        P.div[j] = spec->div[j];
+    }
+    return 0;
+}
+
+// both row formats: checks, staging, count pass + prefix sum (controls), write pass, status
+static int expand_impl(const emb_model* m, int64_t n, int32_t T, const double* init_values, const void* words, const uint8_t* dts,
+                       const int64_t* offsets, bool packed, const emb_sample_opts* opts, const emb_controls_spec* spec,
+                       double* samples, int64_t capacity, double* controls, int64_t* ctl_offsets, int64_t* total_rows) {
+    if (total_rows) *total_rows = 0;
+    if (!m || !opts || n < 0 || T < 1 || capacity < 0 || (capacity > 0 && !controls) ||
+        (n > 0 && (!init_values || !words || !offsets || (packed && !dts))))
+        return set_err(EMB_E_ARG, "null or out-of-range argument");
+    const HostModel& H = *m->h;
+    if (packed && T > 1023) return set_err(EMB_E_ARG, "events_expand: packed rows need T <= 1023");
+    if (!packed && T > 65535) return set_err(EMB_E_ARG, "events_expand: 8-byte rows need T <= 65535");
+    if (opts->mem & ~0xFF) return set_err(EMB_E_ARG, "events_expand: EMB_MEM_ASYNC is not supported; the call is synchronous");
+    emb::ExpandParams P{};
+    int rc;
+    if ((rc = expand_columns(H, spec, P))) return rc;
+    const bool want_ctl = controls || ctl_offsets || total_rows;
+    if (!samples && !want_ctl) return 0;
+    if (n == 0 && (!ctl_offsets || opts->mem == EMB_MEM_HOST)) {
+        if (ctl_offsets) ctl_offsets[0] = 0;
+        return 0;
+    }
+    Call call;
+    if ((rc = call.open(opts, &H))) return rc;
+    const cudaStream_t st = call.st;
+    Stager& sg = call.sg;
+    if (n == 0) {   // device offsets
+        const int64_t zero = 0;
+        CU(cudaMemcpyAsync(ctl_offsets, &zero, 8, cudaMemcpyHostToDevice, st));
+        CU(cudaStreamSynchronize(st));
+        return 0;
+    }
+    P.n = n;
+    P.T = T;
+    emb::EventRows R{};
+    const void* d_in = nullptr;
+    if ((rc = sg.in(init_values, (size_t)n * (size_t)H.n_initial * 8, &d_in))) return rc;
+    P.init_values = (const double*)d_in;
+    if ((rc = sg.in(offsets, (size_t)(n + 1) * 8, &d_in))) return rc;
+    R.offsets = (const int64_t*)d_in;
+    // host rows are staged up to offsets[n] (the kernels refuse a track whose rows end beyond it); device rows are read in place
+    const size_t rows = sg.mem == EMB_MEM_DEVICE ? 1 : (size_t)std::max<int64_t>(offsets[n], 0);
+    if ((rc = sg.in(words, rows * (packed ? 4 : 8), &d_in))) return rc;
+    R.words = (const uint32_t*)d_in;
+    if (packed && (rc = sg.in(dts, rows, &d_in))) return rc;
+    R.dts = packed ? (const uint8_t*)d_in : nullptr;
+    if ((rc = call.status_word(&P.status))) return rc;
+    Tmp counts, tiles, off_tmp;
+    if (want_ctl) {
+        // count pass: control rows per track, then their prefix sum into ctl_offsets
+        long long* d_off = nullptr;
+        if ((rc = sg.out(ctl_offsets, (size_t)(n + 1) * 8, false, (void**)&d_off))) return rc;
+        if (!d_off) {
+            CU(tmp_alloc(&off_tmp.p, (size_t)(n + 1) * 8, st));
+            d_off = (long long*)off_tmp.p;
+        }
+        CU(tmp_alloc(&counts.p, (size_t)n * 4, st));
+        CU(tmp_alloc(&tiles.p, (size_t)emb::scan_scratch_len(n) * 8, st));
+        P.counts = (uint32_t*)counts.p;
+        cudaError_t e = (cudaError_t)emb::launch_events_expand(call.D, P, R, packed, true, st);
+        if (e != cudaSuccess) return cuda_fail(e, "launch k_events_expand_count");
+        e = (cudaError_t)emb::launch_scan_counts((const uint32_t*)counts.p, d_off, n, (long long*)tiles.p, st);
+        if (e != cudaSuccess) return cuda_fail(e, "launch k_scan_counts");
+        long long total = 0;
+        int32_t flag = 0;
+        CU(cudaMemcpyAsync(&total, d_off + n, 8, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(&flag, P.status, 4, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        if (total_rows) *total_rows = total;
+        if (flag) return expand_status_error(flag);
+        if (total > capacity) {
+            if ((rc = sg.finish())) return rc;   // ctl_offsets are valid
+            return set_err(EMB_E_LIMIT, "control buffer too small: " + std::to_string(total) + " rows needed");
+        }
+        P.ctl_offsets = d_off;
+        if ((rc = sg.out(controls, (size_t)total * (size_t)(1 + P.n_cols) * 8, false, (void**)&P.controls))) return rc;
+    }
+    if ((rc = sg.out(samples, (size_t)n * (size_t)T * (size_t)H.n_initial * 8, false, (void**)&P.samples))) return rc;
+    const cudaError_t e = P.samples || P.controls ? (cudaError_t)emb::launch_events_expand(call.D, P, R, packed, false, st)
+                                                  : cudaSuccess;
+    int32_t status;
+    if ((rc = call.finish(e, packed ? "k_events_expand (packed)" : "k_events_expand", status))) return rc;
+    return expand_status_error(status);
+}
+
+int emb_track_events_expand(const emb_model* m, int64_t n, int32_t T, const double* init_values, const emb_event* events,
+                            const int64_t* offsets, const emb_sample_opts* opts, const emb_controls_spec* spec,
+                            double* samples, int64_t capacity, double* controls, int64_t* ctl_offsets, int64_t* total_rows) {
+    return expand_impl(m, n, T, init_values, events, nullptr, offsets, false, opts, spec, samples, capacity, controls, ctl_offsets,
+                       total_rows);
+}
+
+int emb_track_events_expand_packed(const emb_model* m, int64_t n, int32_t T, const double* init_values, const uint32_t* words,
+                                   const uint8_t* dts, const int64_t* offsets, const emb_sample_opts* opts,
+                                   const emb_controls_spec* spec, double* samples, int64_t capacity, double* controls,
+                                   int64_t* ctl_offsets, int64_t* total_rows) {
+    return expand_impl(m, n, T, init_values, words, dts, offsets, true, opts, spec, samples, capacity, controls, ctl_offsets,
+                       total_rows);
 }
 
 // IntegrateParams from emb_integrate_opts (labels -> tile ordinals, unit ratios); 0 or an error code

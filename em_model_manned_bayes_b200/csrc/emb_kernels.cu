@@ -9,6 +9,7 @@
 #include <atomic>
 
 #include "emb_device.cuh"
+#include "emb_events_expand.cuh"
 #include "emb_fast.cuh"
 #include "emb_initial.cuh"
 #include "emb_launch.h"
@@ -346,6 +347,29 @@ __global__ void __launch_bounds__(128) k_loglik_events(const __grid_constant__ D
     loglik_track_events<PACKED>(M, P, R, s_dyn, s, FROZEN, [&](int k) -> uint32_t& { return s_cnt[k * bs + tid]; });
 }
 
+// event lists -> samples and control rows (emb_events_expand.cuh): one warp per track
+constexpr int EE_BLOCK = 256;
+
+template <bool PACKED>
+__global__ void __launch_bounds__(EE_BLOCK) k_events_expand_count(const __grid_constant__ DevModel M,
+                                                                  const __grid_constant__ ExpandParams P,
+                                                                  const __grid_constant__ EventRows R) {
+    const int64_t s = (int64_t)blockIdx.x * (EE_BLOCK / 32) + (threadIdx.x >> 5);
+    if (s >= P.n) return;
+    const ExpandLanes L{(int)(threadIdx.x & 31)};
+    const uint32_t rows = events_expand_count<PACKED>(M, P, R, s, L);
+    if (L.lane == 0) P.counts[s] = rows;
+}
+
+template <bool PACKED>
+__global__ void __launch_bounds__(EE_BLOCK) k_events_expand(const __grid_constant__ DevModel M, const __grid_constant__ ExpandParams P,
+                                                            const __grid_constant__ EventRows R) {
+    __shared__ ExpandShared sh[EE_BLOCK / 32];
+    const int64_t s = (int64_t)blockIdx.x * (EE_BLOCK / 32) + (threadIdx.x >> 5);
+    if (s >= P.n) return;
+    events_expand_track<PACKED>(M, P, R, s, ExpandLanes{(int)(threadIdx.x & 31)}, sh[threadIdx.x >> 5]);
+}
+
 }  // namespace
 
 int launch_publish(const long long* total, const int32_t* flag, long long* mapped_dst, void* stream) {
@@ -538,6 +562,21 @@ int launch_loglik_events(const DevModel& M, const LoglikParams& P, const EventRo
     if (P.n <= 0) return 0;
     if (packed) launch_loglik_events_t<true>(M, P, R, (cudaStream_t)stream);
     else launch_loglik_events_t<false>(M, P, R, (cudaStream_t)stream);
+    g_launch_count.fetch_add(1);
+    return (int)cudaGetLastError();
+}
+
+int launch_events_expand(const DevModel& M, const ExpandParams& P, const EventRows& R, bool packed, bool count, void* stream) {
+    if (P.n <= 0) return 0;
+    const unsigned grid = (unsigned)((P.n + EE_BLOCK / 32 - 1) / (EE_BLOCK / 32));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (count) {
+        if (packed) k_events_expand_count<true><<<grid, EE_BLOCK, 0, st>>>(M, P, R);
+        else k_events_expand_count<false><<<grid, EE_BLOCK, 0, st>>>(M, P, R);
+    } else {
+        if (packed) k_events_expand<true><<<grid, EE_BLOCK, 0, st>>>(M, P, R);
+        else k_events_expand<false><<<grid, EE_BLOCK, 0, st>>>(M, P, R);
+    }
     g_launch_count.fetch_add(1);
     return (int)cudaGetLastError();
 }

@@ -39,6 +39,9 @@ int launch_loglik_tracks(const DevModel& M, const LoglikParams& P, void* stream)
 // tracks as event lists (emb_loglik_events.cuh): 8-byte rows or, with `packed`, the 5-byte packed rows; M.fast as above
 struct EventRows;
 int launch_loglik_events(const DevModel& M, const LoglikParams& P, const EventRows& R, bool packed, void* stream);
+// event lists -> samples and control rows (emb_events_expand.cuh): the count pass (P.counts) or the write pass
+struct ExpandParams;
+int launch_events_expand(const DevModel& M, const ExpandParams& P, const EventRows& R, bool packed, bool count, void* stream);
 
 // terminal trajectory chains (emb_terminal.cu): 4 chains per encounter
 struct TermParams;

@@ -309,7 +309,7 @@ class EncounterModel:
             return np.zeros(shape, dtype=dtype)
         import torch
         tdt = {np.int8: torch.int8, np.float32: torch.float32, np.float64: torch.float64, np.uint16: torch.int16, np.int16: torch.int16, np.uint8: torch.uint8,
-               np.uint64: torch.int64}[dtype]
+               np.uint64: torch.int64, np.int64: torch.int64}[dtype]
         return torch.zeros(shape, dtype=tdt, device=like)
 
     # -- sampling ----------------------------------------------------------------------------------
@@ -486,6 +486,72 @@ class EncounterModel:
         L.check(rc)
         return init, trans
 
+    # -- event lists -> out_samples and control rows (emb200.h: emb_track_events_expand[_packed]) ----------------------------
+    def expand_events_gpu(self, events, offsets=None, T: Optional[int] = None, init_values=None, dts=None,
+                          want_samples: bool = True, spec=None, device=None):
+        """The other two outputs of UncorEncounterModel.sample, computed on the device from event lists.
+        `events`: a whole `EventResult` or `PackedEventResult` (it must carry init_values), or raw rows -- emb_event rows
+        (`EVENT_DTYPE` array, or the int64 tensor of a device `EventResult`), or packed words with their `dts` -- together
+        with `offsets` (int64 [n+1]), `T` and `init_values` (n_initial, n) float64.
+        `spec`: None for plain events2controls.m (the variables temporal_map(:,1), unscaled), or (vars, mul, div): 1-based
+        initial variables and per column y = (x * mul) / div (`UncorEncounterModel.out_eme_spec()` gives the out_EME matrix).
+        Returns (samples (n, T, n_initial) float64 or None -- samples[s] is out_samples{s}' -- and a `ControlsResult`).
+        numpy in, numpy out; torch CUDA tensors in, tensors on their device out."""
+        if isinstance(events, (EventResult, PackedEventResult)):
+            r = events
+            if r.init_values is None:
+                raise L.EmbError(L.EMB_E_ARG, "expand_events_gpu: the result needs init_values (want_init)")
+            offsets, T, init_values = r.offsets, r.T, r.init_values
+            events, dts = (r.words, r.dts) if isinstance(r, PackedEventResult) else (r.events, None)
+        if offsets is None or T is None or init_values is None:
+            raise L.EmbError(L.EMB_E_ARG, "expand_events_gpu: offsets, T and init_values are required")
+        arrays = [init_values, events, offsets] + ([dts] if dts is not None else [])
+        o, like = self._score_call(arrays, device, False)
+        if init_values.shape[0] != self.n_initial:
+            raise L.EmbError(L.EMB_E_ARG, "expand_events_gpu: init_values must be n_initial x n")
+        n, T = int(init_values.shape[1]), int(T)
+        if like is None:
+            iv = np.ascontiguousarray(init_values, dtype=np.float64)
+            off = np.ascontiguousarray(offsets, dtype=np.int64)
+            ev = np.ascontiguousarray(events)
+            dt = None if dts is None else np.ascontiguousarray(dts, dtype=np.uint8)
+        else:
+            import torch
+            iv, off, ev = init_values.to(torch.float64).contiguous(), offsets.contiguous(), events.contiguous()
+            dt = None if dts is None else dts.contiguous()
+        if int(off.shape[0]) != n + 1:
+            raise L.EmbError(L.EMB_E_ARG, "expand_events_gpu: offsets must have n + 1 entries")
+        cs = L.ControlsSpec()
+        if spec is not None:
+            vars_, mul, div = (list(c) for c in spec)
+            if not (len(vars_) == len(mul) == len(div)) or len(vars_) > len(cs.vars):
+                raise L.EmbError(L.EMB_E_ARG, "expand_events_gpu: spec needs equally long vars, mul and div of at most 8 columns")
+            cs.n_cols = len(vars_)
+            for j in range(cs.n_cols):
+                cs.vars[j], cs.mul[j], cs.div[j] = int(vars_[j]), float(mul[j]), float(div[j])
+        k = cs.n_cols or self.n_dyn
+        samples = self._alloc((n, T, self.n_initial), np.float64, like) if want_samples else None
+        ctl_off = self._alloc((n + 1,), np.int64, like)
+        total = C.c_int64(0)
+        lib = L.lib()
+
+        def call(capacity, rows):
+            if dt is None:
+                return lib.emb_track_events_expand(self._h, n, T, _ptr(iv), _ptr(ev), _ptr(off), C.byref(o), C.byref(cs),
+                                                   _ptr(samples), capacity, _ptr(rows), _ptr(ctl_off), C.byref(total))
+            return lib.emb_track_events_expand_packed(self._h, n, T, _ptr(iv), _ptr(ev), _ptr(dt), _ptr(off), C.byref(o),
+                                                      C.byref(cs), _ptr(samples), capacity, _ptr(rows), _ptr(ctl_off),
+                                                      C.byref(total))
+
+        rc = call(0, None)                                  # sizes the control rows (and writes everything if there are none)
+        if rc == L.EMB_E_LIMIT and total.value > 0:
+            rows = self._alloc((int(total.value), 1 + k), np.float64, like)
+            rc = call(int(total.value), rows)
+        else:
+            rows = self._alloc((0, 1 + k), np.float64, like)
+        L.check(rc)
+        return samples, ControlsResult(rows=rows, offsets=ctl_off)
+
 
 def async_status(device: int = -1) -> None:
     """Synchronise `device` and raise if an enqueue_only pass exhausted its rejection loop (emb_async_status)."""
@@ -562,6 +628,17 @@ class PackedEventResult:
         o = np.asarray(self.offsets.cpu() if hasattr(self.offsets, "cpu") else self.offsets)
         a, b = int(o[s]), int(o[s + 1])
         return np.stack([dt[a:b].astype(np.float64), var[a:b].astype(np.float64), val[a:b]], axis=1)
+
+
+@dataclass
+class ControlsResult:
+    """Control rows of `EncounterModel.expand_events_gpu`: rows[offsets[s]:offsets[s+1]] belong to track s."""
+    rows: object          # (total, 1 + k) float64: [t, y_1 .. y_k]
+    offsets: object       # int64 [n + 1]
+
+    def track(self, s: int):
+        """the control matrix of track s (events2controls.m, or the out_EME event matrix with that spec)"""
+        return self.rows[int(self.offsets[s]):int(self.offsets[s + 1])]
 
 
 def _row_times(dt: np.ndarray, offsets: np.ndarray) -> np.ndarray:
@@ -861,6 +938,28 @@ class UncorEncounterModel(EncounterModel):
         if math.isnan(vr):
             vr = 0.0
         return dict(minVel_ft_s=float(min_speed), maxVel_ft_s=float(max_speed), maxVertRate_ft_s=vr)
+
+    def out_eme_spec(self):
+        """The control columns of out_EME (UncorEncounterModel.m:286-297): [dh ft/min -> ft/s, dpsi deg/s -> rad/s,
+        dv kt/s -> ft/s^2] as (vars, mul, div) for `expand_events_gpu`: x / 60, (pi/180) * x, x * 1.68780972222222."""
+        return [self.idxDH, self.idxDPsi, self.idxDV], [1.0, math.pi / 180.0, 1.68780972222222], [60.0, 1.0, 1.0]
+
+    def sample_batch(self, n_samples: int, sample_time: int, seed=float("nan"), isQuantize500=False, layers=None, device=None,
+                     packed: bool = True, want_samples: bool = False):
+        """The four outputs of UncorEncounterModel.m:192-313 in batch form, all computed on the device:
+        (out_inits (n, n_initial) float64, the event result (`PackedEventResult`, or with packed=False the 8-byte
+        `EventResult` that `sample` reads), samples (n, sample_time, n_initial) float64 or None -- samples[s] is
+        out_samples{s}' -- and the out_EME event matrices as a `ControlsResult`).  With packed=False the values are the
+        fp32 row values `sample` reads, so samples and controls equal its out_samples and out_EME.event bit for bit.
+        `device`: keep everything in HBM as torch tensors; default host numpy."""
+        if isinstance(seed, float) and math.isnan(seed):
+            seed = int(np.random.SeedSequence().generate_state(2, dtype=np.uint32).view(np.uint64)[0])
+        o = self.uncor_opts(isQuantize500, layers)
+        fn = self.sample_events_packed if packed else self.sample_events
+        res = fn(n_samples, sample_time, seed=int(seed), opts=o, device=device)
+        samples, ctl = self.expand_events_gpu(res, want_samples=want_samples, spec=self.out_eme_spec())
+        out_inits = np.ascontiguousarray(res.init_values.T) if device is None else res.init_values.T
+        return out_inits, res, samples, ctl
 
     def sample(self, n_samples: int, sample_time: int, seed=float("nan"), isQuantize500=False, layers=None):
         """UncorEncounterModel.m:192-313 -> (out_inits n x n_initial, out_events list of k x 3 [dt var value],

@@ -356,6 +356,44 @@ int emb_loglik_track_events_packed(const emb_model* m, int64_t n, int32_t T, con
                                    const uint8_t* dts, const int64_t* offsets, const emb_sample_opts* opts, double* initial,
                                    double* transition);
 
+/* ---- event lists -> out_samples and control rows (UncorEncounterModel.m:283-300) ----------------------------------- */
+/* Columns of the control rows: y_j = (x[vars[j]] * mul[j]) / div[j], two correctly rounded fp64 operations (a factor of 1 is
+ * exact).  n_cols = 0 (or a NULL spec) is plain events2controls.m: the variables temporal_map(:,1), unscaled.  The out_EME
+ * matrix of UncorEncounterModel.m:286-297 is vars = [idxDH, idxDPsi, idxDV], mul = [1, pi/180, 1.68780972222222],
+ * div = [60, 1, 1]: the operations /60, deg2rad = (pi/180)*x and *1.68780972222222 of :295-297. */
+typedef struct emb_controls_spec {
+    int32_t n_cols;                /* 0..EMB_MAX_DYN */
+    int32_t vars[EMB_MAX_DYN];     /* 1-based initial variable ids */
+    double mul[EMB_MAX_DYN];
+    double div[EMB_MAX_DYN];
+} emb_controls_spec;
+/* The other two outputs of UncorEncounterModel.sample, computed on the device from event lists: init_values [n_initial][n]
+ * fp64 (out_inits, the layout of emb_track_out.init_values), offsets int64 [n+1], and the rows -- 8-byte rows (the value is
+ * the row's fp32 `value` widened to fp64) or packed rows (the variable from gord through emb_model_get_gated, the value
+ * decoded in fp64 as above: a + w*u with u = (frac + 0.5) 2^-23, 0 in a zero bin, the bin itself for a '*' variable).
+ * Defined by reduction to the host statements:
+ *   samples (nullable): fp64 [n][T][n_initial]; track s is the column-major n_initial x T matrix out_samples{s}, which is
+ *     events2samples.m:9-27 (model.py expand_events): a row is visible from column sum(dt up to and including it) on, the last
+ *     row wins within a column, rows at column >= T change nothing, and sum(dt) < T holds the last state.
+ *   controls: events2controls.m:9-31 -- one row for every list row with dt > 0 (closing rows included), in list order,
+ *     [t, y_1 .. y_k] in fp64 row-major (1 + k doubles), t the seconds before the row and x the state before the row is
+ *     applied (every earlier row, also those at column >= T).  ctl_offsets int64 [n+1] counts rows (nullable);
+ *     *total_rows (nullable) always receives the total.  If the total exceeds `capacity`, samples and controls are not
+ *     written, ctl_offsets and *total_rows are, and EMB_E_LIMIT is returned; capacity = 0 with a NULL `controls` sizes
+ *     the list.  With controls, ctl_offsets and total_rows all NULL no control pass runs.
+ * Only mem, device and stream of `opts` are read.  EMB_E_ARG, found on the device: a variable id outside 0..n_initial, a
+ * gated ordinal above n_gated, a packed bin outside 1..r of its variable, offsets negative or decreasing.  Refused before
+ * the device is touched: EMB_MEM_ASYNC, T < 1, T > 65535 (8-byte rows) or T > 1023 (packed rows), n_cols outside
+ * 0..EMB_MAX_DYN, a column variable outside 1..n_initial, a non-finite mul or div, n_cols = 0 on a model without a
+ * transition network ("dynvar:empty").  Host row buffers are read up to row offsets[n]. */
+int emb_track_events_expand(const emb_model* m, int64_t n, int32_t T, const double* init_values, const emb_event* events,
+                            const int64_t* offsets, const emb_sample_opts* opts, const emb_controls_spec* spec,
+                            double* samples, int64_t capacity, double* controls, int64_t* ctl_offsets, int64_t* total_rows);
+int emb_track_events_expand_packed(const emb_model* m, int64_t n, int32_t T, const double* init_values, const uint32_t* words,
+                                   const uint8_t* dts, const int64_t* offsets, const emb_sample_opts* opts,
+                                   const emb_controls_spec* spec, double* samples, int64_t capacity, double* controls,
+                                   int64_t* ctl_offsets, int64_t* total_rows);
+
 /* ---- misc ------------------------------------------------------------------------------------- */
 int emb_host_alloc(void** p, int64_t bytes); /* pinned host memory */
 int emb_host_free(void* p);

@@ -16,9 +16,12 @@
 //   [out_inits, bins, values, attempts] = emb_mex('sample_tracks', h, seed, first, n, T, opts)
 //   [out_inits, bins, values, hist_i, hist_t] = emb_mex('sample_tracks_multi', h, seed, first, n, T, opts, n_devices)
 //          all GPUs of the box from one call (emb_sample_tracks_multi): bins / values are 1 x D cells of per-device tiles
-//   [events, offsets, out_inits, attempts, init_bins] = emb_mex('sample_events', h, seed, first, n, T, opts)
+//   [events, offsets, out_inits, attempts, init_bins, out_samples, ctl] = emb_mex('sample_events', h, seed, first, n, T, opts)
 //          events: 4 x rows double [dt; var; value; bin], offsets: (n+1) x 1 (0-based first row of each track),
-//          init_bins: n x n_initial int8 (the initial bins, what 'loglik_events' needs)
+//          init_bins: n x n_initial int8 (the initial bins, what 'loglik_events' needs),
+//          out_samples: n x 1 cell of n_initial x T (events2samples.m), ctl: n x 1 cell of the out_EME event matrices
+//          [t, dh/60, deg2rad(dpsi), dv*1.68780972222222] (UncorEncounterModel.m:286-297) -- both computed on the GPU from
+//          the same rows (emb_track_events_expand[_packed]), and only when requested
 //   [traj, len] = emb_mex('terminal_propagate', hs, seed, first, geo, tmax_s, limits, opts)
 //          hs: 1 x 10 uint64 handles {own_fwd(1:2), own_bck(1:2), int_fwd(1:3), int_bck(1:3)}; geo: n x 12 double
 //          [own_intent own_distance own_bearing own_alt own_heading own_speed int_...]; limits: 5 x 2 double
@@ -45,6 +48,7 @@
 // one `start` row per sample, the cell of @CorTerminalModel/InitStartTerminal.m as a matrix).
 // Errors become mexErrMsgIdAndTxt with the reference's identifiers where the reference has one
 // ('dynvar:empty', UncorEncounterModel.m:231-234; 'prior:notdbe', EncounterModel.m:200).
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <string>
@@ -459,14 +463,17 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         init.attempts = (uint16_t*)mxGetData(att);
         init.init_bins = (int8_t*)mxGetData(ibins);
         int64_t total = 0;
+        std::vector<uint32_t> words;
+        std::vector<uint8_t> dts;
+        std::vector<emb_event> ev;
         // 5-byte packed rows (what the device writes and what crosses PCIe); the value of a row is evaluated here in fp64 from
         // its bin and 23-bit uniform exactly as dediscretize.m:39 does.  Models outside the packed format (more than 7
         // time-varying variables or T > 1023) take the 8-byte rows.
         int rc = emb_sample_track_events_packed(m, &rng, n, T, &o, 0, nullptr, nullptr, off.data(), &init, &total);   // sizes the list
         const bool packed = rc == 0 || (rc == EMB_E_LIMIT && total > 0);
         if (packed) {
-            std::vector<uint32_t> words((size_t)total + 1);
-            std::vector<uint8_t> dts((size_t)total + 1);
+            words.resize((size_t)total + 1);
+            dts.resize((size_t)total + 1);
             CHECK(emb_sample_track_events_packed(m, &rng, n, T, &o, total, words.data(), dts.data(), off.data(), &init, &total));
             int32_t gated[EMB_MAX_GATED];
             const int ng = (int)emb_model_get_gated(m, gated, EMB_MAX_GATED);
@@ -495,7 +502,6 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
                 e[4 * k] = dt; e[4 * k + 1] = var; e[4 * k + 2] = val; e[4 * k + 3] = bin;
             }
         } else {
-        std::vector<emb_event> ev;
         rc = emb_sample_track_events(m, &rng, n, T, &o, 0, nullptr, off.data(), &init, &total);   // sizes the list
         if (rc != 0 && rc != EMB_E_LIMIT) fail(rc);
         ev.resize((size_t)total + 1);
@@ -512,6 +518,73 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         if (nlhs > 2) plhs[2] = inits; else mxDestroyArray(inits);
         if (nlhs > 3) plhs[3] = att; else mxDestroyArray(att);
         if (nlhs > 4) plhs[4] = ibins; else mxDestroyArray(ibins);
+        if (nlhs > 5) {   // out_samples and the out_EME matrices on the GPU, from the rows above (host buffers)
+            emb_controls_spec spec{};
+            if (nlhs > 6) {   // UncorEncounterModel.m:225-234, 286-297
+                std::string lab((size_t)emb_model_get_labels(m, 0, nullptr, 0), '\0');
+                emb_model_get_labels(m, 0, &lab[0], (int64_t)lab.size());
+                auto find = [&](const char* name) {
+                    int id = 1;
+                    for (size_t a = 0; a < lab.size();) {
+                        const size_t b = std::min(lab.find('\n', a), lab.size() - 1);
+                        if (lab.compare(a, b - a, name) == 0) return id;
+                        a = b + 1;
+                        ++id;
+                    }
+                    mexErrMsgIdAndTxt("dynvar:empty", "Model does not have a dynamic variable for either acceleration, vertical "
+                                                      "rate, or turn rate");
+                    return 0;
+                };
+                spec.n_cols = 3;
+                spec.vars[0] = find("\"\\dot h\"");
+                spec.vars[1] = find("\"\\dot \\psi\"");
+                spec.vars[2] = find("\"\\dot v\"");
+                const double mul[3] = {1.0, 3.141592653589793 / 180.0, 1.68780972222222}, div[3] = {60.0, 1.0, 1.0};
+                for (int j = 0; j < 3; ++j) {
+                    spec.mul[j] = mul[j];
+                    spec.div[j] = div[j];
+                }
+            }
+            emb_sample_opts eo;
+            emb_sample_opts_init(&eo);
+            eo.device = o.device;
+            std::vector<double> smp((size_t)n * (size_t)T * (size_t)ni);
+            std::vector<int64_t> coff((size_t)n + 1);
+            std::vector<double> rows;
+            int64_t ctl_total = 0;
+            auto expand = [&](int64_t capacity, double* r, int64_t* co, int64_t* tot) {
+                return packed ? emb_track_events_expand_packed(m, n, T, mxGetPr(inits), words.data(), dts.data(), off.data(), &eo,
+                                                               &spec, smp.data(), capacity, r, co, tot)
+                              : emb_track_events_expand(m, n, T, mxGetPr(inits), ev.data(), off.data(), &eo, &spec, smp.data(),
+                                                        capacity, r, co, tot);
+            };
+            if (nlhs > 6) {
+                rc = expand(0, nullptr, coff.data(), &ctl_total);   // sizes the control rows
+                if (rc != 0 && rc != EMB_E_LIMIT) fail(rc);
+                rows.resize((size_t)ctl_total * 4 + 1);
+                CHECK(expand(ctl_total, rows.data(), coff.data(), &ctl_total));
+            } else {
+                CHECK(expand(0, nullptr, nullptr, nullptr));
+            }
+            plhs[5] = mxCreateCellMatrix(n, 1);
+            for (int64_t s = 0; s < n; ++s) {
+                mxArray* x = mxCreateDoubleMatrix(ni, T, mxREAL);   // [T][n_initial] of track s is the column-major ni x T
+                std::memcpy(mxGetPr(x), smp.data() + (size_t)s * T * ni, sizeof(double) * (size_t)T * ni);
+                mxSetCell(plhs[5], s, x);
+            }
+            if (nlhs > 6) {
+                plhs[6] = mxCreateCellMatrix(n, 1);
+                for (int64_t s = 0; s < n; ++s) {
+                    const int64_t k = coff[(size_t)s + 1] - coff[(size_t)s];
+                    mxArray* x = mxCreateDoubleMatrix(k, 4, mxREAL);
+                    double* pr = mxGetPr(x);
+                    const double* r = rows.data() + (size_t)coff[(size_t)s] * 4;
+                    for (int64_t q = 0; q < k; ++q)
+                        for (int c = 0; c < 4; ++c) pr[c * k + q] = r[q * 4 + c];
+                    mxSetCell(plhs[6], s, x);
+                }
+            }
+        }
     } else {
         mexErrMsgIdAndTxt("emb200:arg", "unknown command '%s'", cmd);
     }

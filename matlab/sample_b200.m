@@ -9,6 +9,7 @@ addRequired(p, 'sample_time', @isnumeric);
 addParameter(p, 'seed', nan, @isnumeric);
 addParameter(p, 'isQuantize500', false, @islogical);
 addParameter(p, 'layers', [], @isnumeric);
+addParameter(p, 'verify', false, @islogical);   % recompute out_samples / out_EME with the reference's functions and compare
 parse(p, n_samples, sample_time, varargin{:});
 seed = p.Results.seed;
 
@@ -40,26 +41,28 @@ for i = 1:self.n_initial
     if ~isempty(self.start{i}), st(i) = self.start{i}; end
 end
 opts.start = st;
-[events, offsets, out_inits] = emb_mex('sample_events', h, key, 0, n_samples, sample_time, opts);
+[events, offsets, out_inits, ~, ~, out_samples, ctl] = emb_mex('sample_events', h, key, 0, n_samples, sample_time, opts);
 % events: 4 x rows [dt; var; value; bin]; rows offsets(ii)+1 : offsets(ii+1) are out_events{ii} of
-% dbn_hierarchical_sample.m:9-37, built on the GPU in the reference's own row order
+% dbn_hierarchical_sample.m:9-37, built on the GPU in the reference's own row order.  out_samples{ii} and ctl{ii} (the
+% event matrix of :286-297) are computed on the GPU from the same rows with the same fp64 operations as the reference's
+% per-track statements; 'verify', true recomputes them with those statements and requires them to be identical.
 
 out_events = cell(n_samples, 1);
-out_samples = cell(n_samples, 1);
 out_EME(n_samples, 1) = EncounterModelEvents;                                               % :222
 tm = self.temporal_map;
-s = struct('temporal_map', tm);
 idxEME = [find(tm(:, 1) == idxDH), find(tm(:, 1) == idxDPsi), find(tm(:, 1) == idxDV)] + 1; % :291
 for ii = 1:n_samples
-    ev = events(1:3, offsets(ii) + 1:offsets(ii + 1))';
-    out_events{ii} = ev;
-    out_samples{ii} = events2samples(out_inits(ii, :), ev);                                 % :283
-    controls = events2controls(out_inits(ii, :), ev, s);                                    % :286
-    controls = controls(:, [1 idxEME]);                                                     % :292
-    controls(:, 2) = controls(:, 2) / 60;                                                   % :295
-    controls(:, 3) = deg2rad(controls(:, 3));                                               % :296
-    controls(:, 4) = controls(:, 4) * 1.68780972222222;                                     % :297
-    out_EME(ii) = EncounterModelEvents('event', controls);                                  % :300
+    out_events{ii} = events(1:3, offsets(ii) + 1:offsets(ii + 1))';
+    out_EME(ii) = EncounterModelEvents('event', ctl{ii});                                  % :300
+    if p.Results.verify
+        controls = events2controls(out_inits(ii, :), out_events{ii}, struct('temporal_map', tm));   % :286
+        controls = controls(:, [1 idxEME]);                                                 % :292
+        controls(:, 2) = controls(:, 2) / 60;                                               % :295
+        controls(:, 3) = deg2rad(controls(:, 3));                                           % :296
+        controls(:, 4) = controls(:, 4) * 1.68780972222222;                                 % :297
+        assert(isequal(out_samples{ii}, events2samples(out_inits(ii, :), out_events{ii})) && ...
+               isequal(ctl{ii}, controls), 'sample_b200: GPU out_samples / out_EME differ from the reference (track %d)', ii);
+    end
 end
 
 if ~isnan(seed) && ~isempty(seed)
