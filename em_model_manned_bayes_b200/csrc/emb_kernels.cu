@@ -474,12 +474,14 @@ int launch_tracks(const DevModel& M, const SampleParams& P0, const TrackOut& O, 
     const bool hist = O.hist_initial || O.hist_transition;
     const int ev = O.ev_counts ? 1 : O.ev_words ? 2 : (O.x.xyz || O.x.is_good) ? 3 : 0;   // event / fused passes never carry histograms (emb_api.cpp)
     bool done = false;
-    // one launch per run of tracks whose global sample index shares its high word (spec v5: counter word 0 is launch-uniform)
+    // one launch per run of tracks whose global sample index shares its high word (spec v5: counter word 0 is launch-uniform);
+    // the last launch also covers the padding tracks up to the end of the last tile, which it zeroes (event passes skip them)
     SampleParams P = P0;
     for (int64_t s0 = 0; s0 < P0.n; s0 = P.s_end) {
         P.s_begin = s0;
         P.s_end = next_segment(P0.first_sample, s0, P0.n);
-        const unsigned grid = (unsigned)((P.s_end - P.s_begin + BLOCK - 1) / BLOCK);
+        const int64_t s_last = P.s_end == P0.n ? num_tiles(P0.n) * TRACK_TILE : P.s_end;
+        const unsigned grid = (unsigned)((s_last - P.s_begin + BLOCK - 1) / BLOCK);
         done = false;
 #define EMB_X(RS_, NG_, FAST_, ORD_)                                                                    \
     if (!done && rs == (RS_) && M.n_gated == (NG_) && fast == (FAST_) && ord == (ORD_)) {               \

@@ -161,7 +161,7 @@ typedef struct emb_track_out {
      * contiguous memory and a thread's stores sit at fixed offsets from one pointer:
      *     element (variable g, track s, second c) = [c/4][s/128][g][s%128][c%4]
      * column c (0-based) is the state during second c+1, i.e. out_samples{ii}(:, c+1) (events2samples.m:9-27);
-     * padding seconds of the last group are 0, padding tracks of the last tile are never written.  Buffer
+     * padding seconds of the last group and padding tracks of the last tile are 0.  Buffer
      * lengths (elements): emb_tracks_bins_len / emb_tracks_values_len */
     int8_t* bins;        /* [ceil(T/4)][ceil(n/128)][n_dyn][128][4]  1-based bins of the dynamic variables  nullable */
     float* values;       /* [ceil(T/4)][ceil(n/128)][n_timevarying][128][4] continuous values               nullable */
