@@ -16,6 +16,7 @@
 
 #include "../../include/emb200.h"
 #include "emb_events_expand.cuh"
+#include "emb_format.cuh"
 #include "emb_integrate.cuh"
 #include "emb_launch.h"
 #include "emb_loglik.cuh"
@@ -1228,6 +1229,106 @@ int emb_track_events_expand_packed(const emb_model* m, int64_t n, int32_t T, con
                                    int64_t* ctl_offsets, int64_t* total_rows) {
     return expand_impl(m, n, T, init_values, words, dts, offsets, true, opts, spec, samples, capacity, controls, ctl_offsets,
                        total_rows);
+}
+
+// ---- the text files of em_sample.m (emb_format.cuh) ------------------------------------------------------------------------
+int emb_format_em_sample(const emb_model* m, int64_t n, int32_t T, int64_t first_id, const double* init_values, const float* values,
+                         const emb_sample_opts* opts, int64_t capacity_initial, char* initial, int64_t* initial_offsets,
+                         int64_t capacity_transition, char* transition, int64_t* transition_offsets, int64_t* total_bytes) {
+    if (total_bytes) total_bytes[0] = total_bytes[1] = 0;
+    const bool want[2] = {initial || initial_offsets, transition || transition_offsets};
+    const int64_t cap[2] = {capacity_initial, capacity_transition};
+    char* text[2] = {initial, transition};
+    int64_t* offsets[2] = {initial_offsets, transition_offsets};
+    if (!m || !opts || n < 0 || T < 1 || cap[0] < 0 || cap[1] < 0 || (cap[0] > 0 && !initial) || (cap[1] > 0 && !transition) ||
+        (n > 0 && ((want[0] && !init_values) || (want[1] && !values))))
+        return set_err(EMB_E_ARG, "null or out-of-range argument");
+    if (opts->mem & ~0xFF) return set_err(EMB_E_ARG, "format_em_sample: EMB_MEM_ASYNC is not supported; the call is synchronous");
+    if (first_id < 1 || first_id > (1ll << 53) - n)
+        return set_err(EMB_E_ARG, "format_em_sample: ids first_id .. first_id + n - 1 must lie in 1 .. 2^53 - 1 (exact as doubles)");
+    const HostModel& H = *m->h;
+    emb::FormatParams P{};
+    int rc;
+    if (want[1]) {
+        if ((rc = need_transition(H))) return rc;
+        if ((int64_t)T * emb::FMT_ROW_MAX > (int64_t)UINT32_MAX)
+            return set_err(EMB_E_LIMIT, "format_em_sample: T too large for the 32-bit byte count of a track");
+        P.n_dyn = (int32_t)H.temporal_map.size();
+        P.n_tv = (int32_t)H.timevarying.size();
+        for (int j = 0; j < P.n_dyn; ++j)
+            P.cols[j] = (int32_t)(std::find(H.timevarying.begin(), H.timevarying.end(), H.temporal_map[(size_t)j].first) -
+                                  H.timevarying.begin());
+    }
+    if (!want[0] && !want[1]) return 0;
+    if (n == 0 && opts->mem == EMB_MEM_HOST) {
+        for (int f = 0; f < 2; ++f)
+            if (offsets[f]) offsets[f][0] = 0;
+        return 0;
+    }
+    Call call;
+    if ((rc = call.open(opts, nullptr))) return rc;
+    const cudaStream_t st = call.st;
+    Stager& sg = call.sg;
+    if (n == 0) {   // device offsets
+        const int64_t zero = 0;
+        for (int f = 0; f < 2; ++f)
+            if (offsets[f]) CU(cudaMemcpyAsync(offsets[f], &zero, 8, cudaMemcpyHostToDevice, st));
+        CU(cudaStreamSynchronize(st));
+        return 0;
+    }
+    P.n = n;
+    P.T = T;
+    P.n_initial = H.n_initial;
+    P.first_id = first_id;
+    const void* d_in = nullptr;
+    if (want[0]) {
+        if ((rc = sg.in(init_values, (size_t)n * (size_t)H.n_initial * 8, &d_in))) return rc;
+        P.init_values = (const double*)d_in;
+    }
+    if (want[1]) {
+        if ((rc = sg.in(values, (size_t)emb_tracks_values_len(m, n, T) * 4, &d_in))) return rc;
+        P.values = (const float*)d_in;
+    }
+    if ((rc = call.status_word(&P.status))) return rc;
+    // count pass and prefix sum of each text: bytes per track into its offsets, the totals to the host
+    Tmp counts, scratch, off_tmp[2];
+    CU(tmp_alloc(&counts.p, (size_t)n * 4, st));
+    CU(tmp_alloc(&scratch.p, (size_t)emb::scan_scratch_len(n) * 8, st));
+    P.counts = (uint32_t*)counts.p;
+    long long* d_off[2] = {nullptr, nullptr};
+    long long total[2] = {0, 0};
+    for (int f = 0; f < 2; ++f) {
+        if (!want[f]) continue;
+        if ((rc = sg.out(offsets[f], (size_t)(n + 1) * 8, false, (void**)&d_off[f]))) return rc;
+        if (!d_off[f]) {
+            CU(tmp_alloc(&off_tmp[f].p, (size_t)(n + 1) * 8, st));
+            d_off[f] = (long long*)off_tmp[f].p;
+        }
+        cudaError_t e = (cudaError_t)emb::launch_format(P, f == 1, true, st);
+        if (e != cudaSuccess) return cuda_fail(e, f ? "launch k_format_transition_count" : "launch k_format_initial_count");
+        e = (cudaError_t)emb::launch_scan_counts(P.counts, d_off[f], n, (long long*)scratch.p, st);
+        if (e != cudaSuccess) return cuda_fail(e, "launch k_scan_counts");
+        CU(cudaMemcpyAsync(&total[f], d_off[f] + n, 8, cudaMemcpyDeviceToHost, st));
+    }
+    int32_t flag = 0;
+    CU(cudaMemcpyAsync(&flag, P.status, 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (total_bytes) total_bytes[0] = total[0], total_bytes[1] = total[1];
+    if (flag) return set_err(EMB_E_ARG, "format_em_sample: a value is not finite (inf or NaN)");
+    if (total[0] > cap[0] || total[1] > cap[1]) {
+        if ((rc = sg.finish())) return rc;   // the offsets are valid
+        return set_err(EMB_E_LIMIT, "text buffer too small: " + std::to_string(total[0]) + " bytes of initial text and " +
+                                        std::to_string(total[1]) + " bytes of transition text needed");
+    }
+    cudaError_t e = cudaSuccess;
+    for (int f = 0; f < 2 && e == cudaSuccess; ++f) {
+        if (!text[f] || !total[f]) continue;
+        if ((rc = sg.out(text[f], (size_t)total[f], false, (void**)&P.text))) return rc;
+        P.offsets = d_off[f];
+        e = (cudaError_t)emb::launch_format(P, f == 1, false, st);
+    }
+    int32_t status;
+    return call.finish(e, "k_format_initial / k_format_transition", status);
 }
 
 // IntegrateParams from emb_integrate_opts (labels -> tile ordinals, unit ratios); 0 or an error code

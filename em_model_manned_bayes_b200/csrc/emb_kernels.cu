@@ -11,6 +11,7 @@
 #include "emb_device.cuh"
 #include "emb_events_expand.cuh"
 #include "emb_fast.cuh"
+#include "emb_format.cuh"
 #include "emb_initial.cuh"
 #include "emb_launch.h"
 #include "emb_loglik.cuh"
@@ -370,6 +371,31 @@ __global__ void __launch_bounds__(EE_BLOCK) k_events_expand(const __grid_constan
     events_expand_track<PACKED>(M, P, R, s, ExpandLanes{(int)(threadIdx.x & 31)}, sh[threadIdx.x >> 5]);
 }
 
+// the text files of em_sample.m (emb_format.cuh): one warp per track, count pass and write pass of each file.  128 registers
+// (16 warps an SM) hold the digit generation without spills; the default heuristic spills it.
+constexpr int FMT_BLOCK = 128;
+constexpr int FMT_MAXNREG = 128;
+
+template <bool TRANS>
+__device__ __forceinline__ void format_count(const FormatParams& P) {
+    const int64_t s = (int64_t)blockIdx.x * (FMT_BLOCK / 32) + (threadIdx.x >> 5);
+    if (s >= P.n) return;
+    const ExpandLanes L{(int)(threadIdx.x & 31)};
+    const uint32_t bytes = format_track<TRANS, false>(P, s, L, nullptr);
+    if (L.lane == 0) P.counts[s] = bytes;
+}
+template <bool TRANS>
+__device__ __forceinline__ void format_write(const FormatParams& P) {
+    __shared__ char stage[FMT_BLOCK / 32][FMT_STAGE_BYTES];
+    const int64_t s = (int64_t)blockIdx.x * (FMT_BLOCK / 32) + (threadIdx.x >> 5);
+    if (s >= P.n) return;
+    format_track<TRANS, true>(P, s, ExpandLanes{(int)(threadIdx.x & 31)}, stage[threadIdx.x >> 5]);
+}
+__global__ void __maxnreg__(FMT_MAXNREG) k_format_initial_count(const __grid_constant__ FormatParams P) { format_count<false>(P); }
+__global__ void __maxnreg__(FMT_MAXNREG) k_format_initial(const __grid_constant__ FormatParams P) { format_write<false>(P); }
+__global__ void __maxnreg__(FMT_MAXNREG) k_format_transition_count(const __grid_constant__ FormatParams P) { format_count<true>(P); }
+__global__ void __maxnreg__(FMT_MAXNREG) k_format_transition(const __grid_constant__ FormatParams P) { format_write<true>(P); }
+
 }  // namespace
 
 int launch_publish(const long long* total, const int32_t* flag, long long* mapped_dst, void* stream) {
@@ -578,6 +604,21 @@ int launch_events_expand(const DevModel& M, const ExpandParams& P, const EventRo
     } else {
         if (packed) k_events_expand<true><<<grid, EE_BLOCK, 0, st>>>(M, P, R);
         else k_events_expand<false><<<grid, EE_BLOCK, 0, st>>>(M, P, R);
+    }
+    g_launch_count.fetch_add(1);
+    return (int)cudaGetLastError();
+}
+
+int launch_format(const FormatParams& P, bool transition, bool count, void* stream) {
+    if (P.n <= 0) return 0;
+    const unsigned grid = (unsigned)((P.n + FMT_BLOCK / 32 - 1) / (FMT_BLOCK / 32));
+    cudaStream_t st = (cudaStream_t)stream;
+    if (transition) {
+        if (count) k_format_transition_count<<<grid, FMT_BLOCK, 0, st>>>(P);
+        else k_format_transition<<<grid, FMT_BLOCK, 0, st>>>(P);
+    } else {
+        if (count) k_format_initial_count<<<grid, FMT_BLOCK, 0, st>>>(P);
+        else k_format_initial<<<grid, FMT_BLOCK, 0, st>>>(P);
     }
     g_launch_count.fetch_add(1);
     return (int)cudaGetLastError();

@@ -42,6 +42,9 @@ int launch_loglik_events(const DevModel& M, const LoglikParams& P, const EventRo
 // event lists -> samples and control rows (emb_events_expand.cuh): the count pass (P.counts) or the write pass
 struct ExpandParams;
 int launch_events_expand(const DevModel& M, const ExpandParams& P, const EventRows& R, bool packed, bool count, void* stream);
+// the text files of em_sample.m (emb_format.cuh): the count pass (P.counts) or the write pass of initial.txt or transition.txt
+struct FormatParams;
+int launch_format(const FormatParams& P, bool transition, bool count, void* stream);
 
 // terminal trajectory chains (emb_terminal.cu): 4 chains per encounter
 struct TermParams;

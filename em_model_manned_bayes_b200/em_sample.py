@@ -8,12 +8,11 @@ Writes the same two text files: `initial.txt` ("id <labels>" header, one row `id
 em_sample.m:59-66,88-92) and `transition.txt` ("initial_id t <labels of the (t+1) variables>" header, one row
 `id t x_dyn...` per sample and second, :68-74,94-100), numbers formatted with C's %g like fprintf.
 The samples come from emb_sample_tracks (dense compact output: column c is `samples(:, c+1)` of
-events2samples.m), so nothing is sampled on the CPU.  `parms.prior = 'constant'` (em_sample.m:50) is an error in
+events2samples.m) and stay on the device, where emb_format_em_sample formats them; only the text crosses PCIe.
+`device` (default: the current CUDA device) runs both.  `parms.prior = 'constant'` (em_sample.m:50) is an error in
 the reference at HEAD (EncounterModel.m:194-203 accepts only numbers and 'dbe', SURVEY F8); the intended
 zero prior is used.  The random stream is the keyed Philox stream with seed `rng_seed`, not MATLAB's twister."""
 from __future__ import annotations
-
-import numpy as np
 
 from .model import EncounterModel
 
@@ -27,25 +26,15 @@ def em_sample(parameters_filename: str, initial_output_filename: str, transition
     if start is not None and len(start):
         parms.start = list(start)                                        # em_sample.m:53-55
     n, T = int(num_initial_samples), int(num_transition_samples)
-    dyn_t = [int(v) for v in parms.temporal_map[:, 0]]
-    tv = list(parms.timevarying_vars)
-    cols = [tv.index(v) for v in dyn_t]
-    with open(initial_output_filename, "w", encoding="utf-8") as fi, \
-            open(transition_output_filename, "w", encoding="utf-8") as ft:
-        fi.write("id " + "".join("%s " % l for l in parms.labels_initial) + "\n")                      # :59-66
-        ft.write("initial_id t " + "".join("%s " % parms.labels_transition[int(k) - 1]
-                                           for k in parms.temporal_map[:, 1]) + "\n")                  # :68-74
+    import torch
+    dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+    with open(initial_output_filename, "wb") as fi, open(transition_output_filename, "wb") as ft:
+        fi.write(("id " + "".join("%s " % l for l in parms.labels_initial) + "\n").encode("utf-8"))                # :59-66
+        ft.write(("initial_id t " + "".join("%s " % parms.labels_transition[int(k) - 1]
+                                            for k in parms.temporal_map[:, 1]) + "\n").encode("utf-8"))           # :68-74
         for first in range(0, n, chunk):
             m = min(chunk, n - first)
-            res = parms.sample_tracks(m, T, seed=rng_seed, first_sample=first, device=device, want_bins=False)
-            iv = res.init_values
-            vals = res.values
-            if device is not None:
-                iv, vals = iv.cpu().numpy(), vals.cpu().numpy()
-            iv = np.asarray(iv).T                                        # (m, n_initial) = samples(:, 1)
-            vals = np.asarray(vals, dtype=np.float64)[:, cols, :]        # (m, n_dyn, T)
-            for k in range(m):
-                ii = first + k + 1
-                fi.write("%d " % ii + " ".join("%g" % x for x in iv[k]) + "\n")                        # :88-92
-                rows = vals[k].T
-                ft.write("".join("%g %g " % (ii, j) + " ".join("%g" % x for x in rows[j]) + "\n" for j in range(T)))  # :94-100
+            res = parms.sample_tracks(m, T, seed=rng_seed, first_sample=first, device=dev, want_bins=False)
+            text_i, _, text_t, _ = parms.format_em_sample(res, first_id=first + 1)                            # :88-100
+            fi.write(text_i.cpu().numpy().tobytes())
+            ft.write(text_t.cpu().numpy().tobytes())

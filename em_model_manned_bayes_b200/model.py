@@ -312,6 +312,14 @@ class EncounterModel:
                np.uint64: torch.int64, np.int64: torch.int64}[dtype]
         return torch.zeros(shape, dtype=tdt, device=like)
 
+    @staticmethod
+    def _empty_bytes(count, like):
+        """An uninitialised uint8 buffer (text that a call overwrites): numpy, or torch on `like` device."""
+        if like is None:
+            return np.empty((count,), dtype=np.uint8)
+        import torch
+        return torch.empty((count,), dtype=torch.uint8, device=like)
+
     # -- sampling ----------------------------------------------------------------------------------
     def sample_initial(self, n: int, seed: int = 0, first_sample: int = 0, start=None, opts=None, device=None,
                        want_values=True, want_attempts=True, out=None, enqueue_only: bool = False, values_fp32: bool = False):
@@ -551,6 +559,57 @@ class EncounterModel:
             rows = self._alloc((0, 1 + k), np.float64, like)
         L.check(rc)
         return samples, ControlsResult(rows=rows, offsets=ctl_off)
+
+    # -- the text files of em_sample.m (emb200.h: emb_format_em_sample) --------------------------------------------------
+    def format_em_sample(self, init_values=None, values_tiled=None, T: Optional[int] = None, first_id: int = 1,
+                         n: Optional[int] = None, device=None):
+        """initial.txt and transition.txt of em_sample.m without their header lines, formatted on the device exactly as
+        printf's "%g" (and "%d" for the id of initial.txt) formats them.  `init_values`: (n_initial, n) float64, or a whole
+        `TrackResult` (then `values_tiled`, `T` and `n` come from it); `values_tiled`: the flat dense tiles of `sample_tracks`
+        for the same n and T.  A text whose input is None is skipped (then give `n`).  Track s has id first_id + s.
+        Returns (initial, initial_offsets, transition, transition_offsets): uint8 text and int64 [n+1] offsets, None for a
+        skipped text.  numpy in, numpy out (computed on `device`); torch CUDA tensors in, tensors on their device out."""
+        if isinstance(init_values, TrackResult):
+            r = init_values
+            init_values, values_tiled, T, n = r.init_values, r.values_tiled, r.T, r.n
+        if T is None or (init_values is None and (values_tiled is None or n is None)):
+            raise L.EmbError(L.EMB_E_ARG, "format_em_sample: T, and init_values or n, are required")
+        arrays = [a for a in (init_values, values_tiled) if a is not None]
+        o, like = self._score_call(arrays, device, False)
+        if init_values is not None:
+            if init_values.shape[0] != self.n_initial:
+                raise L.EmbError(L.EMB_E_ARG, "format_em_sample: init_values must be n_initial x n")
+            n = int(init_values.shape[1])
+        n, T = int(n), int(T)
+        lib = L.lib()
+        if like is None:
+            iv = None if init_values is None else np.ascontiguousarray(init_values, dtype=np.float64)
+            vt = None if values_tiled is None else np.ascontiguousarray(values_tiled, dtype=np.float32).reshape(-1)
+        else:
+            import torch
+            iv = None if init_values is None else init_values.to(torch.float64).contiguous()
+            vt = None if values_tiled is None else values_tiled.to(torch.float32).contiguous().reshape(-1)
+        if vt is not None and int(vt.shape[0]) != int(lib.emb_tracks_values_len(self._h, n, T)):
+            raise L.EmbError(L.EMB_E_ARG, "format_em_sample: values_tiled must have emb_tracks_values_len(n, T) elements")
+        off = [self._alloc((n + 1,), np.int64, like) if a is not None else None for a in (iv, vt)]
+        totals = (C.c_int64 * 2)()
+
+        def call(caps, bufs):
+            return lib.emb_format_em_sample(self._h, n, T, int(first_id), _ptr(iv), _ptr(vt), C.byref(o), caps[0], _ptr(bufs[0]),
+                                            _ptr(off[0]), caps[1], _ptr(bufs[1]), _ptr(off[1]), totals)
+
+        # One call into buffers of the longest possible text (emb_format.cuh: a "%g" has at most 13 bytes, an id's "%d" at
+        # most 16 below 2^53), so the count pass runs once; the exact totals and a second call only if that bound were short.
+        bound = [n * (17 + 14 * self.n_initial) if off[0] is not None else 0,
+                 n * T * (28 + 14 * self.n_dyn) if off[1] is not None else 0]
+        bufs = [self._empty_bytes(bound[f], like) if off[f] is not None else None for f in range(2)]
+        rc = call(bound, bufs)
+        if rc == L.EMB_E_LIMIT:
+            bufs = [self._empty_bytes(int(totals[f]), like) if off[f] is not None else None for f in range(2)]
+            rc = call((int(totals[0]), int(totals[1])), bufs)
+        L.check(rc)
+        bufs = [None if b is None else b[:int(totals[f])] for f, b in enumerate(bufs)]
+        return bufs[0], off[0], bufs[1], off[1]
 
 
 def async_status(device: int = -1) -> None:

@@ -394,6 +394,26 @@ int emb_track_events_expand_packed(const emb_model* m, int64_t n, int32_t T, con
                                    const emb_controls_spec* spec, double* samples, int64_t capacity, double* controls,
                                    int64_t* ctl_offsets, int64_t* total_rows);
 
+/* ---- the legacy text files of em_sample.m:59-100 (initial.txt and transition.txt without their header lines), formatted on
+ *      the device from the outputs of emb_sample_tracks ------------------------------------------------------------------- */
+/* Numbers are printed exactly as C's printf / MATLAB's fprintf print them on Linux: "%g" is the correctly rounded 6-digit
+ * decimal of the exact binary value (ties to even), for every finite double.  Track s has id first_id + s.
+ *   initial.txt, one row per track:  "%d" of the id, " %g" of each of the n_initial values of init_values, "\n"
+ *   transition.txt, T rows per track, t = 0 .. T-1:  "%g %g" of (id, t), " %g" of the value of each dynamic variable
+ *     (temporal_map(:,1) order) in second t, read from the dense tiles and widened from fp32, "\n"
+ * init_values: double [n_initial][n] (emb_track_out.init_values); values: the dense tiles of emb_sample_tracks for the same n
+ * and T (emb_tracks_values_len(m, n, T) floats).  Track s of a text is text[offsets[s] .. offsets[s+1]); offsets: int64 [n+1].
+ * A text is skipped when its buffer and its offsets are both NULL (its input may then be NULL too).  total_bytes[2] (host,
+ * nullable) receives both totals (0 for a skipped text).  If a total exceeds its capacity, no text is written, the offsets and
+ * totals are, and EMB_E_LIMIT is returned: capacity 0 with a NULL buffer sizes the call.
+ * Only mem, device and stream of `opts` are read; every buffer is in opts->mem memory.  EMB_E_ARG, found on the device: a value
+ * that is not finite (libc and Python spell inf and NaN differently; the sampler writes none).  Refused before the device is
+ * touched: EMB_MEM_ASYNC, T < 1, first_id < 1 or first_id + n - 1 >= 2^53 (ids must be exact doubles for "%g"), transition
+ * text for a model without a transition network ("dynvar:empty"); EMB_E_LIMIT when T rows of a track could exceed 2^32 bytes. */
+int emb_format_em_sample(const emb_model* m, int64_t n, int32_t T, int64_t first_id, const double* init_values, const float* values,
+                         const emb_sample_opts* opts, int64_t capacity_initial, char* initial, int64_t* initial_offsets,
+                         int64_t capacity_transition, char* transition, int64_t* transition_offsets, int64_t* total_bytes);
+
 /* ---- misc ------------------------------------------------------------------------------------- */
 int emb_host_alloc(void** p, int64_t bytes); /* pinned host memory */
 int emb_host_free(void* p);

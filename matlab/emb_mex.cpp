@@ -35,6 +35,9 @@
 //          ur_heading, min_speed, max_speed;  xyz: n x (T+1) x 3 single, is_good: n x 1 uint8
 //   [xyz, is_good, out_inits] = emb_mex('sample_tracks_xyz', h, seed, first, n, T, opts, iopts)
 //          sampling and the loop of sample2track.m:188-244 in one kernel pass (no dense tiles); outputs as above
+//   [initial, transition] = emb_mex('em_sample_text', h, seed, first, n, T, opts)   % em_sample.m:88-100 on the GPU
+//          the rows of initial.txt and transition.txt (without header lines) as uint8 row vectors, ids first+1 .. first+n,
+//          numbers as fprintf's "%g" prints them (emb_format_em_sample); matlab/em_sample_b200.m writes the files
 //   [total, per_var] = emb_mex('loglik_initial', h, bins)              % log p of initial states (emb_loglik_initial)
 //          bins: n x n_initial int8 (1-based); total n x 1, per_var n x n_initial double
 //   [initial, transition] = emb_mex('loglik_tracks', h, init_bins, bins, T, correct_dbn)   % log p of tracks
@@ -300,6 +303,35 @@ void mexFunction(int nlhs, mxArray* plhs[], int nrhs, const mxArray* prhs[]) {
         if (nlhs > 1) plhs[1] = bins; else mxDestroyArray(bins);
         if (nlhs > 2) plhs[2] = vals; else mxDestroyArray(vals);
         if (nlhs > 3) plhs[3] = att; else mxDestroyArray(att);
+    } else if (c == "em_sample_text") {                           // em_sample.m:88-100: the rows of initial.txt and transition.txt
+        // [initial, transition] = emb_mex('em_sample_text', h, seed, first, n, T, opts): uint8 row vectors (the files without
+        // their header lines), tracks first .. first+n-1 with ids first+1 .. first+n, numbers formatted on the GPU as "%g"
+        emb_rng rng{(uint64_t)mxGetScalar(prhs[2]), (uint64_t)mxGetScalar(prhs[3])};
+        const int64_t n = (int64_t)mxGetScalar(prhs[4]);
+        const int32_t T = (int32_t)mxGetScalar(prhs[5]);
+        emb_sample_opts o;
+        fill_opts(nrhs > 6 ? prhs[6] : nullptr, ni, &o);
+        // The MEX side has host buffers only (the ABI hands out no device memory), so the samples land in host vectors and
+        // emb_format_em_sample stages them back to the device in each of its two calls: about 100 MB of extra PCIe traffic per
+        // 65,536 x 60 s chunk of cor_v1.  The Python em_sample keeps them on the device and moves only the text.
+        std::vector<double> inits((size_t)n * (size_t)ni);
+        std::vector<float> vals((size_t)emb_tracks_values_len(m, n, T));
+        emb_track_out out{};
+        out.init_values = inits.data();
+        out.values = vals.data();
+        CHECK(emb_sample_tracks(m, &rng, n, T, &o, &out));
+        std::vector<int64_t> off_i((size_t)n + 1), off_t((size_t)n + 1);
+        int64_t total[2] = {0, 0};
+        const int64_t first_id = (int64_t)rng.first_sample + 1;
+        const int rc = emb_format_em_sample(m, n, T, first_id, inits.data(), vals.data(), &o, 0, nullptr, off_i.data(), 0, nullptr,
+                                            off_t.data(), total);   // sizes both texts
+        if (rc != 0 && rc != EMB_E_LIMIT) fail(rc);
+        plhs[0] = mxCreateNumericMatrix(1, (mwSize)total[0], mxUINT8_CLASS, mxREAL);
+        mxArray* tr = mxCreateNumericMatrix(1, (mwSize)total[1], mxUINT8_CLASS, mxREAL);
+        if (rc == EMB_E_LIMIT)
+            CHECK(emb_format_em_sample(m, n, T, first_id, inits.data(), vals.data(), &o, total[0], (char*)mxGetData(plhs[0]),
+                                       off_i.data(), total[1], (char*)mxGetData(tr), off_t.data(), total));
+        if (nlhs > 1) plhs[1] = tr; else mxDestroyArray(tr);
     } else if (c == "loglik_initial") {                           // log p of initial states (emb200.h: emb_loglik_initial)
         // [total, per_var] = emb_mex('loglik_initial', h, bins)   bins: n x n_initial int8 (== the ABI's [n_initial][n])
         const int64_t n = (int64_t)mxGetM(prhs[2]);
