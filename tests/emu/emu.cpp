@@ -152,7 +152,7 @@ int emu_sample_tracks(void* h, uint64_t seed, uint64_t first, int64_t n, int32_t
         const uint32_t rs = fast_shape_of(D);
         const bool fast = D.fast != 0;
         static FastShared S;
-        fast_fill_shared(D, S, 0, 1);
+        if (rs) fast_fill_shared(D, S, 0, 1);   // only a fast shape fits FastShared (FAST_MAX_EDGES), as on the device
 #define EMB_X(RS_, NG_, FAST_, ORD_)                                                   \
     if (!done && rs == (RS_) && D.n_gated == (NG_) && fast == (FAST_) && order_code(D) == (ORD_)) { \
         static CallTable<NG_> U;                                                      \
@@ -189,8 +189,8 @@ int emu_sample_track_events(void* h, uint64_t seed, uint64_t first, int64_t n, i
     std::vector<long long> off((size_t)n + 1);
     HostHist hh{nullptr, nullptr};
     static FastShared S;
-    fast_fill_shared(D, S, 0, 1);
     const uint32_t rs = g_use_fast ? fast_shape_of(D) : 0;
+    if (rs) fast_fill_shared(D, S, 0, 1);       // only a fast shape fits FastShared (FAST_MAX_EDGES), as on the device
     const bool fast = D.fast != 0;
     int max_bins = 0;
     for (int g = 0; g < D.n_gated; ++g) max_bins = std::max(max_bins, (int)D.init[D.gated_var[g]].r);
