@@ -172,6 +172,8 @@ def lib():
         "emb_track_events_expand_packed": (C.c_int, [vp, i64, i32, vp, vp, vp, vp, P(SampleOpts), P(ControlsSpec), vp, i64, vp, vp,
                                                      P(i64)]),
         "emb_format_em_sample": (C.c_int, [vp, i64, i32, i64, vp, vp, P(SampleOpts), i64, vp, vp, i64, vp, vp, P(i64)]),
+        "emb_format_tracks_csv": (C.c_int, [i64, i32, vp, vp, P(SampleOpts), i64, vp, vp, P(i64)]),
+        "emb_parse_table": (C.c_int, [vp, i64, i32, P(SampleOpts), i64, vp, P(i64), P(i64)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(L, name)  # AttributeError if a declared symbol is missing
@@ -191,6 +193,7 @@ EXPORTED = [
     "emb_terminal_screen", "emb_loglik_initial", "emb_loglik_tracks",
     "emb_loglik_track_events", "emb_loglik_track_events_packed",
     "emb_track_events_expand", "emb_track_events_expand_packed", "emb_format_em_sample",
+    "emb_format_tracks_csv", "emb_parse_table",
 ]
 TRAJ_FIELDS = ("x_nm", "y_nm", "z_ft", "heading_deg", "v_ft_s")
 

@@ -22,6 +22,7 @@
 #include "emb_loglik.cuh"
 #include "emb_loglik_events.cuh"
 #include "emb_model.h"
+#include "emb_parse.cuh"
 
 using emb::DevModel;
 using emb::HostModel;
@@ -1329,6 +1330,153 @@ int emb_format_em_sample(const emb_model* m, int64_t n, int32_t T, int64_t first
     }
     int32_t status;
     return call.finish(e, "k_format_initial / k_format_transition", status);
+}
+
+// ---- the CSV rows of sample2track.m (emb_format.cuh) --------------------------------------------------------------------------
+int emb_format_tracks_csv(int64_t n, int32_t T, const float* xyz, const uint8_t* mask, const emb_sample_opts* opts, int64_t capacity,
+                          char* text, int64_t* offsets, int64_t* total_bytes) {
+    if (total_bytes) *total_bytes = 0;
+    if (!opts || n < 0 || T < 0 || capacity < 0 || (capacity > 0 && !text) || (n > 0 && !xyz))
+        return set_err(EMB_E_ARG, "null or out-of-range argument");
+    if (opts->mem & ~0xFF) return set_err(EMB_E_ARG, "format_tracks_csv: EMB_MEM_ASYNC is not supported; the call is synchronous");
+    if (((int64_t)T + 1) * emb::FMT_CSV_ROW_MAX > (int64_t)UINT32_MAX)
+        return set_err(EMB_E_LIMIT, "format_tracks_csv: T too large for the 32-bit byte count of a track");
+    if (n == 0 && opts->mem == EMB_MEM_HOST) {
+        if (offsets) offsets[0] = 0;
+        return 0;
+    }
+    Call call;
+    int rc;
+    if ((rc = call.open(opts, nullptr))) return rc;
+    const cudaStream_t st = call.st;
+    Stager& sg = call.sg;
+    if (n == 0) {   // device offsets
+        const int64_t zero = 0;
+        if (offsets) CU(cudaMemcpyAsync(offsets, &zero, 8, cudaMemcpyHostToDevice, st));
+        CU(cudaStreamSynchronize(st));
+        return 0;
+    }
+    emb::CsvParams P{};
+    P.n = n;
+    P.T = T;
+    const void* d_in = nullptr;
+    if ((rc = sg.in(xyz, (size_t)3 * ((size_t)T + 1) * (size_t)n * 4, &d_in))) return rc;
+    P.xyz = (const float*)d_in;
+    if ((rc = sg.in(mask, (size_t)n, &d_in))) return rc;
+    P.mask = (const uint8_t*)d_in;
+    if ((rc = call.status_word(&P.status))) return rc;
+    // count pass and prefix sum: bytes per track into the offsets, the total to the host
+    Tmp counts, scratch, off_tmp;
+    CU(tmp_alloc(&counts.p, (size_t)n * 4, st));
+    CU(tmp_alloc(&scratch.p, (size_t)emb::scan_scratch_len(n) * 8, st));
+    P.counts = (uint32_t*)counts.p;
+    long long* d_off = nullptr;
+    if ((rc = sg.out(offsets, (size_t)(n + 1) * 8, false, (void**)&d_off))) return rc;
+    if (!d_off) {
+        CU(tmp_alloc(&off_tmp.p, (size_t)(n + 1) * 8, st));
+        d_off = (long long*)off_tmp.p;
+    }
+    cudaError_t e = (cudaError_t)emb::launch_format_csv(P, true, st);
+    if (e != cudaSuccess) return cuda_fail(e, "launch k_format_csv_count");
+    e = (cudaError_t)emb::launch_scan_counts(P.counts, d_off, n, (long long*)scratch.p, st);
+    if (e != cudaSuccess) return cuda_fail(e, "launch k_scan_counts");
+    long long total = 0;
+    int32_t flag = 0;
+    CU(cudaMemcpyAsync(&total, d_off + n, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&flag, P.status, 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (total_bytes) *total_bytes = total;
+    if (flag) return set_err(EMB_E_ARG, "format_tracks_csv: a coordinate of an unmasked track is not finite (inf or NaN)");
+    if (total > capacity) {
+        if ((rc = sg.finish())) return rc;   // the offsets are valid
+        return set_err(EMB_E_LIMIT, "text buffer too small: " + std::to_string(total) + " bytes of CSV text needed");
+    }
+    e = cudaSuccess;
+    if (text && total) {
+        if ((rc = sg.out(text, (size_t)total, false, (void**)&P.text))) return rc;
+        P.offsets = d_off;
+        e = (cudaError_t)emb::launch_format_csv(P, false, st);
+    }
+    int32_t status;
+    return call.finish(e, "k_format_csv", status);
+}
+
+// ---- decimal text tables (emb_parse.cuh) --------------------------------------------------------------------------------------
+int emb_parse_table(const char* text, int64_t bytes, int32_t cols, const emb_sample_opts* opts, int64_t capacity_rows, double* values,
+                    int64_t* total_rows, int64_t* bad_line) {
+    if (total_rows) *total_rows = 0;
+    if (bad_line) *bad_line = 0;
+    if (!opts || bytes < 0 || cols < 1 || cols > emb::PARSE_MAX_COLS || capacity_rows < 0 || (capacity_rows > 0 && !values) ||
+        (bytes > 0 && !text))
+        return set_err(EMB_E_ARG, "parse_table: null or out-of-range argument (bytes >= 0, cols in 1 .. 256)");
+    if (opts->mem & ~0xFF) return set_err(EMB_E_ARG, "parse_table: EMB_MEM_ASYNC is not supported; the call is synchronous");
+    if (bytes == 0) return 0;
+    Call call;
+    int rc;
+    if ((rc = call.open(opts, nullptr))) return rc;
+    const cudaStream_t st = call.st;
+    Stager& sg = call.sg;
+    emb::ParseParams P{};
+    const void* d_text = nullptr;
+    if ((rc = sg.in(text, (size_t)bytes, &d_text))) return rc;
+    P.text = (const char*)d_text;
+    P.bytes = bytes;
+    P.cols = cols;
+    P.aligned = ((uintptr_t)d_text & 15) == 0;
+    P.chunks = (bytes + emb::parse_chunk_bytes() - 1) / emb::parse_chunk_bytes();
+    // line discovery: newlines per chunk, their prefix sum, the number of lines to the host
+    Tmp chunk_nl, nl_before, scratch_c, starts, rows, row_of, scratch_l, err;
+    CU(tmp_alloc(&chunk_nl.p, (size_t)P.chunks * 4, st));
+    CU(tmp_alloc(&nl_before.p, (size_t)(P.chunks + 1) * 8, st));
+    CU(tmp_alloc(&scratch_c.p, (size_t)emb::scan_scratch_len(P.chunks) * 8, st));
+    P.chunk_newlines = (uint32_t*)chunk_nl.p;
+    P.newlines_before = (const long long*)nl_before.p;
+    cudaError_t e = (cudaError_t)emb::launch_parse(P, 0, st);
+    if (e != cudaSuccess) return cuda_fail(e, "launch k_parse_newline_count");
+    e = (cudaError_t)emb::launch_scan_counts(P.chunk_newlines, (long long*)nl_before.p, P.chunks, (long long*)scratch_c.p, st);
+    if (e != cudaSuccess) return cuda_fail(e, "launch k_scan_counts");
+    long long newlines = 0;
+    CU(cudaMemcpyAsync(&newlines, (const long long*)nl_before.p + P.chunks, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    P.lines = newlines + 1;
+    // line starts, the checks of every line (blank lines give no row), the prefix sum of the rows
+    CU(tmp_alloc(&starts.p, (size_t)(P.lines + 1) * 8, st));
+    CU(tmp_alloc(&rows.p, (size_t)P.lines * 4, st));
+    CU(tmp_alloc(&row_of.p, (size_t)(P.lines + 1) * 8, st));
+    CU(tmp_alloc(&scratch_l.p, (size_t)emb::scan_scratch_len(P.lines) * 8, st));
+    CU(tmp_alloc(&err.p, 8, st));
+    CU(cudaMemsetAsync(err.p, 0xFF, 8, st));
+    P.starts = (long long*)starts.p;
+    P.rows = (uint32_t*)rows.p;
+    P.row_of = (const long long*)row_of.p;
+    P.error = (unsigned long long*)err.p;
+    e = (cudaError_t)emb::launch_parse(P, 1, st);
+    if (e != cudaSuccess) return cuda_fail(e, "launch k_parse_line_starts");
+    e = (cudaError_t)emb::launch_parse(P, 2, st);
+    if (e != cudaSuccess) return cuda_fail(e, "launch k_parse_lines");
+    e = (cudaError_t)emb::launch_scan_counts(P.rows, (long long*)row_of.p, P.lines, (long long*)scratch_l.p, st);
+    if (e != cudaSuccess) return cuda_fail(e, "launch k_scan_counts");
+    long long total = 0;
+    unsigned long long word = 0;
+    CU(cudaMemcpyAsync(&total, P.row_of + P.lines, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&word, err.p, 8, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (word != emb::PARSE_NO_ERROR) {
+        const long long line = (long long)(word >> 2);
+        if (bad_line) *bad_line = line;
+        static const char* what[4] = {"a field is not a decimal number", "a field has more than 19 significant digits",
+                                      "a value rounds to infinity", "wrong number of fields"};
+        return set_err(EMB_E_ARG, "parse_table: line " + std::to_string(line) + " of the text: " + what[word & 3] +
+                                      ((word & 3) == emb::PARSE_E_FIELDS ? " (" + std::to_string(cols) + " expected)" : std::string()));
+    }
+    if (total_rows) *total_rows = total;
+    if (total > capacity_rows)
+        return set_err(EMB_E_LIMIT, "values buffer too small: " + std::to_string(total) + " rows needed");
+    if (!total) return 0;
+    if ((rc = sg.out(values, (size_t)total * (size_t)cols * 8, false, (void**)&P.values))) return rc;
+    e = (cudaError_t)emb::launch_parse(P, 3, st);
+    if (e != cudaSuccess) return cuda_fail(e, "launch k_parse_values");
+    return sg.finish();
 }
 
 // IntegrateParams from emb_integrate_opts (labels -> tile ordinals, unit ratios); 0 or an error code

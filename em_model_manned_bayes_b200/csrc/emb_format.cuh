@@ -1,5 +1,6 @@
 // emb_format.cuh -- the legacy text files of em_sample.m (initial.txt, transition.txt) formatted on the device: C's "%g" of a
-// double and "%d" of an int64, and the per-track routines of k_format_{initial,transition}[_count] (emb_kernels.cu).
+// double and "%d" of an int64, and the per-track routines of k_format_{initial,transition}[_count] (emb_kernels.cu); and the CSV
+// rows of sample2track.m ("%.0f", k_format_csv[_count], at the end of this file).
 // __host__ __device__ like emb_events_expand.cuh, so that tests/emu runs the same code on the CPU.
 //
 // "%g" (C99 7.19.6.1, precision 6) is defined on the exact binary value v = m * 2^e: D = the 6-digit integer nearest to
@@ -8,18 +9,19 @@
 // The quotient and the comparison of the remainder with half the divisor are computed in exact integer arithmetic on
 // A / B = v / 10^k (A = m 2^max(e,0) 10^max(-k,0), B = 2^max(-e,0) 10^max(k,0)): in 128 bits when A and B fit in 125 bits
 // (every |v| from about 1e-17 to 1e37, so every sampled value and every id), otherwise in multi-word integers of up to 1280
-// bits (subnormals need 10^329 * 2^53).  A double quotient only proposes q; the integer remainder corrects it.  Nothing is
-// approximated, so the result is exact for every finite double (DESIGN.md section 13).
+// bits (emb_exact.cuh; A <= 2^53 * 10^329 < 2^1147 for the subnormals, B <= 2^1074).  A double quotient only proposes q; the
+// integer remainder corrects it.  Nothing is approximated, so the result is exact for every finite double (DESIGN.md section 13).
 //
 // Shape: one warp per track.  Lanes take consecutive items (transition: the rows of consecutive seconds; initial: the id and the
 // values of the row); a warp scan of their byte lengths gives every lane its offset, the lanes move their items into the warp's
 // shared-memory stage at those offsets, and the warp stores the stage as one contiguous block.  The count pass and the write pass
-// emit through the same templates (fmt_emit_*, fmt_item) into a counting or a writing sink, so their byte counts agree by
-// construction.
+// emit through the same templates (fmt_emit_*, fmt_item, fmt_stage_track) into a counting or a writing sink, so their byte
+// counts agree by construction.
 #pragma once
 #include <cstdint>
 
 #include "emb_events_expand.cuh"   // ExpandLanes (a warp on the device, one lane in the emulation), ll_flag
+#include "emb_exact.cuh"           // fmt_bits, u128, FmtBig and its operations
 
 namespace emb {
 
@@ -57,33 +59,6 @@ struct G6 {
     bool bad;   // inf or NaN
 };
 
-EMB_HD uint64_t fmt_bits(double v) {
-#if defined(__CUDA_ARCH__)
-    return (uint64_t)__double_as_longlong(v);
-#else
-    uint64_t b;
-    std::memcpy(&b, &v, 8);
-    return b;
-#endif
-}
-EMB_HD int fmt_clz64(uint64_t x) {   // x != 0
-#if defined(__CUDA_ARCH__)
-    return __clzll((long long)x);
-#else
-    return __builtin_clzll(x);
-#endif
-}
-EMB_HD int fmt_ctz64(uint64_t x) {   // x != 0
-#if defined(__CUDA_ARCH__)
-    return __ffsll((long long)x) - 1;
-#else
-    return __builtin_ctzll(x);
-#endif
-}
-
-typedef unsigned __int128 u128;
-
-
 EMB_HD int fmt_bitlen(u128 x) {
     const uint64_t hi = (uint64_t)(x >> 64), lo = (uint64_t)x;
     return hi ? 128 - fmt_clz64(hi) : lo ? 64 - fmt_clz64(lo) : 0;
@@ -114,79 +89,6 @@ EMB_HD void fmt_divmod128(u128 A, u128 B, uint32_t& q, int& half) {
     half = r < B ? -1 : r > B ? 1 : 0;
 }
 
-// Multi-word unsigned integers for the quotients outside the 128-bit range (little-endian 32-bit limbs).
-struct FmtBig {
-    static constexpr int N = 40;   // 1280 bits: A <= 2^53 * 10^329 < 2^1147, B <= 2^1074
-    uint32_t w[N];
-    int n;                         // limbs in use; w[n-1] != 0 unless n == 0
-};
-EMB_HD void big_set(FmtBig& a, uint64_t v) {
-    a.w[0] = (uint32_t)v;
-    a.w[1] = (uint32_t)(v >> 32);
-    a.n = a.w[1] ? 2 : a.w[0] ? 1 : 0;
-}
-EMB_HD void big_mul(FmtBig& a, uint32_t f) {
-    if (!f) a.n = 0;
-    uint64_t c = 0;
-    for (int i = 0; i < a.n; ++i) {
-        c += (uint64_t)a.w[i] * f;
-        a.w[i] = (uint32_t)c;
-        c >>= 32;
-    }
-    if (c) a.w[a.n++] = (uint32_t)c;
-}
-EMB_HD void big_mul_pow10(FmtBig& a, int j) {
-    for (; j >= 9; j -= 9) big_mul(a, 1000000000u);
-    uint32_t f = 1;
-    for (; j > 0; --j) f *= 10u;
-    if (f > 1) big_mul(a, f);
-}
-EMB_HD void big_shl(FmtBig& a, int s) {
-    if (!a.n || !s) return;
-    const int limbs = s >> 5, bits = s & 31;
-    int n = a.n + limbs;
-    a.w[n] = 0;
-    for (int i = a.n - 1; i >= 0; --i) {
-        const uint64_t x = (uint64_t)a.w[i] << bits;
-        a.w[i + limbs + 1] |= (uint32_t)(x >> 32);
-        a.w[i + limbs] = (uint32_t)x;
-    }
-    for (int i = 0; i < limbs; ++i) a.w[i] = 0;
-    a.n = a.w[n] ? n + 1 : n;
-}
-EMB_HD int big_cmp(const FmtBig& a, const FmtBig& b) {
-    if (a.n != b.n) return a.n < b.n ? -1 : 1;
-    for (int i = a.n - 1; i >= 0; --i)
-        if (a.w[i] != b.w[i]) return a.w[i] < b.w[i] ? -1 : 1;
-    return 0;
-}
-EMB_HD void big_sub(FmtBig& a, const FmtBig& b) {   // a -= b, a >= b
-    int64_t c = 0;
-    for (int i = 0; i < a.n; ++i) {
-        c += (int64_t)a.w[i] - (i < b.n ? (int64_t)b.w[i] : 0);
-        a.w[i] = (uint32_t)c;
-        c >>= 32;
-    }
-    while (a.n && !a.w[a.n - 1]) --a.n;
-}
-EMB_HD void big_add(FmtBig& a, const FmtBig& b) {
-    uint64_t c = 0;
-    const int n = a.n > b.n ? a.n : b.n;
-    for (int i = 0; i < n; ++i) {
-        c += (uint64_t)(i < a.n ? a.w[i] : 0) + (i < b.n ? b.w[i] : 0);
-        a.w[i] = (uint32_t)c;
-        c >>= 32;
-    }
-    a.n = n;
-    if (c) a.w[a.n++] = (uint32_t)c;
-}
-// a / 2^(32 (a.n - 3)) as a double (the top three limbs; relative error below 2^-63 before rounding)
-EMB_HD double big_top(const FmtBig& a) {
-    double r = 0.0;
-    for (int i = a.n - 1; i >= 0 && i >= a.n - 3; --i) r = r * 4294967296.0 + (double)a.w[i];
-    for (int i = a.n; i < 3; ++i) r *= 4294967296.0;   // fewer than three limbs: the same scale
-    return r;
-}
 EMB_HD void fmt_divmod_big(const FmtBig& A, const FmtBig& B, uint32_t& q, int& half) {
     double ratio = big_top(A) / big_top(B);
     for (int i = B.n; i < A.n; ++i) ratio *= 4294967296.0;
@@ -388,28 +290,26 @@ EMB_HD bool fmt_item(const FormatParams& P, int64_t s, int j, const G6& id, S& o
     return TRANS ? fmt_transition_row(P, s, j, id, out) : fmt_initial_item(P, s, j, out);
 }
 
-// Both passes of track s: the count pass returns its bytes; the write pass (WRITE) also stores them from P.offsets[s] on.
-// stage: FMT_STAGE_BYTES of the warp's shared memory (write pass): a slot of FMT_ROW_MAX bytes per lane, into which the lane
-// emits its item once, then the items packed at their scanned offsets, stored to global memory as one contiguous block.
-template <bool TRANS, bool WRITE>
-EMB_HD uint32_t format_track(const FormatParams& P, int64_t s, const ExpandLanes& L, char* stage) {
+// The staging shared by every text of this file: `items` items of one track, lane j of the warp taking items j, j + W, ...;
+// `item(j, sink)` emits item j (at most FMT_ROW_MAX bytes) and returns false for a non-finite value.  The count pass
+// (WRITE = false) returns the track's bytes; the write pass also stores them from dst on.  stage: FMT_STAGE_BYTES of the warp's
+// shared memory (write pass): a slot of FMT_ROW_MAX bytes per lane, into which the lane emits its item once, then the items
+// packed at their scanned offsets, stored to global memory as one contiguous block.
+template <bool WRITE, class Item>
+EMB_HD uint32_t fmt_stage_track(const Item& item, int items, char* dst, const ExpandLanes& L, char* stage, bool& ok) {
     const int W = ExpandLanes::width();
-    const int items = TRANS ? P.T : P.n_initial + 1;
-    const G6 id = TRANS ? fmt_g6((double)(P.first_id + s)) : G6{};
-    char* dst = WRITE ? P.text + P.offsets[s] : nullptr;
     char* slot = stage + FMT_STAGE + L.lane * FMT_ROW_MAX;
     uint32_t total = 0;
-    bool ok = true;
     for (int base = 0; base < items; base += W) {
         const int j = base + L.lane;
         int32_t len = 0;
         if (WRITE) {
             FmtWrite w{slot};
-            if (j < items) fmt_item<TRANS>(P, s, j, id, w);
+            if (j < items) item(j, w);
             len = (int32_t)(w.p - slot);
         } else {
             FmtCount c;
-            if (j < items) ok &= fmt_item<TRANS>(P, s, j, id, c);
+            if (j < items) ok &= item(j, c);
             len = c.n;
         }
         const int32_t incl = L.scan(len);
@@ -422,6 +322,143 @@ EMB_HD uint32_t format_track(const FormatParams& P, int64_t s, const ExpandLanes
         }
         total += (uint32_t)chunk;
     }
+    return total;
+}
+
+template <bool TRANS>
+struct FmtEmSampleItem {
+    const FormatParams& P;
+    int64_t s;
+    G6 id;
+    template <class S>
+    EMB_HD bool operator()(int j, S& out) const { return fmt_item<TRANS>(P, s, j, id, out); }
+};
+
+// Both passes of track s of initial.txt or transition.txt (fmt_stage_track).
+template <bool TRANS, bool WRITE>
+EMB_HD uint32_t format_track(const FormatParams& P, int64_t s, const ExpandLanes& L, char* stage) {
+    const int items = TRANS ? P.T : P.n_initial + 1;
+    const FmtEmSampleItem<TRANS> item{P, s, TRANS ? fmt_g6((double)(P.first_id + s)) : G6{}};
+    bool ok = true;
+    const uint32_t total = fmt_stage_track<WRITE>(item, items, WRITE ? P.text + P.offsets[s] : nullptr, L, stage, ok);
+    if (!ok) ll_flag(P.status, FMT_BAD_VALUE);
+    return total;
+}
+
+// ---- the CSV rows of sample2track.m (emb_format_tracks_csv) -------------------------------------------------------------------
+// One file body per track: T+1 rows "%d,%.0f,%.0f,%.0f\n" of (t, x_ft, y_ft, z_ft), t = 0 .. T, exactly as the Python statement
+// "%d,%.0f,%.0f,%.0f\n" % (t, x, y, z) formats the fp32 points widened to double.
+//
+// "%.0f" of a double is the integer nearest its exact value, ties to even, with "-" whenever the sign bit is set (so -0.4 and
+// -0.0 print "-0").  A finite float32 f = M 2^E (M < 2^24) is decided in integers: for |f| < 2^23 (E < 0) the quotient M >> -E
+// and its remainder against half of 2^-E; for |f| >= 2^23 f is an integer, M << E < 2^128, printed exactly from four 32-bit limbs
+// by repeated division by 10^9 (up to 39 digits).
+
+struct CsvParams {
+    int64_t n;
+    int32_t T;
+    const float* xyz;                 // [3][T+1][n] (emb_tracks_integrate)
+    const uint8_t* mask;              // [n] or nullptr; 0: no text for the track
+    const long long* offsets;         // [n+1] bytes before each track (write pass)
+    char* text;                       // write pass
+    uint32_t* counts;                 // [n] bytes of each track (count pass)
+    int32_t* status;                  // FMT_BAD_VALUE
+};
+
+// longest CSV row: "%d" of t < 2^31 (10 bytes), three ",-" and 39 digits (FLT_MAX), "\n"; it fits the staging slot
+constexpr int FMT_CSV_ROW_MAX = 10 + 3 * (2 + 39) + 1;
+static_assert(FMT_CSV_ROW_MAX <= FMT_ROW_MAX, "a CSV row must fit the staging slot of a lane");
+
+EMB_HD uint32_t fmt_float_bits(float f) {
+#if defined(__CUDA_ARCH__)
+    return (uint32_t)__float_as_uint(f);
+#else
+    uint32_t b;
+    std::memcpy(&b, &f, 4);
+    return b;
+#endif
+}
+
+template <class S>
+EMB_HD void fmt_emit_u32(uint32_t u, S& out) {
+    char dig[10];
+    int nd = 0;
+    do {
+        dig[nd++] = (char)('0' + u % 10u);
+        u /= 10u;
+    } while (u);
+    while (nd) out.put(dig[--nd]);
+}
+
+// "%.0f" of f widened to double; false (and nothing emitted) for inf and NaN
+template <class S>
+EMB_HD bool fmt_emit_f0(float f, S& out) {
+    const uint32_t b = fmt_float_bits(f);
+    const int be = (int)((b >> 23) & 0xFFu);
+    if (be == 0xFF) return false;
+    if (b >> 31) out.put('-');
+    const uint32_t M = (b & 0x7FFFFFu) | (be ? 0x800000u : 0u);
+    if (be < 150) {   // |f| < 2^23: f = M 2^-sh, sh = 1 .. 149
+        const int sh = 150 - (be ? be : 1);
+        uint32_t u = 0;
+        if (sh <= 25) {   // otherwise |f| < 2^24 2^-26, which rounds to 0
+            u = M >> sh;
+            const uint32_t rem = M & ((1u << sh) - 1u), half = 1u << (sh - 1);
+            u += (rem > half || (rem == half && (u & 1u))) ? 1u : 0u;
+        }
+        fmt_emit_u32(u, out);
+        return true;
+    }
+    const u128 v = (u128)M << (be - 150);   // an integer below 2^128
+    uint32_t w[4] = {(uint32_t)v, (uint32_t)(v >> 32), (uint32_t)(v >> 64), (uint32_t)(v >> 96)};
+    char dig[40];
+    int nd = 0;
+    bool more;
+    do {   // the lowest nine digits per round: w /= 10^9, r = the remainder
+        uint64_t r = 0;
+        for (int i = 3; i >= 0; --i) {
+            const uint64_t cur = (r << 32) | w[i];
+            w[i] = (uint32_t)(cur / 1000000000u);
+            r = cur % 1000000000u;
+        }
+        more = (w[0] | w[1] | w[2] | w[3]) != 0;
+        for (int k = 0; k < 9 && (more || r); ++k) {   // all nine below a higher group, no leading zeros in the top one
+            dig[nd++] = (char)('0' + r % 10u);
+            r /= 10u;
+        }
+    } while (more);
+    while (nd) out.put(dig[--nd]);
+    return true;
+}
+
+// row t of a track: "%d,%.0f,%.0f,%.0f\n" of (t, x, y, z); false if a coordinate is not finite
+template <class S>
+EMB_HD bool fmt_csv_row(const CsvParams& P, int64_t s, int t, S& out) {
+    fmt_emit_d(t, out);
+    const int64_t plane = (int64_t)(P.T + 1) * P.n;
+    const float* p = P.xyz + (int64_t)t * P.n + s;
+    bool ok = true;
+    for (int c = 0; c < 3; ++c) {
+        out.put(',');
+        ok &= fmt_emit_f0(p[c * plane], out);
+    }
+    out.put('\n');
+    return ok;
+}
+
+struct FmtCsvItem {
+    const CsvParams& P;
+    int64_t s;
+    template <class S>
+    EMB_HD bool operator()(int t, S& out) const { return fmt_csv_row(P, s, t, out); }
+};
+
+// Both passes of track s of the CSV text: 0 bytes for a masked track (fmt_stage_track).
+template <bool WRITE>
+EMB_HD uint32_t format_csv_track(const CsvParams& P, int64_t s, const ExpandLanes& L, char* stage) {
+    if (P.mask && !P.mask[s]) return 0;
+    bool ok = true;
+    const uint32_t total = fmt_stage_track<WRITE>(FmtCsvItem{P, s}, P.T + 1, WRITE ? P.text + P.offsets[s] : nullptr, L, stage, ok);
     if (!ok) ll_flag(P.status, FMT_BAD_VALUE);
     return total;
 }

@@ -16,6 +16,7 @@
 #include "emb_launch.h"
 #include "emb_loglik.cuh"
 #include "emb_loglik_events.cuh"
+#include "emb_parse.cuh"
 
 namespace emb {
 
@@ -396,6 +397,88 @@ __global__ void __maxnreg__(FMT_MAXNREG) k_format_initial(const __grid_constant_
 __global__ void __maxnreg__(FMT_MAXNREG) k_format_transition_count(const __grid_constant__ FormatParams P) { format_count<true>(P); }
 __global__ void __maxnreg__(FMT_MAXNREG) k_format_transition(const __grid_constant__ FormatParams P) { format_write<true>(P); }
 
+// the CSV rows of sample2track.m (emb_format.cuh: format_csv_track), the same shape and register cap
+__global__ void __maxnreg__(FMT_MAXNREG) k_format_csv_count(const __grid_constant__ CsvParams P) {
+    const int64_t s = (int64_t)blockIdx.x * (FMT_BLOCK / 32) + (threadIdx.x >> 5);
+    if (s >= P.n) return;
+    const ExpandLanes L{(int)(threadIdx.x & 31)};
+    const uint32_t bytes = format_csv_track<false>(P, s, L, nullptr);
+    if (L.lane == 0) P.counts[s] = bytes;
+}
+__global__ void __maxnreg__(FMT_MAXNREG) k_format_csv(const __grid_constant__ CsvParams P) {
+    __shared__ char stage[FMT_BLOCK / 32][FMT_STAGE_BYTES];
+    const int64_t s = (int64_t)blockIdx.x * (FMT_BLOCK / 32) + (threadIdx.x >> 5);
+    if (s >= P.n) return;
+    format_csv_track<true>(P, s, ExpandLanes{(int)(threadIdx.x & 31)}, stage[threadIdx.x >> 5]);
+}
+
+// decimal text tables (emb_parse.cuh).  Line discovery: one warp per PARSE_CHUNK bytes, each lane 16 bytes per round (one vector
+// load when the text is 16-byte aligned); then one thread per line for the checks and for the values.
+constexpr int PARSE_BLOCK = 256;
+constexpr int PARSE_CHUNK = 4096;
+constexpr int PARSE_ROUNDS = PARSE_CHUNK / 512;
+
+// the 16 bytes at pos, zeros past the end of the text
+__device__ __forceinline__ uint4 parse_load16(const ParseParams& P, int64_t pos) {
+    if (P.aligned && pos + 16 <= P.bytes) return __ldg(reinterpret_cast<const uint4*>(P.text + pos));
+    uint32_t w[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+    for (int b = 0; b < 16; ++b)
+        if (pos + b < P.bytes) w[b >> 2] |= (uint32_t)(uint8_t)P.text[pos + b] << (8 * (b & 3));
+    return make_uint4(w[0], w[1], w[2], w[3]);
+}
+__device__ __forceinline__ uint32_t parse_nl4(uint32_t x) { return __vcmpeq4(x, 0x0A0A0A0Au); }   // 0xFF in each '\n' byte
+__device__ __forceinline__ int parse_nl16(const uint4& v) {
+    return (__popc(parse_nl4(v.x)) + __popc(parse_nl4(v.y)) + __popc(parse_nl4(v.z)) + __popc(parse_nl4(v.w))) >> 3;
+}
+
+__global__ void __launch_bounds__(PARSE_BLOCK) k_parse_newline_count(const __grid_constant__ ParseParams P) {
+    const int64_t c = (int64_t)blockIdx.x * (PARSE_BLOCK / 32) + (threadIdx.x >> 5);
+    if (c >= P.chunks) return;
+    const int lane = threadIdx.x & 31;
+    int n = 0;
+#pragma unroll
+    for (int r = 0; r < PARSE_ROUNDS; ++r) n += parse_nl16(parse_load16(P, c * PARSE_CHUNK + r * 512 + lane * 16));
+    n = __reduce_add_sync(0xFFFFFFFFu, n);
+    if (lane == 0) P.chunk_newlines[c] = (uint32_t)n;
+}
+
+// starts[k + 1] = one past the k-th newline; starts[0] = 0 and starts[lines] = bytes + 1 (a newline after the end)
+__global__ void __launch_bounds__(PARSE_BLOCK) k_parse_line_starts(const __grid_constant__ ParseParams P) {
+    const int64_t c = (int64_t)blockIdx.x * (PARSE_BLOCK / 32) + (threadIdx.x >> 5);
+    if (c >= P.chunks) return;
+    const int lane = threadIdx.x & 31;
+    long long base = P.newlines_before[c];
+    for (int r = 0; r < PARSE_ROUNDS; ++r) {
+        const int64_t pos = c * PARSE_CHUNK + r * 512 + lane * 16;
+        const uint4 v = parse_load16(P, pos);
+        const int n = parse_nl16(v);
+        int incl = n;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int y = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+            if (lane >= o) incl += y;
+        }
+        long long k = base + incl - n;
+        const uint32_t m[4] = {parse_nl4(v.x), parse_nl4(v.y), parse_nl4(v.z), parse_nl4(v.w)};
+#pragma unroll
+        for (int b = 0; b < 16; ++b)
+            if ((m[b >> 2] >> (8 * (b & 3))) & 1u) P.starts[++k] = pos + b + 1;
+        base += __shfl_sync(0xFFFFFFFFu, incl, 31);
+    }
+    if (lane == 0 && c == 0) P.starts[0] = 0;
+    if (lane == 0 && c == P.chunks - 1) P.starts[P.lines] = P.bytes + 1;
+}
+
+__global__ void __launch_bounds__(PARSE_BLOCK) k_parse_lines(const __grid_constant__ ParseParams P) {
+    const int64_t i = (int64_t)blockIdx.x * PARSE_BLOCK + threadIdx.x;
+    if (i < P.lines) parse_check_line(P, i);
+}
+__global__ void __launch_bounds__(PARSE_BLOCK) k_parse_values(const __grid_constant__ ParseParams P) {
+    const int64_t i = (int64_t)blockIdx.x * PARSE_BLOCK + threadIdx.x;
+    if (i < P.lines) parse_values_line(P, i);
+}
+
 }  // namespace
 
 int launch_publish(const long long* total, const int32_t* flag, long long* mapped_dst, void* stream) {
@@ -604,6 +687,32 @@ int launch_events_expand(const DevModel& M, const ExpandParams& P, const EventRo
     } else {
         if (packed) k_events_expand<true><<<grid, EE_BLOCK, 0, st>>>(M, P, R);
         else k_events_expand<false><<<grid, EE_BLOCK, 0, st>>>(M, P, R);
+    }
+    g_launch_count.fetch_add(1);
+    return (int)cudaGetLastError();
+}
+
+int launch_format_csv(const CsvParams& P, bool count, void* stream) {
+    if (P.n <= 0) return 0;
+    const unsigned grid = (unsigned)((P.n + FMT_BLOCK / 32 - 1) / (FMT_BLOCK / 32));
+    if (count) k_format_csv_count<<<grid, FMT_BLOCK, 0, (cudaStream_t)stream>>>(P);
+    else k_format_csv<<<grid, FMT_BLOCK, 0, (cudaStream_t)stream>>>(P);
+    g_launch_count.fetch_add(1);
+    return (int)cudaGetLastError();
+}
+
+int64_t parse_chunk_bytes() { return PARSE_CHUNK; }
+
+int launch_parse(const ParseParams& P, int pass, void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t items = pass < 2 ? (P.chunks + PARSE_BLOCK / 32 - 1) / (PARSE_BLOCK / 32) : (P.lines + PARSE_BLOCK - 1) / PARSE_BLOCK;
+    if (items <= 0) return 0;
+    const unsigned grid = (unsigned)items;
+    switch (pass) {
+        case 0: k_parse_newline_count<<<grid, PARSE_BLOCK, 0, st>>>(P); break;
+        case 1: k_parse_line_starts<<<grid, PARSE_BLOCK, 0, st>>>(P); break;
+        case 2: k_parse_lines<<<grid, PARSE_BLOCK, 0, st>>>(P); break;
+        default: k_parse_values<<<grid, PARSE_BLOCK, 0, st>>>(P); break;
     }
     g_launch_count.fetch_add(1);
     return (int)cudaGetLastError();

@@ -45,6 +45,14 @@ int launch_events_expand(const DevModel& M, const ExpandParams& P, const EventRo
 // the text files of em_sample.m (emb_format.cuh): the count pass (P.counts) or the write pass of initial.txt or transition.txt
 struct FormatParams;
 int launch_format(const FormatParams& P, bool transition, bool count, void* stream);
+// the CSV rows of sample2track.m (emb_format.cuh): the count pass (P.counts) or the write pass
+struct CsvParams;
+int launch_format_csv(const CsvParams& P, bool count, void* stream);
+// decimal text tables (emb_parse.cuh), pass 0: newlines per chunk of parse_chunk_bytes() bytes (k_parse_newline_count), 1: line
+// starts (k_parse_line_starts), 2: field checks and row flags per line (k_parse_lines), 3: the values (k_parse_values)
+struct ParseParams;
+int64_t parse_chunk_bytes();
+int launch_parse(const ParseParams& P, int pass, void* stream);
 
 // terminal trajectory chains (emb_terminal.cu): 4 chains per encounter
 struct TermParams;

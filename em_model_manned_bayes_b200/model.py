@@ -44,10 +44,15 @@ def untile(buf, nvar: int, n: int, T: int):
     return a.reshape(ntile * TRACK_TILE, nvar, nch * 4)[:n, :, :T]
 
 
-def tile(vals: np.ndarray) -> np.ndarray:
-    """(n, nvar, T) -> the dense layout as a flat array (the inverse of `untile`; padding tracks and seconds are 0)."""
+def tile(vals):
+    """(n, nvar, T) -> the dense layout as a flat array (the inverse of `untile`; padding tracks and seconds are 0).  numpy in,
+    numpy out; a torch tensor in, a tensor on its device out."""
     n, nvar, T = vals.shape
     nch, ntile = (T + 3) // 4, (n + TRACK_TILE - 1) // TRACK_TILE
+    if not isinstance(vals, np.ndarray):
+        pad = vals.new_zeros((ntile * TRACK_TILE, nvar, nch * 4))
+        pad[:n, :, :T] = vals
+        return pad.reshape(ntile, TRACK_TILE, nvar, nch, 4).permute(3, 0, 2, 1, 4).contiguous().reshape(-1)
     pad = np.zeros((ntile * TRACK_TILE, nvar, nch * 4), dtype=vals.dtype)
     pad[:n, :, :T] = vals
     return np.ascontiguousarray(pad.reshape(ntile, TRACK_TILE, nvar, nch, 4).transpose(3, 0, 2, 1, 4)).ravel()

@@ -414,6 +414,38 @@ int emb_format_em_sample(const emb_model* m, int64_t n, int32_t T, int64_t first
                          const emb_sample_opts* opts, int64_t capacity_initial, char* initial, int64_t* initial_offsets,
                          int64_t capacity_transition, char* transition, int64_t* transition_offsets, int64_t* total_bytes);
 
+/* ---- the CSV rows of sample2track.m:246-290 (BAYES_t*_id*_alt*_speed*.csv without its header line), formatted on the device
+ *      from the output of emb_tracks_integrate --------------------------------------------------------------------------------- */
+/* For each track s with mask[s] != 0 (every track if mask is NULL): T+1 rows "%d,%.0f,%.0f,%.0f\n" of (t, x_ft, y_ft, z_ft),
+ * t = 0 .. T, the fp32 points widened to double, exactly as C's printf and Python's '%' print them: "%.0f" is the integer nearest
+ * the exact value, ties to even, with '-' whenever the sign bit is set (-0.4 and -0.0 print "-0"); every finite float is exact
+ * (|f| >= 2^23 is an integer below 2^128, printed in full).  A masked track gets no bytes.
+ * xyz: float [3][T+1][n] (emb_tracks_integrate's layout); mask: uint8 [n], nullable.  Track s is text[offsets[s] ..
+ * offsets[s+1]); offsets: int64 [n+1], nullable.  *total_bytes (host, nullable) receives the total.  If it exceeds capacity, no
+ * text is written, the offsets and the total are, and EMB_E_LIMIT is returned: capacity 0 with a NULL text sizes the call.
+ * Only mem, device and stream of `opts` are read; every buffer is in opts->mem memory.  EMB_E_ARG, found on the device: a
+ * coordinate of an unmasked track that is not finite (libc and Python spell inf and NaN differently).  Refused before the
+ * device is touched: EMB_MEM_ASYNC, n < 0, T < 0; EMB_E_LIMIT when the T+1 rows of a track could exceed 2^32 bytes. */
+int emb_format_tracks_csv(int64_t n, int32_t T, const float* xyz, const uint8_t* mask, const emb_sample_opts* opts, int64_t capacity,
+                          char* text, int64_t* offsets, int64_t* total_bytes);
+
+/* ---- decimal text tables (the bodies of em_sample.m's initial.txt and transition.txt, as sample2track.m reads them) parsed to
+ *      fp64 on the device; no model ----------------------------------------------------------------------------------------- */
+/* text[0 .. bytes): the body of a file without its header line.  Lines and fields follow np.loadtxt: a line ends at '\n' or at
+ * the end of the text; fields are separated by runs of ' ', '\t' and '\r' (so CRLF files parse); a line without a field is
+ * skipped; every other line must have exactly `cols` fields.  A field is [+-]?(d+(.d*)?|.d+)([eE][+-]?d+)? with at most 19
+ * significant digits once the leading and trailing zeros of its digits are dropped; anything else (inf, nan, hex, "1,5", "1e",
+ * "--1", "1..2") is refused.  Its value is the correctly rounded double, ties to even: bit for bit what Python's float() and
+ * np.loadtxt return, -0 included, underflow to the correctly rounded subnormal or +-0; a value that rounds to +-inf is refused.
+ * values: double [rows][cols], row-major, the non-blank lines in order; *total_rows (host, nullable) receives their number.  If
+ * it exceeds capacity_rows, no value is written and EMB_E_LIMIT is returned: capacity 0 with a NULL values sizes the call.
+ * A refused text returns EMB_E_ARG; *bad_line (host, nullable; 0 otherwise) receives the 1-based line (of the text, so the
+ * header is not counted) of the first error, which the error message also names.  Only mem, device and stream of `opts` are
+ * read; text and values are in opts->mem memory.  Refused before the device is touched: EMB_MEM_ASYNC, bytes < 0, cols outside
+ * 1 .. 256. */
+int emb_parse_table(const char* text, int64_t bytes, int32_t cols, const emb_sample_opts* opts, int64_t capacity_rows, double* values,
+                    int64_t* total_rows, int64_t* bad_line);
+
 /* ---- misc ------------------------------------------------------------------------------------- */
 int emb_host_alloc(void** p, int64_t bytes); /* pinned host memory */
 int emb_host_free(void* p);
